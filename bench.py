@@ -5,7 +5,7 @@ decoder, open_set/models/mask2former_head.py:787-849) over one batch of syntheti
 outputs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--batch B_per_gpu] [--precision bf16|fp32] [--queries Q]
+                    [--batch B_per_gpu] [--precision bf16|fp32] [--queries Q] [--dump-outputs DIR]
 
 N>1 is launched by torch.distributed.run, one rank per GPU; images shard by batch, no data-path
 collective (SURVEY.md section 8e), so "scaling" is weak.  Rank 0 prints ONE JSON line.  Besides the
@@ -40,6 +40,7 @@ FFN = 2048
 D_L = 768
 NCLS1 = 49
 LAYERS = 9
+DUMP_BYTES = 60 * 10**6         # --dump-outputs: at most this much in all, float32
 
 
 def flops_per_image(Q, height=H, width=W):
@@ -53,6 +54,24 @@ def flops_per_image(Q, height=H, width=W):
     f += LAYERS * (8 * Q * C * C + 4 * Q * Q * C)
     f += LAYERS * (4 * Q * C * FFN)
     return float(f)
+
+
+def dump_outputs(out_dir, outs):
+    """Writes what one step of the path returned -- the cls / emb / mask lists of the head calls, each list stacked into
+    one array -- as out_dir/{cls,emb,mask}.npy in float32, so that two builds can be compared output for output.  An
+    array larger than its even share of DUMP_BYTES is replaced by a fixed sample of its flattened elements: the array is
+    cut into cap blocks that together cover it to the last element (block i starts at floor(i * numel / cap)), and one
+    element is taken from each block at a seeded offset -- the same positions on every run with the same shapes."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(outs)
+    for name, xs in zip(('cls', 'emb', 'mask'), outs):
+        a = torch.stack([x for x in xs if x is not None])           # (--final-mask-only: the last mask only)
+        if a.numel() > cap:
+            starts = torch.arange(cap + 1) * a.numel() // cap
+            offs = torch.randint(0, 2**62, (cap,), generator=torch.Generator().manual_seed(0)) % (starts[1:] - starts[:-1])
+            a = a.reshape(-1)[(starts[:-1] + offs).to(a.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), a.float().cpu().numpy())
 
 
 def einsum_flops_per_launch(Q, batch):
@@ -670,6 +689,7 @@ def run_b200_arm(args):
     fly_in = [(mf_d, mems_d)] + [(mf_d.clone(), [m.clone() for m in mems_d]) for _ in range(n_fly - 1)]
     fly_streams = [torch.cuda.Stream() for _ in range(n_fly)]
     step_no = [0]
+    last_out = [None]           # what the last timed step returned (--dump-outputs)
 
     def step_resident():
         i = step_no[0] % n_fly
@@ -698,7 +718,7 @@ def run_b200_arm(args):
         e0.record()
         fork()
         for _ in range(n):
-            step_resident()
+            last_out[0] = step_resident()
         join()
         e1.record()
         barrier()
@@ -732,6 +752,8 @@ def run_b200_arm(args):
         torch.cuda.synchronize()
         launches = (lib.cgg_launch_count() - l0) * args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out[0])
     ms = reduce_max(ms, world, dev)
     value = whole_job_value(world, B, args.steps, ms)
 
@@ -1006,7 +1028,16 @@ def main():
                     help='opt-in inference shortcut: produce the last head call mask only (NOT the headline contract)')
     ap.add_argument('--in-flight', type=int, default=4,
                     help='batches in flight in the device-resident throughput leg (one head + stream each)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy, float32; '
+                         'arrays too large for the %d MB budget as a fixed sample.  --impl b200 only: the reference '
+                         'arm runs one image per step, not the b200 arm\'s batch, so its outputs would not line up'
+                         % (DUMP_BYTES // 10**6))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     if args.impl == 'reference':
         run_reference_arm(args)
     else:

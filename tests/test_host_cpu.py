@@ -119,3 +119,27 @@ def test_no_gc_during_capture_context():
     finally:
         if was:
             gc.enable()
+
+
+def test_bench_dump_outputs_fixed_sample_within_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: small arrays whole (shape kept), larger ones as one element from each of `cap` blocks
+    that cover the array to its last element, at the same positions on every call, float32, within the byte budget."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 3 * 4 * 1000)
+    g = torch.Generator().manual_seed(0)
+    outs = ([torch.randn((2, 5, 7), generator=g) for _ in range(10)], [torch.randn((1, 1, 199), generator=g) for _ in range(10)],
+            [None] * 9 + [torch.randn((2, 5, 16, 16), generator=g).bfloat16()])
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    got = {n: np.load(tmp_path / 'a' / (n + '.npy')) for n in ('cls', 'emb', 'mask')}
+    assert all(v.dtype == np.float32 and np.array_equal(v, np.load(tmp_path / 'b' / (n + '.npy'))) for n, v in got.items())
+    assert np.array_equal(got['cls'], torch.stack(outs[0]).numpy())
+    # emb: 1990 elements, just under twice the 1000-element share: the blocks must still reach its last element
+    for name, full in (('emb', torch.stack(outs[1])), ('mask', outs[2][-1].float())):
+        full = full.reshape(-1).numpy()
+        starts = [i * full.size // 1000 for i in range(1001)]
+        assert got[name].shape == (1000,) and starts[-1] == full.size
+        assert all(got[name][i] in full[starts[i]:starts[i + 1]] for i in range(1000)), name
+        assert not np.array_equal(got[name], full[starts[:-1]])     # offsets within the blocks vary
+    assert sum(f.stat().st_size for f in (tmp_path / 'a').iterdir()) <= bench.DUMP_BYTES + 3 * 128

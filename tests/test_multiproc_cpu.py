@@ -5,11 +5,30 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def _np(x):
+    """Results cross the queue BY VALUE (numpy): a torch tensor would be handed over through the sender's fd-sharing
+    socket, which is gone if the worker exits before the parent unpickles."""
+    if torch.is_tensor(x):
+        return x.detach().numpy().copy()
+    if isinstance(x, (tuple, list)):
+        return tuple(_np(v) for v in x)
+    return x
+
+
+def _pt(x):
+    if isinstance(x, np.ndarray):
+        return torch.from_numpy(x)
+    if isinstance(x, tuple):
+        return tuple(_pt(v) for v in x)
+    return x
 
 
 def _worker(rank, world, port, q):
@@ -60,7 +79,7 @@ def _gather_worker(rank, world, port, q):
     embs, mask, preds = gather_captions_and_preds(list(cap_all[sl]), list(mask_all[sl]), pred)
     loss = sum(O.grounding_loss(preds[l], embs, mask, 10.0, 2.0) for l in range(preds.shape[0]))
     loss.backward()
-    q.put((rank, embs.clone(), mask.clone(), preds.detach().clone(), float(loss), pred.grad.clone()))
+    q.put(_np((rank, embs, mask, preds, float(loss), pred.grad)))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -84,7 +103,7 @@ def test_batched_caption_gather_matches_single_process():
     procs = [ctx.Process(target=_gather_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    res = sorted((q.get(timeout=120) for _ in range(2)), key=lambda r: r[0])
+    res = sorted((_pt(q.get(timeout=120)) for _ in range(2)), key=lambda r: r[0])
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
@@ -117,7 +136,7 @@ def _reducer_worker(rank, world, port, q):
     assert all(p.grad.data_ptr() == red.buckets[red.index[p][0]]['flat'].data_ptr() + 4 * red.index[p][1] for p in net.parameters())
     net(x).pow(2).mean().backward()
     red.finish()
-    q.put((rank, len(red.buckets), [p.grad.clone() for p in net.parameters()]))
+    q.put(_np((rank, len(red.buckets), [p.grad for p in net.parameters()])))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -131,7 +150,7 @@ def test_bucketed_grad_reducer_two_ranks_gloo():
     procs = [ctx.Process(target=_reducer_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    res = sorted((q.get(timeout=120) for _ in range(2)), key=lambda r: r[0])
+    res = sorted((_pt(q.get(timeout=120)) for _ in range(2)), key=lambda r: r[0])
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
@@ -186,7 +205,7 @@ def _fused_reducer_worker(rank, world, port, q):
         h = torch.relu(_FusedLinear.apply(x, W1, red))
         (_FusedLinear.apply(h, W2, red) + b2).pow(2).mean().backward()
         red.finish()
-    q.put((rank, [p.grad.clone() for p in (W1, W2, b2)]))
+    q.put(_np((rank, [p.grad for p in (W1, W2, b2)])))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -201,7 +220,7 @@ def test_grad_reducer_counts_a_fused_parameter_once():
     procs = [ctx.Process(target=_fused_reducer_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    res = sorted((q.get(timeout=120) for _ in range(2)), key=lambda r: r[0])
+    res = sorted((_pt(q.get(timeout=120)) for _ in range(2)), key=lambda r: r[0])
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
