@@ -975,6 +975,28 @@ extern "C" int cgg_softmax_rows(cgg_handle* h, float* x, int rows, int n, void* 
   return CGG_OK;
 }
 
+extern "C" size_t cgg_panoptic_scratch_bytes(int batch, int num_q) {
+  if (batch < 1 || num_q < 1) return 0;
+  return panoptic_scratch_bytes(batch, num_q);
+}
+
+extern "C" int cgg_panoptic_fuse(cgg_handle* h, const void* logits, int is_bf16, const float* probs, const int* geom, int batch,
+                                 int num_q, int classes_p1, int num_things, int h4, int w4, int up_h, int up_w, int max_out_h,
+                                 int max_out_w, double object_mask_thr, double iou_thr, int filter_low_score, int* pan,
+                                 int* mask_area, int* original_area, int* seg_value, void* scratch, size_t scratch_bytes,
+                                 void* stream) {
+  if (!h || !logits || !probs || !geom || !pan || !scratch) return CGG_ERR_NULL;
+  if (batch < 1 || batch > 65535 || num_q < 1 || num_q > 4096 || classes_p1 < 2 || num_things < 0 ||
+      num_things > classes_p1 - 1 || h4 < 1 || w4 < 1 || up_h < 1 || up_w < 1 || max_out_h < 1 || max_out_h > 65535 ||
+      max_out_w < 1)
+    return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  if (scratch_bytes < panoptic_scratch_bytes(batch, num_q)) return fail(h, CGG_ERR_WORKSPACE, "panoptic scratch too small");
+  CU(launch_panoptic_fuse(logits, is_bf16 != 0, probs, geom, batch, num_q, classes_p1, num_things, h4, w4, up_h, up_w, max_out_h,
+                          max_out_w, object_mask_thr, iou_thr, filter_low_score != 0, pan, mask_area, original_area, seg_value,
+                          scratch, (cudaStream_t)stream));
+  return CGG_OK;
+}
+
 // ====================================================================== the pixel decoder before the path (row f3)
 extern "C" int cgg_ms_deform_attn(cgg_handle* h, const float* value, long value_stride, const float* offsets, long offset_stride,
                                   const float* weight_logits, long logit_stride, float* out, int batch, int tokens, int heads,

@@ -146,6 +146,11 @@ cudaError_t launch_instance_mask_stats(const void* logits, bool bf16, const int*
                                        int up_w, int max_out_h, int max_out_w, uint32_t* bits, int* count, float* sig_sum,
                                        int* bbox, cudaStream_t s);
 cudaError_t launch_softmax_rows(float* x, int rows, int n, cudaStream_t s);
+size_t panoptic_scratch_bytes(int B, int Q);
+cudaError_t launch_panoptic_fuse(const void* logits, bool bf16, const float* probs, const int* geom, int B, int Q, int n_cls_p1,
+                                 int num_things, int h4, int w4, int up_h, int up_w, int max_out_h, int max_out_w,
+                                 double object_mask_thr, double iou_thr, bool filter_low_score, int* pan, int* mask_area,
+                                 int* original_area, int* seg_value, void* scratch, cudaStream_t s);
 
 // fp32 (rows, cols) -> bf16 (rows, 2*cols) hi/lo pairs: [hi | lo] per row
 cudaError_t launch_cast_bf16_split(const float* in, __nv_bfloat16* out, int rows, int cols, cudaStream_t s);

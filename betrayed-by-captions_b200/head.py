@@ -657,10 +657,12 @@ class _Runtime:
 
 
 def build_head_from_state_dict(sd, num_queries, num_classes_p1=49, precision='fp32', device='cuda', num_layers=9,
-                               cuda_graph=False, final_mask_only=False, **kwargs):
-    """Convenience used by tests / bench: a head carrying the given (reference-keyed) weights."""
+                               cuda_graph=False, final_mask_only=False, num_stuff_classes=0, **kwargs):
+    """Convenience used by tests / bench: a head carrying the given (reference-keyed) weights.  The last
+    num_stuff_classes of the num_classes_p1 - 1 classes are stuff (panoptic output), the others things."""
     kwargs.setdefault('use_class_emb', 'v2l_transform.weight' in sd)
-    head = Mask2FormerHeadOpenB200(num_things_classes=num_classes_p1 - 1, num_stuff_classes=0,
+    head = Mask2FormerHeadOpenB200(num_things_classes=num_classes_p1 - 1 - num_stuff_classes,
+                                   num_stuff_classes=num_stuff_classes,
                                    num_queries=num_queries, precision=precision, cuda_graph=cuda_graph,
                                    final_mask_only=final_mask_only, **kwargs,
                                    transformer_decoder=dict(num_layers=num_layers))

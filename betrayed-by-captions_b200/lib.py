@@ -22,7 +22,8 @@ EXPORTS = ['cgg_create', 'cgg_destroy', 'cgg_last_error', 'cgg_version', 'cgg_la
            'cgg_attention_f32', 'cgg_attention_backward', 'cgg_attn_softmax_rows', 'cgg_attn_dscore', 'cgg_point_sample', 'cgg_point_sample_backward',
            'cgg_matching_cost', 'cgg_point_losses', 'cgg_point_losses_backward', 'cgg_weighted_ce', 'cgg_weighted_ce_backward',
            # test-time step after the path
-           'cgg_upsample_masks', 'cgg_instance_mask_stats', 'cgg_softmax_rows',
+           'cgg_upsample_masks', 'cgg_instance_mask_stats', 'cgg_softmax_rows', 'cgg_panoptic_scratch_bytes',
+           'cgg_panoptic_fuse',
            # the pixel decoder before the path
            'cgg_ms_deform_attn', 'cgg_ms_deform_attn_backward', 'cgg_group_norm_scratch_bytes', 'cgg_group_norm_tokens',
            'cgg_group_norm_tokens_backward', 'cgg_upsample_add_tokens', 'cgg_upsample_add_tokens_backward',
@@ -136,6 +137,10 @@ def load():
     lib.cgg_upsample_masks.argtypes = [vp, vp, i, vp, i, i, i, i, i, vp]
     lib.cgg_instance_mask_stats.argtypes = [vp, vp, i, vp, i, i, i, i, i, i, i, i, vp, vp, vp, vp, vp]
     lib.cgg_softmax_rows.argtypes = [vp, vp, i, i, vp]
+    lib.cgg_panoptic_scratch_bytes.argtypes = [i, i]
+    lib.cgg_panoptic_scratch_bytes.restype = sz
+    dbl = C.c_double
+    lib.cgg_panoptic_fuse.argtypes = [vp, vp, i, vp, vp, i, i, i, i, i, i, i, i, i, i, dbl, dbl, i, vp, vp, vp, vp, vp, sz, vp]
     ip = C.POINTER(C.c_int)
     lib.cgg_ms_deform_attn.argtypes = [vp, vp, lg, vp, lg, vp, lg, vp, i, i, i, i, i, ip, ip, vp]
     lib.cgg_ms_deform_attn_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, ip, ip, vp]

@@ -354,13 +354,31 @@ int cgg_weighted_ce_backward(cgg_handle *h, const float *logits, const int64_t *
  *   writing full-resolution logits.  geom (DEVICE, B x 4 int32) = {crop_h, crop_w, out_h, out_w} per image (out = crop
  *   when not rescaling).  Outputs: bits (B, Q, max_out_h, ceil(max_out_w/32)) u32 packed binary masks (may be NULL),
  *   count (B,Q) int32, sig_sum (B,Q) fp32, bbox (B,Q,4) int32 = x0, y0, x1+1, y1+1 (zeros for an empty mask).
- * cgg_softmax_rows: in-place row softmax (get_cls_emb_scores, maskformer_fusion_head.py:312-313). */
+ * cgg_softmax_rows: in-place row softmax (get_cls_emb_scores, maskformer_fusion_head.py:312-313).
+ * cgg_panoptic_fuse: the fusion head's panoptic output (mmdet 2.28.2 MaskFormerFusionHead.panoptic_postprocess with the
+ *   class-embedding probabilities) from the same logits and the same resample / crop / rescale as cgg_instance_mask_stats,
+ *   with no host round trip.  probs (B, Q, classes_p1) fp32 on the device (column classes_p1 - 1 = void); geom as above.
+ *   scores, labels = probs.max(-1); keep = label != void & score > (float)object_mask_thr; per pixel the kept query with
+ *   the largest score * sigmoid(logit) wins (first in query order on ties); a kept query whose winning area over its
+ *   #(sigmoid >= 0.5) is >= iou_thr (double) becomes a segment: label + 1000 * instance_id for things (label <
+ *   num_things, ids 1, 2, ... in query order over the valid things), label for stuff (one value per class).  pan
+ *   (B, max_out_h, max_out_w) int32 is written inside each image's out_h x out_w only: the segment value, or classes_p1 - 1
+ *   where no segment covers the pixel (with filter_low_score, also where the winner's sigmoid is < 0.5).  mask_area,
+ *   original_area, seg_value (B, Q) int32 per query id (may be NULL): winning pixels, pixels with sigmoid >= 0.5, segment
+ *   value; 0, 0, -1 for queries not kept, seg_value -1 for a dropped query.  scratch: device memory of at least
+ *   cgg_panoptic_scratch_bytes(batch, num_q) bytes, else CGG_ERR_WORKSPACE.  num_q <= 4096. */
 int cgg_upsample_masks(cgg_handle *h, const void *logits, int is_bf16, float *out, int planes, int h4, int w4, int up_h,
                        int up_w, void *stream);
 int cgg_instance_mask_stats(cgg_handle *h, const void *logits, int is_bf16, const int *geom, int batch, int num_q, int h4,
                             int w4, int up_h, int up_w, int max_out_h, int max_out_w, uint32_t *bits, int *count,
                             float *sig_sum, int *bbox, void *stream);
 int cgg_softmax_rows(cgg_handle *h, float *x, int rows, int n, void *stream);
+size_t cgg_panoptic_scratch_bytes(int batch, int num_q);
+int cgg_panoptic_fuse(cgg_handle *h, const void *logits, int is_bf16, const float *probs, const int *geom, int batch,
+                      int num_q, int classes_p1, int num_things, int h4, int w4, int up_h, int up_w, int max_out_h,
+                      int max_out_w, double object_mask_thr, double iou_thr, int filter_low_score, int *pan,
+                      int *mask_area, int *original_area, int *seg_value, void *scratch, size_t scratch_bytes,
+                      void *stream);
 
 /* ---- the step before the path: mmdet MSDeformAttnPixelDecoder (SURVEY.md 8f rank 3) ------------------------------
  * `mask_features, multi_scale_memorys = self.pixel_decoder(feats)` (mask2former_head.py:787; configured at
