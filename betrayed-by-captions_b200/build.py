@@ -30,7 +30,7 @@ def build(force=False, verbose=False):
     procs = []
     for src in SOURCES:
         obj = os.path.join(CSRC, src.replace('.cu', '.o'))
-        extra = os.environ.get('CGG_NVCC_EXTRA', '').split()      # e.g. -DCGG_AT_TRACING for the attention trace
+        extra = os.environ.get('CGG_NVCC_EXTRA', '').split()      # extra nvcc flags, e.g. -Xptxas -warn-spills
         cmd = [nvcc] + NVCC_FLAGS + extra + (['-Xptxas', '-v'] if verbose else []) + ['-c', os.path.join(CSRC, src), '-o', obj]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
         objs.append(obj)

@@ -73,6 +73,12 @@ int fail(cgg_handle* h, int code, const std::string& msg) {
     int s__ = (call);                  \
     if (s__ != CGG_OK) return s__;     \
   } while (0)
+// a tc_* stage on TcState `t`: a failure hands its message to the handle
+#define TC(t, call)                                                                          \
+  do {                                                                                       \
+    int s__ = (call);                                                                        \
+    if (s__ != CGG_OK) return fail(h, s__, std::string(#call) + ": " + tc_last_error(t));   \
+  } while (0)
 
 inline size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
@@ -253,10 +259,7 @@ extern "C" int cgg_prepare(cgg_handle* h, const cgg_weights* w, int H4, int W4, 
       CU(launch_gemm_f32(v, s));
     }
   }
-  if (h->tc) {
-    int st = tc_prepare(h->tc, w, H4, W4, h->lh, h->lw, h->nl, h->wkv, h->rk, h->bkv, s);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_prepare: ") + tc_last_error(h->tc));
-  }
+  if (h->tc) TC(h->tc, tc_prepare(h->tc, w, H4, W4, h->lh, h->lw, h->nl, h->wkv, h->rk, h->bkv, s));
   h->prepared = true;
   return CGG_OK;
 }
@@ -293,8 +296,8 @@ static int kv_project_levels(cgg_handle* h, const cgg_weights* w, int batch, con
     if (!memories[l]) return fail(h, CGG_ERR_NULL, "null memory level");
     const int K = h->lh[l] * h->lw[l], N = h->nl[l] * 2 * C;
     if (h->cfg.precision == CGG_BF16) {
-      int st = tc_kv_project(h->tc, l, batch, memories[l], at<void>(workspace, ws.kv[l]), at<void>(workspace, ws.tcws), s, cta_cap);
-      if (st != CGG_OK) return fail(h, st, std::string("tc_kv_project: ") + tc_last_error(h->tc));
+      TC(h->tc, tc_kv_project(h->tc, l, batch, memories[l], at<void>(workspace, ws.kv[l]), at<void>(workspace, ws.tcws), s,
+                              cta_cap));
       continue;
     }
     GemmF32 p;
@@ -343,8 +346,7 @@ static int head_call_impl(cgg_handle* h, const cgg_weights* w, int batch, const 
   float* me = mask_embed_out ? mask_embed_out : at<float>(workspace, ws.me);
   // K1: post_norm + the three heads (head.py:734-746)
   if (c.precision == CGG_BF16) {
-    int st = tc_query_heads(h->tc, w, batch, x, cls, emb, me, at<void>(workspace, ws.tcws), s, call_slot, z_ready);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_query_heads: ") + tc_last_error(h->tc));
+    TC(h->tc, tc_query_heads(h->tc, w, batch, x, cls, emb, me, at<void>(workspace, ws.tcws), s, call_slot, z_ready));
   } else {
   CU(launch_layernorm(x, nullptr, w->post_norm_w, w->post_norm_b, z, rows, C, 1e-5f, true, s));
   ST(linear_rows(h, s, z, nullptr, 1, w->cls_w, w->cls_b, cls, rows, c.num_classes_p1, C));
@@ -357,18 +359,13 @@ static int head_call_impl(cgg_handle* h, const cgg_weights* w, int batch, const 
   if (c.pred_emb_norm && c.d_lang > 0) CU(launch_l2norm_rows(emb, rows, c.d_lang, s));
   if (c.precision == CGG_BF16) {
     void* tws = at<void>(workspace, ws.tcws);
-#define TC(call)                                                                                \
-  do {                                                                                          \
-    int st__ = (call);                                                                          \
-    if (st__ != CGG_OK) return fail(h, st__, std::string(#call) + ": " + tc_last_error(h->tc)); \
-  } while (0)
-    TC(tc_store_mask_embed(h->tc, batch, call_slot, me, tws, s));
+    TC(h->tc, tc_store_mask_embed(h->tc, batch, call_slot, me, tws, s));
     if (bitmap) {
       // K3 on tensor cores: me x (mask_features resampled to the level) -> threshold -> ballot
-      if (!fds_ready) TC(tc_downsample(h->tc, batch, mask_features, tws, s));
-      TC(tc_mask_bits(h->tc, batch, call_slot, target_level, bitmap, all_masked, tws, s));
+      if (!fds_ready) TC(h->tc, tc_downsample(h->tc, batch, mask_features, tws, s));
+      TC(h->tc, tc_mask_bits(h->tc, batch, call_slot, target_level, bitmap, all_masked, tws, s));
     }
-    if (!defer_einsum) TC(tc_mask_einsum(h->tc, batch, call_slot, 1, mask_features, mask, 0, tws, s));
+    if (!defer_einsum) TC(h->tc, tc_mask_einsum(h->tc, batch, call_slot, 1, mask_features, mask, 0, tws, s));
     return CGG_OK;
   }
   // K2: mask_pred[b,q,p] = sum_c me[b,q,c] F[b,c,p]   (head.py:748)
@@ -403,9 +400,8 @@ extern "C" int cgg_mask_einsum(cgg_handle* h, int batch, int first_call, int num
   if (first_call < 0 || num_calls < 1 || first_call + num_calls > h->cfg.num_layers + 1)
     return fail(h, CGG_ERR_BAD_SHAPE, "bad head-call range");
   const long call_stride = (long)batch * h->cfg.num_queries * h->H4 * h->W4;
-  int st = tc_mask_einsum(h->tc, batch, first_call, num_calls, mask_features, mask, call_stride,
-                          at<void>(workspace, ws.tcws), (cudaStream_t)stream);
-  if (st != CGG_OK) return fail(h, st, std::string("tc_mask_einsum: ") + tc_last_error(h->tc));
+  TC(h->tc, tc_mask_einsum(h->tc, batch, first_call, num_calls, mask_features, mask, call_stride,
+                           at<void>(workspace, ws.tcws), (cudaStream_t)stream));
   return CGG_OK;
 }
 
@@ -416,8 +412,7 @@ extern "C" int cgg_masked_attention(cgg_handle* h, int batch, int num_keys, cons
   if (batch <= 0 || num_keys <= 0) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   if (h->cfg.precision == CGG_BF16) {
-    int st = tc_attention(h->tc, batch, num_keys, q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, s);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_attention: ") + tc_last_error(h->tc));
+    TC(h->tc, tc_attention(h->tc, batch, num_keys, q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, s));
     return CGG_OK;
   }
   CU(launch_attention_f32(q, k, v, false, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, batch,
@@ -452,9 +447,8 @@ static int decoder_layer_impl(cgg_handle* h, const cgg_weights* w, int batch, in
   if (c.precision == CGG_BF16) {
     const long kvs = (long)n * 2 * C, kvb = (long)K * kvs;
     const __nv_bfloat16* kv = at<__nv_bfloat16>(workspace, ws.kv[l]);
-    int st = tc_decoder_layer(h->tc, w, batch, layer, x_in, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kvs, kvb, K,
-                              bitmap, all_masked, x_out, at<void>(workspace, ws.tcws), s, chained_in, chained_out, q_ready);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_decoder_layer: ") + tc_last_error(h->tc));
+    TC(h->tc, tc_decoder_layer(h->tc, w, batch, layer, x_in, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kvs, kvb, K,
+                               bitmap, all_masked, x_out, at<void>(workspace, ws.tcws), s, chained_in, chained_out, q_ready));
     return CGG_OK;
   }
   const cgg_layer_weights& lw = w->layers[layer];
@@ -470,15 +464,9 @@ static int decoder_layer_impl(cgg_handle* h, const cgg_weights* w, int batch, in
   // ---- masked cross-attention (K5): q = ((x + query_embed) Wq^T + bq) / sqrt(d)
   ST(linear_rows(h, s, x_in, w->query_embed, Q, lw.cross_in_w, lw.cross_in_b, qb, rows, C, C, qscale));
   const long kv_stride = (long)n * 2 * C, kv_bstride = (long)K * kv_stride;
-  if (c.precision == CGG_BF16) {
-    const __nv_bfloat16* kv = at<__nv_bfloat16>(workspace, ws.kv[l]);
-    ST(cgg_masked_attention(h, batch, K, qb, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kv_stride, kv_bstride,
-                            bitmap, all_masked, o, stream));
-  } else {
-    const float* kv = at<float>(workspace, ws.kv[l]);
-    ST(cgg_masked_attention(h, batch, K, qb, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kv_stride, kv_bstride,
-                            bitmap, all_masked, o, stream));
-  }
+  const float* kv = at<float>(workspace, ws.kv[l]);
+  ST(cgg_masked_attention(h, batch, K, qb, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kv_stride, kv_bstride,
+                          bitmap, all_masked, o, stream));
   ST(linear_rows(h, s, o, nullptr, 1, lw.cross_out_w, lw.cross_out_b, t, rows, C, C, 1.f, x_in));
   CU(launch_layernorm(t, nullptr, lw.norm_w[0], lw.norm_b[0], x1, rows, C, 1e-5f, true, s));
   // ---- self-attention (K6): q = k-input = x1 + query_embed, v-input = x1
@@ -534,10 +522,7 @@ extern "C" int cgg_decoder_forward(cgg_handle* h, const cgg_weights* w, int batc
   } else {
     ST(cgg_kv_project(h, w, batch, memories, workspace, workspace_bytes, stream));
   }
-  if (tcm) {
-    int st = tc_downsample(h->tc, batch, mask_features, tws, s);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_downsample: ") + tc_last_error(h->tc));
-  }
+  if (tcm) TC(h->tc, tc_downsample(h->tc, batch, mask_features, tws, s));
   CU(launch_broadcast_rows(w->query_feat, xs, batch, Q, C, s));          // head.py:808-809
   for (int j = 0; j <= L; ++j) {
     const bool need_mask = j < L;                                           // the last mask is never used
@@ -546,8 +531,7 @@ extern "C" int cgg_decoder_forward(cgg_handle* h, const cgg_weights* w, int batc
     if (q_par) {
       CU(cudaEventRecord(h->ev_me[j], s));
       CU(cudaStreamWaitEvent(h->side[1], h->ev_me[j], 0));
-      int st = tc_layer_qproj(h->tc, w, batch, j, tws, h->side[1]);
-      if (st != CGG_OK) return fail(h, st, std::string("tc_layer_qproj: ") + tc_last_error(h->tc));
+      TC(h->tc, tc_layer_qproj(h->tc, w, batch, j, tws, h->side[1]));
       CU(cudaEventRecord(h->ev_join[1], h->side[1]));
     }
     uint32_t* bm = need_mask ? ((bitmaps && bitmaps[j]) ? bitmaps[j] : at<uint32_t>(workspace, ws.bitmap)) : nullptr;
@@ -567,12 +551,10 @@ extern "C" int cgg_decoder_forward(cgg_handle* h, const cgg_weights* w, int batc
   }
   if (tcm && h->final_mask_only) {
     // inference shortcut: the last head call's logits only, into a (B,Q,H4,W4) buffer
-    int st = tc_mask_einsum(h->tc, batch, L, 1, mask_features, mask, (long)batch * Q * HW, tws, s);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_mask_einsum: ") + tc_last_error(h->tc));
+    TC(h->tc, tc_mask_einsum(h->tc, batch, L, 1, mask_features, mask, (long)batch * Q * HW, tws, s));
   } else if (tcm) {
     // K2 of all L+1 head calls in one pass over mask_features
-    int st = tc_mask_einsum(h->tc, batch, 0, L + 1, mask_features, mask, (long)batch * Q * HW, tws, s);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_mask_einsum: ") + tc_last_error(h->tc));
+    TC(h->tc, tc_mask_einsum(h->tc, batch, 0, L + 1, mask_features, mask, (long)batch * Q * HW, tws, s));
   }
   return CGG_OK;
 }
@@ -605,12 +587,6 @@ namespace {
 
 inline int round_up_i(int x, int m) { return (x + m - 1) / m * m; }
 
-// CGG_K7_SIMT=1: the fp32 SIMT similarity of round 1 (one dot product per (token, query) inside the pair kernel)
-bool k7_tensor_cores() {
-  static const bool simt = getenv("CGG_K7_SIMT") != nullptr && atoi(getenv("CGG_K7_SIMT")) != 0;
-  return !simt;
-}
-
 template <typename T>
 int grow(cgg_handle* h, T** p, size_t* have, size_t want_elems, cudaStream_t s, bool zero) {
   if (*have >= want_elems) return CGG_OK;
@@ -642,8 +618,7 @@ int k7_similarity(cgg_handle* h, const float* pred, const float* cap, int Bg, in
   CU(launch_cast_bf16_split(cap, h->k7.cap_hl, rows_c, D, s));
   TcSeg sg = {};
   sg.col0 = 0; sg.ncols = rows_p; sg.ptr = h->k7.S; sg.ld = rows_p; sg.alpha = 1.0f / temperature; sg.rb_mod = 1;
-  int st = tc_linear(t, h->k7.cap_hl, rows_c, D, h->k7.pred_hl, np, nullptr, &sg, 1, s, /*split_k=*/true);
-  if (st != CGG_OK) return fail(h, st, std::string("tc_linear (grounding similarity): ") + tc_last_error(t));
+  TC(t, tc_linear(t, h->k7.cap_hl, rows_c, D, h->k7.pred_hl, np, nullptr, &sg, 1, s, /*split_k=*/true));
   return CGG_OK;
 }
 
@@ -665,7 +640,7 @@ extern "C" int cgg_grounding_loss(cgg_handle* h, const float* pred, const float*
   float* g1 = static_cast<float*>(scratch);
   float* g2 = g1 + (size_t)Bg * Bg;
   const float* S_pre = nullptr;
-  if (k7_tensor_cores() && D % 64 == 0) {
+  if (D % 64 == 0) {
     ST(k7_similarity(h, pred, cap, Bg, Q, T, D, temperature, s));
     S_pre = h->k7.S;
   }
@@ -694,7 +669,7 @@ extern "C" int cgg_grounding_loss_backward(cgg_handle* h, const float* pred, con
   float* d2 = d1 + (size_t)Bg * Bg;
   float* loss = d2 + (size_t)Bg * Bg;
   float* dS = loss + 1;
-  if (k7_tensor_cores() && D % 64 == 0) {
+  if (D % 64 == 0) {
     // tensor-core mode: S once (tcgen05), pair kernels on S, then dpred[(j,q), :] = sum_(i,t) dS[(j,q), (i,t)] cap[(i,t), :]
     // as a second split-precision tcgen05 GEMM (M = Bg*Q tokens, N = D, K = Bg*T padded to 64)
     ST(k7_similarity(h, pred, cap, Bg, Q, T, D, temperature, s));
@@ -709,8 +684,7 @@ extern "C" int cgg_grounding_loss_backward(cgg_handle* h, const float* pred, con
     TcState* t = h->tc ? h->tc : h->tc_aux;
     TcSeg sg = {};
     sg.col0 = 0; sg.ncols = D; sg.ptr = dpred; sg.ld = D; sg.alpha = 1.0f; sg.rb_mod = 1;
-    int st = tc_linear(t, h->k7.dst_hl, rows_p, Kp, h->k7.capT_hl, nd, nullptr, &sg, 1, s, /*split_k=*/true);
-    if (st != CGG_OK) return fail(h, st, std::string("tc_linear (grounding backward): ") + tc_last_error(t));
+    TC(t, tc_linear(t, h->k7.dst_hl, rows_p, Kp, h->k7.capT_hl, nd, nullptr, &sg, 1, s, /*split_k=*/true));
     return CGG_OK;
   }
   // recompute the pair distances, then d loss / d cost, d loss / d S, and dpred_j = sum_{i,t} dS[j][i][t][:]^T cap[i][t][:]

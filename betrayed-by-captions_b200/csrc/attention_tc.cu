@@ -18,7 +18,6 @@
 //   at the end), so the groups never synchronise per tile.
 // The MMA thread issues P V of tile j and Q K^T of tile j+3 back to back and commits ONCE: phase n of step[b] means
 // "S(3n+b) ready" and "P V(3(n-1)+b) done" (a tcgen05.commit costs the issuing thread several hundred cycles).
-#include <cstdio>
 #include <cuda_fp16.h>
 #include "kernels.h"
 #include "tc_ptx.cuh"
@@ -47,7 +46,6 @@ struct AttnP {
   const uint32_t* bitmap; const uint8_t* all_masked;
   const uint8_t* live;           // [image][query tile][key tile] from attention_live_kernel; nullptr: every tile live
   int Q, K, heads, W32, ntiles, nqt;
-  int trace;
   int has_r, r_col0, r_lo_off;   // key-bias table term: S += Q (R_hi + R_lo)^T, R columns r_col0 + head*32
   int out_hl;                    // out_bf16: 0 = bf16 rows of C, 1 = [hi(C) | lo(C)] bf16 pairs, 2 = IEEE half rows of C
 };
@@ -183,20 +181,6 @@ __device__ __forceinline__ float2 add2(float2 a, float2 b) {
 __device__ __forceinline__ void mbar_expect_tx_only(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(ptx::smem_u32(bar)), "r"(bytes) : "memory");
 }
-
-// Debug trace (build with -DCGG_AT_TRACING, run with CGG_AT_TRACE=<softmax warp>): SM clock stamps of live
-// tiles 16..23 of CTA (0,0).
-__device__ long long g_at_trace[64];
-#ifdef CGG_AT_TRACING
-#define AT_TRACE(ti, slot)                                                                                   \
-  do {                                                                                                       \
-    if (p.trace && blockIdx.x == 0 && blockIdx.y == 0 && (ti) >= 16 && (ti) < 24) g_at_trace[((ti) - 16) * 8 + (slot)] = clock64(); \
-  } while (0)
-#define AT_TRACE_W(ti, slot) do { if (warp == p.trace && lane == 0) AT_TRACE(ti, slot); } while (0)
-#else
-#define AT_TRACE(ti, slot) do { } while (0)
-#define AT_TRACE_W(ti, slot) do { } while (0)
-#endif
 
 // D[tmem] (+)= A[tmem] * B[smem desc]: the A operand (M = 128 rows on the TMEM lanes, K-major, two bf16 per column)
 // comes from tensor memory
@@ -405,10 +389,8 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
     for (int j = 0; j < n_live; ++j) {
       const int s = j % AT_STAGES;
       ptx::mbar_wait(&p_full[j % 3], (uint32_t)(j / 3) & 1u);
-      if (lane == 0) AT_TRACE(j, 0);
       if (j + 3 < n_live) wait_kv(j + 3);
       ptx::tc_fence_after();
-      if (lane == 0) AT_TRACE(j, 1);
       if (ptx::elect_one()) {
         const uint64_t vd = vd0 + (uint64_t)(s * (AT_STAGE_BYTES >> 4));
         const uint32_t pa = tmem_S + (uint32_t)((j % 3) * 128);
@@ -426,7 +408,6 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
         ptx::mma_commit(&step[j % 3]);
       }
       __syncwarp();
-      if (lane == 0) AT_TRACE(j, 2);
     }
   } else {
     // ------------- softmax: thread = query row x key quarter cq of every tile
@@ -446,11 +427,9 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
       const uint32_t mw = mrow[s * (AT_MASK_BYTES / 4)];
       ptx::mbar_wait(&step[buf], (uint32_t)(it / 3) & 1u);               // S(it) ready (and P.V(it-3) done)
       ptx::tc_fence_after();
-      AT_TRACE_W(it, 3);
       uint32_t sv[32];
       tmem_ld32_issue(tmem_S + (uint32_t)(buf * 128 + cq * 32) + lane_off, sv);
       tmem_ld32_wait(sv);
-      AT_TRACE_W(it, 4);
       float v[32];
 #pragma unroll
       for (int i = 0; i < 32; ++i) v[i] = ((mw >> i) & 1u) ? -INFINITY : __uint_as_float(sv[i]);
@@ -484,7 +463,6 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
         l_run *= sc;
       }
       if (move) m_ref = mx;
-      AT_TRACE_W(it, 5);
       const float mneg = (m_ref == -INFINITY) ? 0.f : -m_ref;
       // p = exp2(s * log2e - m_ref) as bf16 pairs straight into the TMEM P tile of this buffer; the row sum adds the
       // fp32 values as a tree of packed pairs
@@ -504,11 +482,9 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
 #pragma unroll
         for (int j = 0; j < n; ++j) e[j] = add2(e[j], e[j + n]);
       l_run += e[0].x + e[0].y;
-      AT_TRACE_W(it, 6);
       tmem_st16_wait(pk);
       ptx::tc_fence_before();
       ptx::mbar_arrive(&p_full[buf]);
-      AT_TRACE_W(it, 7);
       // hand the previous tile's K/V stage back once its P.V has completed (long done by now)
       if (it > 0 && warp == 2) {
         ptx::mbar_wait(&step[(it - 1) % 3], (uint32_t)(((it - 1) / 3) + 1) & 1u);
@@ -573,18 +549,20 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
 int make_map_kv(TcState* t, CUtensorMap* m, const void* base, int K, long kv_stride, long kv_bstride, int B, int C) {
   if ((kv_stride * 2) % 16 != 0 || (kv_bstride * 2) % 16 != 0 || (reinterpret_cast<uintptr_t>(base) & 15))
     return tc_fail(t, CGG_ERR_UNSUPPORTED, "K/V rows must be 16-byte aligned");
-  cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)K, (cuuint64_t)B};
-  cuuint64_t strides[2] = {(cuuint64_t)kv_stride * 2, (cuuint64_t)kv_bstride * 2};
-  cuuint32_t box[3] = {32, AT_KT, 1};
-  cuuint32_t es[3] = {1, 1, 1};
-  CUresult r = t->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(KV) failed: " + std::to_string((int)r));
+  const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)K, (cuuint64_t)B};
+  const cuuint64_t strides[2] = {(cuuint64_t)kv_stride * 2, (cuuint64_t)kv_bstride * 2};
+  const cuuint32_t box[3] = {32, AT_KT, 1};
+  if (!encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "KV", &t->err))
+    return CGG_ERR_CUDA;
   return CGG_OK;
 }
 
 }  // namespace
+
+cudaError_t tc_attention_setup() {
+  return cudaFuncSetAttribute(masked_attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AT_SMEM);
+}
 
 int tc_attention(TcState* t, int batch, int num_keys, const float* q, const void* k, const void* v, long kv_stride,
                  long kv_bstride, const uint32_t* bitmap, const uint8_t* all_masked, float* out, __nv_bfloat16* out_bf16,
@@ -600,14 +578,12 @@ int tc_attention(TcState* t, int batch, int num_keys, const float* q, const void
   if (st != CGG_OK) return st;
   CUtensorMap mR = mK;
   if (r_table) {
-    cuuint64_t dims[2] = {(cuuint64_t)r_cols, (cuuint64_t)num_keys};
-    cuuint64_t strides[1] = {(cuuint64_t)r_cols * 2};
-    cuuint32_t box[2] = {32, AT_KT};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = t->encode(&mR, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(r_table), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(R) failed: " + std::to_string((int)r));
+    const cuuint64_t dims[2] = {(cuuint64_t)r_cols, (cuuint64_t)num_keys};
+    const cuuint64_t strides[1] = {(cuuint64_t)r_cols * 2};
+    const cuuint32_t box[2] = {32, AT_KT};
+    if (!encode_tensor_map(&mR, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, r_table, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "R", &t->err))
+      return CGG_ERR_CUDA;
   }
   const int W32 = (num_keys + 31) / 32;
   AttnP p;
@@ -625,27 +601,9 @@ int tc_attention(TcState* t, int batch, int num_keys, const float* q, const void
     TCU(cudaGetLastError());
     p.live = t->live_buf;
   }
-  if (!t->attn_attr_set) {
-    TCU(cudaFuncSetAttribute(masked_attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AT_SMEM));
-    t->attn_attr_set = true;
-  }
-  static const bool trace = getenv("CGG_AT_TRACE") != nullptr;
-  p.trace = trace ? atoi(getenv("CGG_AT_TRACE")) : 0;
   TCU(launch_pdl(masked_attention_tc_kernel, dim3(heads * nqt, batch), dim3(AT_THREADS), AT_SMEM, s, mK, mV, mR, p));
   count_launch();
   TCU(cudaGetLastError());
-  if (trace && ntiles >= 24) {
-    cudaStreamSynchronize(s);
-    long long tr[64];
-    cudaMemcpyFromSymbol(tr, g_at_trace, sizeof(tr));
-    fprintf(stderr, "[attention trace] K=%d cycles rel. to tile 16: mma(P ready, K/V(j+3) ready, PV+QK(j+3) committed) "
-                    "softmax(mask read, S loaded, rescaled, P issued, P arrived)\n", num_keys);
-    for (int i = 0; i < 8; ++i) {
-      fprintf(stderr, "  j=%d:", 16 + i);
-      for (int j = 0; j < 8; ++j) fprintf(stderr, " %7lld", tr[i * 8 + j] - tr[0]);
-      fprintf(stderr, "\n");
-    }
-  }
   return CGG_OK;
 }
 

@@ -24,8 +24,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <string>
-#include <stdio.h>
-#include <stdlib.h>
 
 namespace cgg {
 
@@ -56,7 +54,6 @@ struct TcGemmP {
   int acc_stride;        // TMEM columns between the two accumulator buffers
   int tmem_cols;         // power of two >= 32
   int epi;
-  int dbg;
   int f16;               // 1: operands are IEEE half instead of bf16 (attention-mask GEMM)
   int ein_split, q_rows; // transposed einsum: 0 = two head calls per step (q_rows = q_pad rows each CTA), 1 = one call per step, CTA r takes rows [r q_rows, (r+1) q_rows)
   int M_valid;           // valid pixels / keys per batch image (features for EPI_LINEAR_T)
@@ -88,19 +85,11 @@ __device__ __forceinline__ uint32_t pack2(__nv_bfloat16 a, __nv_bfloat16 b) {
   return (uint32_t)__bfloat16_as_ushort(a) | ((uint32_t)__bfloat16_as_ushort(b) << 16);
 }
 
-
-// Debug trace (CGG_TC_TIMING=1): SM clock stamps of N tiles 16..23 of CTA 0 of the pair kernel.
-__device__ long long g_tc_trace[64];
-#define TC_TRACE(gi, slot)                                                                         \
-  do {                                                                                             \
-    if ((p.dbg & 1) && blockIdx.x == 0 && (gi) >= 16 && (gi) < 24) g_tc_trace[((gi) - 16) * 8 + (slot)] = clock64(); \
-  } while (0)
-
 constexpr int EPI_WARPS = 16;                 // epilogue warps (4 per TMEM lane quarter)
 constexpr int EPI_PARTS = EPI_WARPS / 4;
 
 struct EpiCtx {
-  int lane, m, batch, part, chunks, wi, col0, g = -1;
+  int lane, m, batch, part, chunks, wi, col0;
   bool m_ok;
   uint32_t taddr;
 };
@@ -137,7 +126,6 @@ __device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, ui
   // 3. the previous tile's stores must have finished READING the staging buffer
   if (leader) ptx::tma_store_wait_read();
   asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
-  if (leader) TC_TRACE(c.g, 6);
   const int row = c.m & (TC_BM - 1);
   auto stage16 = [&](const uint32_t (&r)[16], int ch) {
     __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(sStage) + (long)(ch * 16) * TC_BM + row;
@@ -148,7 +136,6 @@ __device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, ui
   if (on1) stage16(r1, ch1);
   if (on2) stage16(r2, ch2);
   if (on3) stage16(r3, ch3);
-  if (leader) TC_TRACE(c.g, 7);
   ptx::fence_proxy_async_smem();
   asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
   if (leader) {
@@ -391,13 +378,6 @@ __device__ __forceinline__ void epi_linear_dispatch(const TcGemmP& p, const EpiC
   }
 }
 
-// Debug timeline (CGG_TC_TIMING=1): globaltimer stamps of CTA (0,0), printed by launch_tc_gemm.
-__device__ unsigned long long g_tc_stamps[16];
-#define TC_STAMP(i)                                                            \
-  do {                                                                         \
-    if ((p.dbg & 1) && blockIdx.x == 0 && blockIdx.y == 0) g_tc_stamps[i] = ptx::global_timer_ns(); \
-  } while (0)
-
 // Specialised per epilogue kind: the operand layout / residency follow from it at compile time
 //   EPI_MASK_T, EPI_ROWMAJOR : A = NCHW feature map, tile resident in smem for all N tiles
 //   EPI_BITS                 : A = NCHW (hi/lo planes), streamed with B
@@ -437,7 +417,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (A_RESIDENT) { batch = w / p.m_tiles; m_tile = w - batch * p.m_tiles; }
     else { m_tile = blockIdx.x; batch = blockIdx.y; }
   };
-  if (threadIdx.x == 0) TC_STAMP(0);
   // K coordinates of chunk kc in the A and B tensor maps
   auto kcoords = [&](int kc, int& ka, int& kb) {
     if (p.split_cpc > 0) {
@@ -468,7 +447,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   __syncthreads();
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) TC_STAMP(1);
   // everything above (barriers, TMEM, descriptor prefetch) overlapped the previous kernel's tail
   ptx::grid_dep_launch();
   // Linear layers: the A operand is a WEIGHT matrix, independent of the previous kernel -- its first ring-full of
@@ -560,7 +538,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (A_RESIDENT && t == 0) ptx::mbar_wait(&a_full[kc], (uint32_t)(tl & 1));
           ptx::mbar_wait(&b_full[s], ph);
           ptx::tc_fence_after();
-          if (it == 0 && lane == 0) TC_STAMP(2);
           if (ptx::elect_one()) {
             const uint64_t ad = ad0 + (uint64_t)(A_RESIDENT ? (uint32_t)kc * (A_CHUNK_BYTES >> 4) : (uint32_t)s * stage16);
             const uint64_t bd = bd0 + (uint64_t)((uint32_t)s * stage16);
@@ -573,7 +550,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
           __syncwarp();
         }
-        if (g == 0 && lane == 0) TC_STAMP(3);
       }
   } else {
     // ---------------- epilogue: EPI_WARPS warps, EPI_WARPS/4 per TMEM lane quarter; each warp takes
@@ -606,7 +582,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const uint32_t use = (uint32_t)(g >> 1);
       ptx::mbar_wait(&acc_full[buf], use & 1u);
       ptx::tc_fence_after();
-      if (g == 0 && warp == 2 && lane == 0) TC_STAMP(4);
       ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
       ctx.col0 = t * p.N_TILE;
       const bool last = last_work && t == p.NT - 1;
@@ -619,13 +594,11 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
       }
-      if (last && warp == 2 && lane == 0) TC_STAMP(5);
     }
     }
   }
   ptx::tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) TC_STAMP(6);
   if (warp == 1) {
     __syncwarp();
     ptx::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
@@ -732,14 +705,12 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
           const uint32_t use = (uint32_t)(g >> 1);
           ptx::mbar_wait(&acc_empty[buf], (use & 1u) ^ 1u);
           ptx::tc_fence_after();
-          if (lane == 0) TC_TRACE(g, 0);
           const uint32_t d_tmem = tmem_base + (uint32_t)(buf * p.acc_stride);
 #pragma unroll
           for (int kc = 0; kc < KC; ++kc) {
             if (t == 0) ptx::mbar_wait(&a_full[kc], (uint32_t)(tl & 1));
             ptx::mbar_wait(&b_full[buf * KC + kc], use & 1u);
             ptx::tc_fence_after();
-            if (kc == 0 && lane == 0) TC_TRACE(g, 1);
             if (ptx::elect_one()) {
               const uint64_t ad = adesc0[kc], bd = buf ? bdesc0[KC + kc] : bdesc0[kc];
 #pragma unroll
@@ -751,7 +722,6 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
             }
             __syncwarp();
           }
-          if (lane == 0) TC_TRACE(g, 2);
         }
     }
   } else {
@@ -771,11 +741,9 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
         const uint32_t use = (uint32_t)(g >> 1);
         ptx::mbar_wait(&acc_full[buf], use & 1u);
         ptx::tc_fence_after();
-        if (warp == 2 && lane == 0) TC_TRACE(g, 3);
         ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
-        ctx.col0 = t * p.N_TILE; ctx.g = g;
+        ctx.col0 = t * p.N_TILE;
         epi_mask_t(p, ctx, sStage, &tmC, warp == 2, last_work && t == p.NT - 1, m_tile, &acc_empty[buf], true);
-        if (warp == 2 && lane == 0) TC_TRACE(g, 4);
       }
     }
   }
@@ -1357,32 +1325,30 @@ int make_map_A(TcState* t, CUtensorMap* m, const void* base, int pixels, int C, 
   if (pitch < 0) pitch = pixels;
   if ((pitch * 2) % 16 != 0 || (reinterpret_cast<uintptr_t>(base) & 15))
     return tc_fail(t, CGG_ERR_UNSUPPORTED, "TMA needs 16-byte aligned channel planes (pixel pitch multiple of 8)");
-  cuuint64_t dims[3] = {(cuuint64_t)pixels, (cuuint64_t)C, (cuuint64_t)B};
-  cuuint64_t strides[2] = {(cuuint64_t)pitch * 2, (cuuint64_t)pitch * C * 2};
-  cuuint32_t box[3] = {64, 64, 1};
-  cuuint32_t es[3] = {1, 1, 1};
-  CUresult r = t->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(A) failed: " + std::to_string((int)r));
+  const cuuint64_t dims[3] = {(cuuint64_t)pixels, (cuuint64_t)C, (cuuint64_t)B};
+  const cuuint64_t strides[2] = {(cuuint64_t)pitch * 2, (cuuint64_t)pitch * C * 2};
+  const cuuint32_t box[3] = {64, 64, 1};
+  if (!encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "A", &t->err))
+    return CGG_ERR_CUDA;
   return CGG_OK;
 }
 // 2-D map over a K-major [rows][C] bf16 matrix: box (64 k, n_tile rows)
 int make_map_B(TcState* t, CUtensorMap* m, const void* base, long rows, int C, int n_tile) {
   // C = row length in elements (pitch == length)
-  cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)C * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)n_tile};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = t->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(B) failed: " + std::to_string((int)r));
+  const cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)C * 2};
+  const cuuint32_t box[2] = {64, (cuuint32_t)n_tile};
+  if (!encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "B", &t->err))
+    return CGG_ERR_CUDA;
   return CGG_OK;
 }
 
+// cta_cap > 0: the persistent (A-resident) kinds run on at most that many CTAs, leaving SMs to a concurrent
+// latency-bound chain
 int launch_tc_gemm(TcState* t, const CUtensorMap& mA, const CUtensorMap& mB, TcGemmP p, int m_tiles, int batch,
-                   cudaStream_t s, const CUtensorMap* mC = nullptr, int kparts = 1) {
+                   cudaStream_t s, const CUtensorMap* mC = nullptr, int kparts = 1, int cta_cap = 0) {
   if (p.N_TILE % 16 != 0 || p.N_TILE < 16 || p.N_TILE > 256) return tc_fail(t, CGG_ERR_BAD_SHAPE, "bad N tile");
   p.acc_stride = p.N_TILE <= 128 ? 128 : 256;
   if (p.N_TILE <= 32) p.acc_stride = 32; else if (p.N_TILE <= 64) p.acc_stride = 64;
@@ -1399,34 +1365,17 @@ int launch_tc_gemm(TcState* t, const CUtensorMap& mA, const CUtensorMap& mB, TcG
   if (stages < 2) return tc_fail(t, CGG_ERR_BAD_SHAPE, "tile does not fit shared memory");
   p.stages = stages;
   const size_t smem = 1024 + a_bytes + stages * b_stage + (8 + 2 * stages + 4) * 8 + 64 + stage_bytes;
-  if (!t->smem_attr_set) {
-    TCU(cudaFuncSetAttribute(tc_gemm_kernel<EPI_MASK_T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    TCU(cudaFuncSetAttribute(tc_gemm_kernel<EPI_ROWMAJOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    TCU(cudaFuncSetAttribute(tc_gemm_kernel<EPI_BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    TCU(cudaFuncSetAttribute(tc_gemm_kernel<EPI_LINEAR_T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    t->smem_attr_set = true;
-  }
   // the kernel instantiation fixes the A-operand layout / residency: check the caller agrees
   const bool want_res = (p.epi == EPI_MASK_T || p.epi == EPI_ROWMAJOR), want_km = (p.epi == EPI_LINEAR_T);
   if (want_res && p.KC > 4) return tc_fail(t, CGG_ERR_BAD_SHAPE, "resident A tile limited to 4 K chunks");
   if ((p.a_resident != 0) != want_res || (p.a_kmajor != 0) != want_km)
     return tc_fail(t, CGG_ERR_BAD_SHAPE, "operand layout does not match the kernel specialisation");
-  static const bool timing = getenv("CGG_TC_TIMING") != nullptr;
-  p.dbg = timing ? 1 : 0;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timing) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaStreamSynchronize(s); cudaEventRecord(e0, s); }
   dim3 grid(m_tiles, batch, kparts);
   const dim3 block(TC_THREADS);
   p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
   if (want_res) {
-    const int persist = 1;
-    if (t->num_sms == 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-    int ctas = persist ? (p.n_work < t->num_sms ? p.n_work : t->num_sms) : p.n_work;
-    if (persist && t->cta_cap > 0 && ctas > t->cta_cap) ctas = t->cta_cap;   // leave SMs to a concurrent latency-bound chain
+    int ctas = p.n_work < t->num_sms ? p.n_work : t->num_sms;
+    if (cta_cap > 0 && ctas > cta_cap) ctas = cta_cap;
     grid = dim3(ctas, 1, 1);
   }
   const CUtensorMap& mCC = mC ? *mC : mB;
@@ -1438,19 +1387,6 @@ int launch_tc_gemm(TcState* t, const CUtensorMap& mA, const CUtensorMap& mB, TcG
   }
   count_launch();
   TCU(cudaGetLastError());
-  if (timing) {
-    cudaEventRecord(e1, s);
-    cudaStreamSynchronize(s);
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
-    unsigned long long st[16];
-    cudaMemcpyFromSymbol(st, g_tc_stamps, sizeof(st));
-    fprintf(stderr, "[tc_gemm] grid %dx%d epi %d NT %d KC %d N_TILE %d stages %d smem %zu: event %.1f us | setup %.1f first-data %.1f mma-issued %.1f "
-            "acc-ready %.1f epi-done %.1f teardown %.1f (us since entry)\n", m_tiles, batch, p.epi, p.NT, p.KC, p.N_TILE, p.stages, smem,
-            ms * 1e3, (st[1] - st[0]) * 1e-3, (st[2] - st[0]) * 1e-3, (st[3] - st[0]) * 1e-3, (st[4] - st[0]) * 1e-3,
-            (st[5] - st[0]) * 1e-3, (st[6] - st[0]) * 1e-3);
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
-  }
   return CGG_OK;
 }
 
@@ -1461,13 +1397,20 @@ TcState* tc_create(const cgg_config& cfg) {
   TcState* t = new (std::nothrow) TcState();
   if (!t) return nullptr;
   t->cfg = cfg;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) {
+  // the SM count and the kernels' shared-memory limit belong to the device: a handle lives on the one it is created on
+  int dev = 0;
+  const auto max_smem = [](auto kernel) {
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) == cudaSuccess;
+  };
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
+      !max_smem(tc_gemm_kernel<EPI_MASK_T>) || !max_smem(tc_gemm_kernel<EPI_ROWMAJOR>) ||
+      !max_smem(tc_gemm_kernel<EPI_BITS>) || !max_smem(tc_gemm_kernel<EPI_LINEAR_T>) || !max_smem(tc_kv_pair_kernel) ||
+      !max_smem(tc_bits_kernel) || !max_smem(tc_einsum_t_kernel) || !max_smem(tc_einsum_pair_kernel) ||
+      tc_attention_setup() != cudaSuccess) {
     delete t;
     return nullptr;
   }
-  t->encode = reinterpret_cast<EncodeTiledFn>(fn);
   const int Q = cfg.num_queries, calls = cfg.num_layers + 1;
   // N tiling: two head calls per 2*round8(Q)-wide tile when that fits one MMA (Q=100 -> 208, 4% pad);
   // otherwise one call per round16(Q) tile; above 256 queries, two tiles per call.
@@ -1586,14 +1529,12 @@ int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* 
   if (p.N_TILE % 64 != 0) return tc_fail(t, CGG_ERR_BAD_SHAPE, "K/V tile width must be a multiple of 64");
   CUtensorMap mC;
   {
-    cuuint64_t dims[3] = {(cuuint64_t)N, (cuuint64_t)K, (cuuint64_t)batch};
-    cuuint64_t strides[2] = {(cuuint64_t)N * 2, (cuuint64_t)K * N * 2};
-    cuuint32_t box[3] = {64, (cuuint32_t)TC_BM, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = t->encode(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, kv_bf16, dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(kv out) failed: " + std::to_string((int)r));
+    const cuuint64_t dims[3] = {(cuuint64_t)N, (cuuint64_t)K, (cuuint64_t)batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)N * 2, (cuuint64_t)K * N * 2};
+    const cuuint32_t box[3] = {64, (cuuint32_t)TC_BM, 1};
+    if (!encode_tensor_map(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, kv_bf16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_NONE, "kv out", &t->err))
+      return CGG_ERR_CUDA;
   }
   const int m_tiles = (K + TC_BM - 1) / TC_BM;
   if (m_tiles % 2 == 0 && K % TC_BM == 0 && p.KC == 4) {
@@ -1609,15 +1550,6 @@ int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* 
     if (stages >= 3) {
       p.stages = stages;
       const size_t smem = 1024 + 4 * A_CHUNK_BYTES + stages * b_stage + stage_bytes + bias_bytes + (8 + 2 * stages + 4) * 8 + 64;
-      if (!t->attr_kv_pair) {      // per handle = per device (the attribute is per device, not per process)
-        TCU(cudaFuncSetAttribute(tc_kv_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        t->attr_kv_pair = true;
-      }
-      if (t->num_sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev);
-      }
       int pairs = t->num_sms / 2;
       if (cta_cap > 0 && pairs > cta_cap / 2) pairs = cta_cap / 2;
       if (pairs > p.n_work / 2) pairs = p.n_work / 2;
@@ -1627,10 +1559,7 @@ int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* 
       return CGG_OK;
     }
   }
-  t->cta_cap = cta_cap;
-  st = launch_tc_gemm(t, mA, mB, p, m_tiles, batch, s, &mC);
-  t->cta_cap = 0;
-  return st;
+  return launch_tc_gemm(t, mA, mB, p, m_tiles, batch, s, &mC, 1, cta_cap);
 }
 
 int tc_downsample(TcState* t, int batch, const void* mask_features_bf16, void* ws, cudaStream_t s) {
@@ -1690,17 +1619,7 @@ int tc_mask_bits(TcState* t, int batch, int call_idx, int level, uint32_t* bitma
     // (blockIdx.y = image) -> the kernel needs the per-image row: pass through b_row and rows_per_batch
     bp.b_row = call_idx * t->q_pad;
     const size_t smem = 1024 + 4 * (size_t)bp.N_TILE * 128 + (size_t)bp.stages * 2 * A_CHUNK_BYTES + (1 + 2 * bp.stages + 4) * 8 + 64;
-    if (!t->attr_bits) {
-      TCU(cudaFuncSetAttribute(tc_bits_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-      t->attr_bits = true;
-    }
-    if (t->num_sms == 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-    const int sms = t->num_sms;
-    int gx = sms / batch;
+    int gx = t->num_sms / batch;
     if (gx < 1) gx = 1;
     if (gx > bp.m_tiles) gx = bp.m_tiles;
     bp.m_tiles = bp.m_tiles;
@@ -1708,14 +1627,12 @@ int tc_mask_bits(TcState* t, int batch, int call_idx, int level, uint32_t* bitma
     // would need one map per image) -> use a 3-D map (k, row-in-image, image)
     CUtensorMap mB3;
     {
-      cuuint64_t dims[3] = {(cuuint64_t)(2 * C), (cuuint64_t)t->rows_per_batch, (cuuint64_t)batch};
-      cuuint64_t strides[2] = {(cuuint64_t)(2 * C) * 2, (cuuint64_t)t->rows_per_batch * (2 * C) * 2};
-      cuuint32_t box[3] = {64, (cuuint32_t)bp.N_TILE, 1};
-      cuuint32_t es[3] = {1, 1, 1};
-      CUresult r = t->encode(&mB3, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base + w.me_all, dims, strides, box, es,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(me) failed: " + std::to_string((int)r));
+      const cuuint64_t dims[3] = {(cuuint64_t)(2 * C), (cuuint64_t)t->rows_per_batch, (cuuint64_t)batch};
+      const cuuint64_t strides[2] = {(cuuint64_t)(2 * C) * 2, (cuuint64_t)t->rows_per_batch * (2 * C) * 2};
+      const cuuint32_t box[3] = {64, (cuuint32_t)bp.N_TILE, 1};
+      if (!encode_tensor_map(&mB3, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base + w.me_all, dims, strides, box,
+                             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "me", &t->err))
+        return CGG_ERR_CUDA;
     }
     TCU(launch_pdl(tc_bits_kernel, dim3(gx, batch), dim3(TC_THREADS), smem, s, mA, mB3, bp));
     count_launch();
@@ -1788,14 +1705,12 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
     return tc_fail(t, CGG_ERR_BAD_SHAPE, "mask outputs of consecutive head calls must be contiguous");
   CUtensorMap mC;
   {
-    cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
-    cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
-    cuuint32_t box[3] = {(cuuint32_t)TC_BM, (cuuint32_t)(t->q_pad < p.N_TILE ? t->q_pad : p.N_TILE), 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = t->encode(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(mask out) failed: " + std::to_string((int)r));
+    const cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
+    const cuuint32_t box[3] = {(cuuint32_t)TC_BM, (cuuint32_t)(t->q_pad < p.N_TILE ? t->q_pad : p.N_TILE), 1};
+    if (!encode_tensor_map(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                           CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out", &t->err))
+      return CGG_ERR_CUDA;
   }
   const int m_tiles = (int)((HW + TC_BM - 1) / TC_BM);
   const bool t_split = t->q_pad > 128;      // one head call per step, its rows split over the CTA pair (Q up to 256)
@@ -1809,26 +1724,15 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
       st = make_map_B(t, &mE, base + w.me_all, (long)batch * t->rows_per_batch + 128, 2 * C, t_rows);
       if (st != CGG_OK) return st;
       {
-        cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
-        cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
-        cuuint32_t box[3] = {64, (cuuint32_t)t_rows, 1};
-        cuuint32_t es[3] = {1, 1, 1};
-        CUresult r = t->encode(&mCt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box, es,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(mask out, swizzled) failed: " + std::to_string((int)r));
+        const cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
+        const cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
+        const cuuint32_t box[3] = {64, (cuuint32_t)t_rows, 1};
+        if (!encode_tensor_map(&mCt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box,
+                               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out, swizzled", &t->err))
+          return CGG_ERR_CUDA;
       }
       p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-      p.dbg = 0; p.ein_split = t_split ? 1 : 0; p.q_rows = t_rows;
-      if (!t->attr_ein_t) {
-        TCU(cudaFuncSetAttribute(tc_einsum_t_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        t->attr_ein_t = true;
-      }
-      if (t->num_sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev);
-      }
+      p.ein_split = t_split ? 1 : 0; p.q_rows = t_rows;
       int pairs = t->num_sms / 2;
       if (pairs > p.n_work / 2) pairs = p.n_work / 2;
       TCU(launch_pdl_cluster(2, tc_einsum_t_kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mE, mCt, p));
@@ -1844,38 +1748,16 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
     p.acc_stride = p.N_TILE <= 128 ? 128 : 256;
     p.tmem_cols = 2 * p.acc_stride;
     p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-    p.dbg = 0;
     const size_t stage_bytes = (size_t)p.N_TILE * TC_BM * 2 + 1024;
     const size_t b_chunk = (size_t)(p.N_TILE / 2) * 128;
     const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * b_chunk + 24 * 8 + 64 + stage_bytes;
     if (smem <= 227 * 1024) {
       p.stages = 8;
-      if (!t->attr_ein_pair) {
-        TCU(cudaFuncSetAttribute(tc_einsum_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        t->attr_ein_pair = true;
-      }
-      if (t->num_sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev);
-      }
       int pairs = t->num_sms / 2;
       if (pairs > p.n_work / 2) pairs = p.n_work / 2;
-      if (getenv("CGG_TC_TIMING")) p.dbg |= 1;
       TCU(launch_pdl_cluster(2, tc_einsum_pair_kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mB, mC, p));
       count_launch();
       TCU(cudaGetLastError());
-      if (p.dbg & 1) {
-        cudaStreamSynchronize(s);
-        long long tr[64];
-        cudaMemcpyFromSymbol(tr, g_tc_trace, sizeof(tr));
-        fprintf(stderr, "[pair einsum trace] cycles rel. to N-tile 16: mma(acc_empty ok, first B ok, committed) epi(acc_full ok, epi done, arrived) epi-inner(after bar1, after chunk loop)\n");
-        for (int i = 0; i < 8; ++i) {
-          fprintf(stderr, "  g=%d:", 16 + i);
-          for (int j = 0; j < 8; ++j) fprintf(stderr, " %7lld", tr[i * 8 + j] - tr[0]);
-          fprintf(stderr, "\n");
-        }
-      }
       return CGG_OK;
     }
   }
@@ -1887,14 +1769,12 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
 // flattened (image, query) pairs; 128 rows per CTA, N walked in tiles of <= 256.
 namespace {
 int make_map_act(TcState* t, CUtensorMap* m, const void* base, long rows, int K) {
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)K * 2};
-  cuuint32_t box[2] = {64, 128};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = t->encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return tc_fail(t, CGG_ERR_CUDA, "cuTensorMapEncodeTiled(act) failed: " + std::to_string((int)r));
+  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)K * 2};
+  const cuuint32_t box[2] = {64, 128};
+  if (!encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "act", &t->err))
+    return CGG_ERR_CUDA;
   return CGG_OK;
 }
 

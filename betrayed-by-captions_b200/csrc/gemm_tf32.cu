@@ -403,10 +403,6 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const Tf32P p) {
   *c = epi_value(p, acc, b, gm, gn) + (p.accumulate ? *c : 0.f);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // operand X[b, r, k] with element strides (sb, sr, sk): 0 = K-major, 1 = MN-major, -1 = TMA cannot describe it
@@ -424,29 +420,25 @@ int operand_major(const float* base, long sb, long sb2, long sr, long sk, int ro
 }  // namespace
 
 struct Tf32Ctx {
-  EncodeTiledFn encode = nullptr;
   // split-K partial sums: one buffer per workspace slot (GemmF32::slot) -- products issued on two streams at once (the
   // weight-gradient products run on a side stream) must not share one
   float* partial[2] = {nullptr, nullptr};
   size_t partial_bytes[2] = {0, 0};
   int sm_count = 148;
-  bool attr_set = false;
   std::string err;
 };
 
 Tf32Ctx* tf32_create() {
   Tf32Ctx* t = new (std::nothrow) Tf32Ctx();
   if (!t) return nullptr;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) {
-    delete t;
-    return nullptr;
-  }
-  t->encode = reinterpret_cast<EncodeTiledFn>(fn);
   int dev = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&t->sm_count, cudaDevAttrMultiProcessorCount, dev);
+  if (cudaFuncSetAttribute(gemm_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                           227 * 1024 - (EPI_WARPS > 4 ? 44 : 24) * 1024) != cudaSuccess) {
+    delete t;
+    return nullptr;
+  }
   return t;
 }
 void tf32_destroy(Tf32Ctx* t) {
@@ -459,7 +451,7 @@ const char* tf32_last_error(const Tf32Ctx* t) { return t ? t->err.c_str() : ""; 
 static int make_map(Tf32Ctx* t, CUtensorMap* m, const float* base, int major, long sb, long sb2, long sr, long sk, int rows,
                     int K, int batch, int batch_inner, int box_rows) {
   cuuint64_t dims[4], strides[3];
-  cuuint32_t box[4], es[4] = {1, 1, 1, 1};
+  cuuint32_t box[4];
   if (major == 0) {      // K-major: (k, row, batch), box (32 k, box_rows rows)
     dims[0] = (cuuint64_t)K; dims[1] = (cuuint64_t)rows;
     strides[0] = (cuuint64_t)(rows > 1 ? sr : ((K + 3) & ~3)) * 4;
@@ -475,12 +467,9 @@ static int make_map(Tf32Ctx* t, CUtensorMap* m, const float* base, int major, lo
   box[2] = box[3] = 1;
   strides[1] = batch_inner > 1 ? (cuuint64_t)sb2 * 4 : strides[0] * dims[1];
   strides[2] = outer > 1 ? (cuuint64_t)sb * 4 : strides[0] * dims[1];
-  CUresult r = t->encode(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         major == 0 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
-                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { t->err = "cuTensorMapEncodeTiled(tf32 operand) failed: " + std::to_string((int)r); return -1; }
-  return 0;
+  return encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, dims, strides, box,
+                           major == 0 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "tf32 operand", &t->err) ? 0 : -1;
 }
 
 // 0 = launched, 1 = not eligible (caller runs the SIMT kernel), < 0 = error (tf32_last_error)
@@ -553,13 +542,6 @@ int launch_gemm_tf32(Tf32Ctx* t, const GemmF32& g, cudaStream_t s) {
     p.epi_mode = 1;
   else if (g.sCm == 1 && (g.relu_from % 32 == 0 || g.relu_from >= g.N) && (!g.bias || al16(g.bias)) && (!g.bias || g.N % 4 == 0)) p.epi_mode = 2;
   else p.epi_mode = 0;
-  if (!t->attr_set) {
-    if (cudaFuncSetAttribute(gemm_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - (EPI_WARPS > 4 ? 44 : 24) * 1024) != cudaSuccess) {
-      t->err = "cudaFuncSetAttribute(gemm_tf32_kernel) failed";
-      return -1;
-    }
-    t->attr_set = true;
-  }
   const long total = mt * nt * g.batch * p.splits;
   gemm_tf32_kernel<<<(unsigned)(total < t->sm_count ? total : t->sm_count), THREADS, smem, s>>>(mA, mB, p);
   count_launch();

@@ -4,27 +4,23 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
+#include <string>
 #include <utility>
 
 namespace cgg {
 
 // Programmatic dependent launch: the kernel may start (and run its prologue) while the previous
 // kernel of the stream is still finishing; it must execute ptx::grid_dep_wait() before touching
-// anything the previous kernel produced or still reads.  CGG_NO_PDL=1 falls back to plain launches.
+// anything the previous kernel produced or still reads.
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl_cluster(int cluster_x, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
                                       cudaStream_t s, Args&&... args) {
-  static const bool off = getenv("CGG_NO_PDL") != nullptr;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
   cudaLaunchAttribute attr[2];
-  int n = 0;
-  if (!off) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  int n = 1;
   if (cluster_x > 1) {
     attr[n].id = cudaLaunchAttributeClusterDimension;
     attr[n].val.clusterDim.x = (unsigned)cluster_x; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = 1;
@@ -36,6 +32,30 @@ inline cudaError_t launch_pdl_cluster(int cluster_x, void (*kernel)(KArgs...), d
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
   return launch_pdl_cluster(1, kernel, grid, block, smem, s, std::forward<Args>(args)...);
+}
+
+// Every TMA tensor map of the project: cuTensorMapEncodeTiled with element strides 1, no interleave and no
+// out-of-bounds fill.  dims and box hold `rank` (2..4) entries, innermost first; byte_strides the rank-1 outer
+// ones.  On failure *err names the map (`what`) and the driver's result.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline bool encode_tensor_map(CUtensorMap* m, CUtensorMapDataType dtype, int rank, const void* base,
+                              const cuuint64_t* dims, const cuuint64_t* byte_strides, const cuuint32_t* box,
+                              CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* what, std::string* err) {
+  static const EncodeTiledFn encode = [] {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess;
+    return ok ? reinterpret_cast<EncodeTiledFn>(fn) : nullptr;
+  }();
+  const cuuint32_t es[4] = {1, 1, 1, 1};
+  const CUresult r = encode ? encode(m, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, byte_strides, box, es,
+                                     CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE)
+                            : CUDA_ERROR_NOT_FOUND;
+  if (r == CUDA_SUCCESS) return true;
+  *err = std::string("cuTensorMapEncodeTiled(") + what + ") failed: " + std::to_string((int)r);
+  return false;
 }
 
 namespace ptx {

@@ -7,16 +7,10 @@
 
 namespace cgg {
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-
 struct TcState {
   cgg_config cfg;
   std::string err;
-  EncodeTiledFn encode = nullptr;
-  int num_sms = 0, cta_cap = 0;
+  int num_sms = 0;
   int H4 = 0, W4 = 0, lh[3] = {0, 0, 0}, lw[3] = {0, 0, 0}, nl[3] = {0, 0, 0};
   __nv_bfloat16* wkv[3] = {nullptr, nullptr, nullptr};   // (nl*2C, C) bf16
   __nv_bfloat16* rk[3] = {nullptr, nullptr, nullptr};    // (K_l, nl*C) bf16 key-bias table
@@ -33,8 +27,6 @@ struct TcState {
   float* bias_h = nullptr;
   int nh_padded = 0;
   bool packed_alloc = false;
-  bool smem_attr_set = false, attn_attr_set = false;   // per-device kernel attributes set (one handle = one device)
-  bool attr_kv_pair = false, attr_bits = false, attr_ein_t = false, attr_ein_pair = false;
   uint8_t* live_buf = nullptr;          // per (image, query tile, key tile) "any key unmasked" flags
   size_t live_bytes = 0;
   void free_all() {
@@ -80,6 +72,7 @@ struct TcWs {
 };
 
 int tc_pack_weights(TcState* t, const cgg_weights* w, cudaStream_t s);   // path_bf16.cu
+cudaError_t tc_attention_setup();   // attention_tc.cu: kernel attributes, once per handle (per device)
 
 inline int tc_fail(TcState* t, int code, const std::string& m) { t->err = m; return code; }
 

@@ -217,24 +217,32 @@ def test_grounding_loss_matches_reference_golden(name):
     assert abs(float(loss) - float(O.grounding_loss(pred, cap, m, 10.0, 2.0))) < 1e-4 * max(1.0, abs(want))
 
 
-@pytest.mark.parametrize('name', list(cases.GROUNDING_CASES))
+@pytest.mark.parametrize('name', list(cases.GROUNDING_CASES) + ['b6_d100'])
 def test_grounding_loss_gradient_matches_reference_golden(name):
     """d loss / d cls_emb_pred from cgg_grounding_loss_backward against the gradients the unmodified reference
-    produced (tests/golden/make_golden.py: strided sample + abs-sum) and the oracle's autograd."""
+    produced (tests/golden/make_golden.py: strided sample + abs-sum) and the oracle's autograd.  b6_d100 is case b6
+    cut to D = 100: not a multiple of 64, so loss and gradient take the SIMT route instead of the tcgen05 GEMMs;
+    there is no golden file for that width, so it is checked against the oracle only (loss included)."""
     from cgg_b200.grounding import GroundingLossB200
     gold = np.load(os.path.join(GOLD, 'grounding.npz'))
-    pred, cap, m = cases.grounding_tensors(name)
+    pred, cap, m = cases.grounding_tensors(name.replace('_d100', ''))
+    if name.endswith('_d100'):
+        pred, cap = pred[..., :100].contiguous(), cap[..., :100].contiguous()
     p_dev = pred.to(DEV).requires_grad_(True)
     loss = GroundingLossB200(loss_weight=2.0)(p_dev, cap.to(DEV), m.to(DEV), 10.0)
     (loss * 1.0).backward()
     g = p_dev.grad.cpu()
     p_ref = pred.clone().requires_grad_(True)
-    O.grounding_loss(p_ref, cap, m, 10.0, 2.0).backward()
+    ref_loss = O.grounding_loss(p_ref, cap, m, 10.0, 2.0)
+    ref_loss.backward()
+    assert abs(float(loss) - float(ref_loss)) < 1e-4 * max(1.0, abs(float(ref_loss)))
     scale = float(p_ref.grad.abs().max())
     assert float((g - p_ref.grad).abs().max()) <= 2e-5 * scale
-    want = gold[name + '_grad_sample']
-    np.testing.assert_allclose(g.flatten()[::cases.GRAD_SAMPLE_STRIDE].numpy(), want, atol=2e-5 * scale, rtol=0)
-    assert abs(float(g.double().abs().sum()) - float(gold[name + '_grad_abssum'])) <= 1e-4 * float(gold[name + '_grad_abssum'])
+    if name in cases.GROUNDING_CASES:
+        want = gold[name + '_grad_sample']
+        np.testing.assert_allclose(g.flatten()[::cases.GRAD_SAMPLE_STRIDE].numpy(), want, atol=2e-5 * scale, rtol=0)
+        abssum = float(gold[name + '_grad_abssum'])
+        assert abs(float(g.double().abs().sum()) - abssum) <= 1e-4 * abssum
     # upstream scaling goes through
     p2 = pred.to(DEV).requires_grad_(True)
     (GroundingLossB200(loss_weight=2.0)(p2, cap.to(DEV), m.to(DEV), 10.0) * 0.25).backward()
