@@ -1,18 +1,15 @@
-// tcgen05 / TMEM / TMA GEMM of the throughput mode (CGG_BF16), sm_100a.
+// tcgen05 / TMEM / TMA GEMMs of the throughput mode (CGG_BF16), sm_100a.
 //
-// One kernel serves the three dense contractions whose big operand is an NCHW feature map:
+// Three dense contractions have an NCHW feature map as their big operand:
 //   K2  mask einsum      D[pixel, (call,q)] = sum_c F[c,pixel]      * me[(call,q), c]
 //   K3  attn-mask bits   D[key,   q]        = sum_c Fds_l[c,key]    * me[q, c]     -> sigmoid<0.5 -> ballot
-//   K4  K/V projection   D[key,   n]        = sum_c mem_l[c,key]    * Wkv[n, c]    (+ bias tables)
-// A (the feature map) is "MN-major": pixels contiguous, channels strided -- exactly NCHW -- so it is
-// fed to the tensor core as-is through TMA with a 128-byte swizzle, no transposition pass.
-// B (mask embeddings / weights) is K-major [rows][256].
-//
-// CTA = 128 pixels x all N.  The A tile (128 px x 256 ch bf16 = 64 KB) is loaded ONCE and stays in
-// shared memory while the CTA walks NT tiles of N (for K2: all 10 head calls, so mask_features is
-// read from HBM once per forward instead of once per call).  B tiles stream through a ring of TMA
-// stages; accumulators are double-buffered in TMEM so the epilogue warps drain tile t while the
-// single MMA-issuing thread runs tile t+1.
+//   K4  K/V projection   D[key,   n]        = sum_c mem_l[c,key]    * Wkv[n, c]    (+ bias)
+// The feature map is "MN-major": pixels contiguous, channels strided -- exactly NCHW -- so it is fed to the
+// tensor core as-is through TMA with a 128-byte swizzle, no transposition pass.  The other operand (mask
+// embeddings / weights) is K-major [rows][256].  K2 and K4 run on CTA pairs (cta_group::2) with the feature tile
+// resident in shared memory; K3 keeps the mask embeddings resident instead.  The linear layers (tc_gemm_kernel)
+// stream both operands.  Ragged shapes need no code in the kernels: TMA fills the out-of-bounds part of a load
+// box with zeros and clips stores at the tensor's extent.
 //   warp 0 : TMA producer (one lane)        warp 1 : TMEM alloc + tcgen05.mma issue (one lane)
 //   warps 2..17 : epilogue (tcgen05.ld -> registers -> global), 4 warps per TMEM lane quarter
 #include "gemm_tc.h"
@@ -34,37 +31,30 @@ constexpr int TC_BM = 128;      // pixels per CTA (UMMA M)
 constexpr int TC_BK = 64;       // channels per smem chunk (one 128B swizzle row of bf16 K... see below)
 constexpr int A_CHUNK_BYTES = 2 * 64 * 64 * 2;   // 2 pixel groups x 64 ch x 64 px x bf16 = 16 KB
 
-enum { EPI_MASK_T = 0, EPI_ROWMAJOR = 1, EPI_BITS = 2, EPI_LINEAR_T = 3 };
-
-struct TcGemmP {
-  int NT, N_TILE, KC, stages;
-  int a_resident;        // 1: the whole A tile (KC chunks) stays in smem for all NT tiles; 0: A chunks stream with B
-  int a_kmajor;          // 0: A is an NCHW feature map (pixels contiguous); 1: A is [rows][K] activations (K contiguous)
-  int k_identity;        // 1: chunk kc sits at K coordinate kc*64 for both operands (kcoord tables unused)
-  int a_kcoord[12];      // channel coordinate of A chunk kc   (operands whose chunks sit at different K coordinates)
-  int b_kcoord[12];      // K coordinate of B chunk kc
-  // split precision (EPI_LINEAR_T): rows of both operands are [hi(split_K) | lo(split_K)] bf16 pairs and the CTA walks
+// Linear layers (tc_gemm_kernel): one 128-feature x N_TILE-token tile per CTA
+struct TcLinP {
+  int N_TILE, KC, stages, tmem_cols;
+  int f16;               // 1: operands are IEEE half instead of bf16
+  // split precision: rows of both operands are [hi(split_K) | lo(split_K)] bf16 pairs and the CTA walks
   // 3 * split_cpc chunks = hi.hi, hi.lo, lo.hi terms of its K range (split_cpc chunks of 64 per term); 0 = off
   int split_cpc, split_K;
-  // EPI_LINEAR_T: up to 3 FEATURE segments (32-aligned starts) of (acc + bias [+ rowbias]) * alpha [+ res] [relu]
+  // up to 3 FEATURE segments (32-aligned starts) of (acc + bias [+ rowbias]) * alpha [+ res] [relu]
   TcSeg seg[3]; int nseg; const float* lin_bias; int n_tokens;
-  long kpart_stride;     // EPI_LINEAR_T with gridDim.z K-parts: part z writes its partial sums at ptr + z*kpart_stride (fp32)
-  int b_row0;            // first B row (e.g. call_idx * q_pad)
-  int b_rows_per_batch;  // B row offset per blockIdx.y (0: weights shared by the batch)
+  long kpart_stride;     // with gridDim.z K-parts: part z writes its partial sums at ptr + z*kpart_stride (fp32)
+};
+
+// CTA-pair kernels (K2 einsum, K2 transposed einsum, K4): persistent pairs walk work items of two 128-pixel
+// tiles of one image; the feature tiles are resident in shared memory, N is walked in NT tiles.
+struct TcPairP {
+  int NT, N_TILE, stages;
+  int b_row0;            // first B row (first_call * q_pad)
+  int b_rows_per_batch;  // B row offset per image (0: weights shared by the batch)
   int acc_stride;        // TMEM columns between the two accumulator buffers
   int tmem_cols;         // power of two >= 32
-  int epi;
-  int f16;               // 1: operands are IEEE half instead of bf16 (attention-mask GEMM)
   int ein_split, q_rows; // transposed einsum: 0 = two head calls per step (q_rows = q_pad rows each CTA), 1 = one call per step, CTA r takes rows [r q_rows, (r+1) q_rows)
-  int M_valid;           // valid pixels / keys per batch image (features for EPI_LINEAR_T)
-  int m_tiles, n_batch, n_work;   // A-resident kinds are persistent: CTA c walks work items c, c+grid, ... of m_tiles*n_batch
-  // EPI_MASK_T
-  __nv_bfloat16* out_mask; long out_call_stride, out_batch_stride, HW; int Q, q_pad, n_calls;
-  // EPI_ROWMAJOR
-  __nv_bfloat16* out_rows; long ld_out, out_rows_batch_stride; const float* bias; const __nv_bfloat16* R;
-  long ldr; int r_ncols;
-  // EPI_BITS
-  uint32_t* bitmap; int W32;
+  int m_pairs, n_batch;  // work items per image (ceil(128-pixel tiles / 2)), images
+  int q_pad, n_calls;    // K2: rows per head call in the B operand, head calls of the launch
+  const float* bias;     // K4: bias of all NT * N_TILE output columns
 };
 
 __device__ __forceinline__ bool masked_from_logit(float d) {
@@ -95,12 +85,11 @@ struct EpiCtx {
 };
 
 // K2 epilogue: out[call][image][q][pixel] bf16.  TMEM lanes = pixels, columns = (call, q): the tile
-// is staged in shared memory as [column][128 pixels] and leaves through TMA stores -- one
-// (128 px x Q rows) box per head call of the tile; rows q >= Q fall outside the tensor and are clipped
-// by the TMA unit.  No per-thread global stores at all.
-__device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, uint8_t* sStage, const CUtensorMap* tmC,
-                                           bool leader_warp, bool last, int m_tile, uint64_t* acc_empty_bar,
-                                           bool arrive_on_leader) {
+// is staged in shared memory as [column][128 pixels] and leaves through one TMA store of a
+// (128 px x N_TILE rows) box; a tile never spans two head calls, and rows q >= Q fall outside the tensor
+// and are clipped by the TMA unit.  No per-thread global stores at all.
+__device__ __forceinline__ void epi_mask_t(const TcPairP& p, const EpiCtx& c, uint8_t* sStage, const CUtensorMap* tmC,
+                                           bool leader_warp, bool last, int m_tile, uint64_t* acc_empty_bar) {
   const bool leader = leader_warp && c.lane == 0;
   // 1. accumulator -> registers (up to 4 chunks of 16 columns per warp, loads in flight together).
   //    This overlaps the TMA engine still reading the previous tile out of the staging buffer.
@@ -119,10 +108,7 @@ __device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, ui
   // 2. the accumulator buffer is free again: the MMAs of the tile after next may start
   ptx::tc_fence_before();
   __syncwarp();
-  if (c.lane == 0) {
-    if (arrive_on_leader) ptx::mbar_arrive_leader(acc_empty_bar);
-    else ptx::mbar_arrive(acc_empty_bar);
-  }
+  if (c.lane == 0) ptx::mbar_arrive_leader(acc_empty_bar);
   // 3. the previous tile's stores must have finished READING the staging buffer
   if (leader) ptx::tma_store_wait_read();
   asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
@@ -139,18 +125,8 @@ __device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, ui
   ptx::fence_proxy_async_smem();
   asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
   if (leader) {
-    const int r0 = c.col0;                       // first (call, q) row of this tile
-    const int N_TILE = c.chunks * 16, q_pad = p.q_pad;
-    if (N_TILE >= q_pad) {
-      for (int sidx = 0; sidx * q_pad + q_pad <= N_TILE || sidx == 0; ++sidx) {
-        const int call = r0 / q_pad + sidx;
-        if (call >= p.n_calls || sidx * q_pad >= N_TILE) break;
-        ptx::tma_store_3d(tmC, sStage + (long)sidx * q_pad * TC_BM * 2, m_tile * TC_BM, 0, call * p.n_batch + c.batch);
-      }
-    } else {
-      const int call = r0 / q_pad, q0 = r0 - call * q_pad;
-      if (call < p.n_calls) ptx::tma_store_3d(tmC, sStage, m_tile * TC_BM, q0, call * p.n_batch + c.batch);
-    }
+    const int call = c.col0 / p.q_pad, q0 = c.col0 - call * p.q_pad;   // first (call, q) row of this tile
+    ptx::tma_store_3d(tmC, sStage, m_tile * TC_BM, q0, call * p.n_batch + c.batch);
     ptx::tma_store_commit();
     if (last) ptx::tma_store_wait_read();   // smem must stay valid until the last store has read it
   }
@@ -161,9 +137,8 @@ __device__ __forceinline__ void epi_mask_t(const TcGemmP& p, const EpiCtx& c, ui
 // 16-byte chunks at chunk ^ (row & 7): conflict-free) and leaves through one TMA store per sub-tile;
 // rows past the image's last key are clipped by the TMA unit.  (The positional / level part of the keys
 // is not added here at all: the attention kernel adds Q R^T, see attention_tc.cu.)
-__device__ __forceinline__ void epi_rowmajor(const TcGemmP& p, const EpiCtx& c, uint8_t* sStage, const float* sBias,
-                                             const CUtensorMap* tmC, bool leader_warp, bool last, int m_tile,
-                                             uint64_t* acc_empty_bar, bool arrive_on_leader = false) {
+__device__ __forceinline__ void epi_rowmajor(const EpiCtx& c, uint8_t* sStage, const float* sBias, const CUtensorMap* tmC,
+                                             bool leader_warp, bool last, int m_tile, uint64_t* acc_empty_bar) {
   const bool leader = leader_warp && c.lane == 0;
   static_assert(EPI_PARTS == 4, "four chunk slots per warp below");
   // 1. accumulator -> registers (up to 4 chunks of 16 columns per warp, loads in flight together); this overlaps
@@ -182,10 +157,7 @@ __device__ __forceinline__ void epi_rowmajor(const TcGemmP& p, const EpiCtx& c, 
   // 2. the accumulator buffer is free again
   ptx::tc_fence_before();
   __syncwarp();
-  if (c.lane == 0) {
-    if (arrive_on_leader) ptx::mbar_arrive_leader(acc_empty_bar);
-    else ptx::mbar_arrive(acc_empty_bar);
-  }
+  if (c.lane == 0) ptx::mbar_arrive_leader(acc_empty_bar);
   // 3. the previous tile's stores must have finished READING the staging buffer
   if (leader) ptx::tma_store_wait_read();
   asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
@@ -220,7 +192,7 @@ __device__ __forceinline__ void epi_rowmajor(const TcGemmP& p, const EpiCtx& c, 
 
 // K3 epilogue: threshold + ballot = 32 consecutive key bits of one query per warp instruction.
 // sigmoid(x) < 0.5 in fp32 holds exactly for x <= -1.7881392e-07 (SURVEY.md section 7.2).
-__device__ __forceinline__ void epi_bits_impl(int Q, int W32, uint32_t* bitmap, const EpiCtx& c) {
+__device__ __forceinline__ void epi_bits(int Q, int W32, uint32_t* bitmap, const EpiCtx& c) {
   uint32_t* brow = bitmap + (long)c.batch * Q * W32 + c.wi;
   const bool w_ok = c.wi < W32;
   for (int ch = c.part; ch < c.chunks; ch += EPI_PARTS) {
@@ -234,7 +206,6 @@ __device__ __forceinline__ void epi_bits_impl(int Q, int W32, uint32_t* bitmap, 
     }
   }
 }
-__device__ __forceinline__ void epi_bits(const TcGemmP& p, const EpiCtx& c) { epi_bits_impl(p.Q, p.W32, p.bitmap, c); }
 
 // Swap-AB linear layers: TMEM lanes = output FEATURES, columns = tokens; for one token a warp holds
 // 32 consecutive features, so every global access is one coalesced line.  The thread's segment is
@@ -247,7 +218,7 @@ struct LinCtx {
   void* ptr = nullptr;
   const float* rowbias = nullptr;
   const float* res = nullptr;
-  __device__ __forceinline__ void init(const TcGemmP& p, int m) {
+  __device__ __forceinline__ void init(const TcLinP& p, int m) {
 #pragma unroll
     for (int sgi = 0; sgi < 3; ++sgi) {
       if (sgi < p.nseg && m >= p.seg[sgi].col0 && m < p.seg[sgi].col0 + p.seg[sgi].ncols) {
@@ -269,12 +240,12 @@ struct LinCtx {
 };
 
 // Per-token operands of the epilogue (row bias or residual) do not depend on the accumulator: they are
-// fetched while the MMAs still run (up to 2 chunks of 16 tokens per warp, the N_TILE = 128 case).
+// fetched while the MMAs still run (up to 2 chunks of 16 tokens per warp: N_TILE <= 128).
 struct LinPre {
   float a[16], b[16];
 };
-__device__ __forceinline__ void lin_prefetch(const TcGemmP& p, const EpiCtx& c, const LinCtx& L, LinPre& pre) {
-  const int tok_base = c.batch * p.NT * p.N_TILE;
+__device__ __forceinline__ void lin_prefetch(const TcLinP& p, const EpiCtx& c, const LinCtx& L, LinPre& pre) {
+  const int tok_base = c.batch * p.N_TILE;
 #pragma unroll
   for (int i = 0; i < 16; ++i) pre.a[i] = pre.b[i] = 0.f;
   if (!L.on || (L.rowbias == nullptr && L.res == nullptr)) return;
@@ -302,45 +273,24 @@ __device__ __forceinline__ void lin_prefetch(const TcGemmP& p, const EpiCtx& c, 
 }
 
 template <int MODE, bool HAS_RB, bool HAS_RES>
-__device__ __forceinline__ void epi_linear_t(const TcGemmP& p, const EpiCtx& c, const LinCtx& L, const LinPre* pre) {
+__device__ __forceinline__ void epi_linear_t(const TcLinP& p, const EpiCtx& c, const LinCtx& L, const LinPre& pre) {
   const int n_tokens = p.n_tokens;
-  const int tok_base = c.batch * p.NT * p.N_TILE + c.col0;
+  const int tok_base = c.batch * p.N_TILE;
   int j = 0;
   for (int ch = c.part; ch < c.chunks; ch += EPI_PARTS, ++j) {
     const int tok0 = tok_base + ch * 16;
     const int nvalid = L.on ? min(16, n_tokens - tok0) : 0;      // <= 0: nothing to store
-    float rb[16], rs[16];
-    if (HAS_RB) {
-      if (pre && j < 2) {
+    float ex[16];                                                 // the prefetched row bias or residual
 #pragma unroll
-        for (int i = 0; i < 16; ++i) rb[i] = j ? pre->b[i] : pre->a[i];
-      } else {
-        int tq = tok0 % L.rb_mod;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          rb[i] = (i < nvalid) ? __ldg(L.rowbias + (long)tq * L.rb_ld + L.f) : 0.f;
-          if (++tq == L.rb_mod) tq = 0;
-        }
-      }
-    }
-    if (HAS_RES) {
-      if (pre && j < 2) {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) rs[i] = j ? pre->b[i] : pre->a[i];
-      } else {
-        const float* rp = L.res + (long)tok0 * L.res_ld + L.f;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) rs[i] = (i < nvalid) ? __ldg(rp + (long)i * L.res_ld) : 0.f;
-      }
-    }
+    for (int i = 0; i < 16; ++i) ex[i] = j ? pre.b[i] : pre.a[i];
     float v[16];
     ptx::tmem_ld16(c.taddr + (uint32_t)(ch * 16), v);
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       float x = v[i] + L.bias;
-      if (HAS_RB) x += rb[i];
+      if (HAS_RB) x += ex[i];
       x *= L.alpha;
-      if (HAS_RES) x += rs[i];
+      if (HAS_RES) x += ex[i];
       x = fmaxf(x, L.floor);
       if (i < nvalid) {
         const long off = (long)(tok0 + i) * L.ld + L.f;
@@ -361,7 +311,7 @@ __device__ __forceinline__ void epi_linear_t(const TcGemmP& p, const EpiCtx& c, 
   }
 }
 
-__device__ __forceinline__ void epi_linear_dispatch(const TcGemmP& p, const EpiCtx& c, const LinCtx& L, const LinPre* pre) {
+__device__ __forceinline__ void epi_linear_dispatch(const TcLinP& p, const EpiCtx& c, const LinCtx& L, const LinPre& pre) {
   // warp-uniform: a warp's 32 features belong to one segment (32-aligned segment starts)
   const bool rb = L.rowbias != nullptr, rs = L.res != nullptr;
   if (L.mode == 0) {
@@ -378,65 +328,40 @@ __device__ __forceinline__ void epi_linear_dispatch(const TcGemmP& p, const EpiC
   }
 }
 
-// Specialised per epilogue kind: the operand layout / residency follow from it at compile time
-//   EPI_MASK_T, EPI_ROWMAJOR : A = NCHW feature map, tile resident in smem for all N tiles
-//   EPI_BITS                 : A = NCHW (hi/lo planes), streamed with B
-//   EPI_LINEAR_T             : A = weights (K-major), streamed with B
-template <int EPI>
+// ------------------------------------------------------------------- linear layers
+// Swap-AB: A = weights [features][K] (128 features per CTA on the TMEM lanes, blockIdx.x), B = activations
+// [tokens][K] (one tile of N_TILE <= 128 tokens, blockIdx.y), K range of part blockIdx.z.  Both operands are
+// K-major and stream together through a ring of TMA stages; one accumulator tile per CTA.
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcGemmP p) {
-  constexpr bool A_KMAJOR = (EPI == EPI_LINEAR_T);
-  constexpr bool A_RESIDENT = (EPI == EPI_MASK_T || EPI == EPI_ROWMAJOR);
+               const __grid_constant__ TcLinP p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  const int b_tile_bytes = p.N_TILE * 128;
-  const int a_in_stage = A_RESIDENT ? 0 : A_CHUNK_BYTES;
-  const int b_stage_bytes = a_in_stage + b_tile_bytes;      // ring stage = [A chunk (if streamed)] [B chunk]
-  uint8_t* sA = smem;
-  uint8_t* sB = sA + (A_RESIDENT ? p.KC * A_CHUNK_BYTES : 0);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sB + p.stages * b_stage_bytes);
-  uint64_t* a_full = bars;            // [4] per A chunk (resident kinds)
-  uint64_t* a_empty = bars + 4;       // [4] the last N tile's MMAs of a work item are done with A chunk kc
-  uint64_t* b_full = bars + 8;
-  uint64_t* b_empty = b_full + p.stages;
-  uint64_t* acc_full = b_empty + p.stages;
-  uint64_t* acc_empty = acc_full + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
-  // EPI_MASK_T staging tile [N_TILE columns][128 pixels] bf16 for the TMA store (128-byte aligned)
-  uint8_t* sStage = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 1023) & ~(uintptr_t)1023);
-  // EPI_ROWMAJOR: the bias vector of all NT * N_TILE output columns, behind the staging tile
-  float* sBias = reinterpret_cast<float*>(sStage + (size_t)p.N_TILE * TC_BM * 2);
+  const int stage_bytes = A_CHUNK_BYTES + p.N_TILE * 128;   // ring stage = [weight chunk] [activation chunk]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + p.stages * stage_bytes);
+  uint64_t* full = bars;
+  uint64_t* empty = full + p.stages;
+  uint64_t* acc_full = empty + p.stages;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // A-resident kinds: persistent CTAs over (pixel tile, image) work items; the others: one tile per CTA
-  const int n_work = A_RESIDENT ? p.n_work : 1;
-  const int w_first = A_RESIDENT ? (int)blockIdx.x : 0;
-  const int w_stride = A_RESIDENT ? (int)gridDim.x : 1;
-  auto tile_of = [&](int w, int& m_tile, int& batch) {
-    if (A_RESIDENT) { batch = w / p.m_tiles; m_tile = w - batch * p.m_tiles; }
-    else { m_tile = blockIdx.x; batch = blockIdx.y; }
-  };
-  // K coordinates of chunk kc in the A and B tensor maps
+  // K coordinates of chunk kc in the weight (A) and activation (B) tensor maps
   auto kcoords = [&](int kc, int& ka, int& kb) {
     if (p.split_cpc > 0) {
       const int term = kc / p.split_cpc, j = kc - term * p.split_cpc;
       const int k0 = ((int)blockIdx.z * p.split_cpc + j) * TC_BK;
       ka = (term == 2 ? p.split_K : 0) + k0;      // weights:     hi, hi, lo
       kb = (term == 1 ? p.split_K : 0) + k0;      // activations: hi, lo, hi
-    } else if (p.k_identity) {
-      ka = kb = ((int)blockIdx.z * p.KC + kc) * TC_BK;
     } else {
-      ka = p.a_kcoord[kc]; kb = p.b_kcoord[kc];
+      ka = kb = ((int)blockIdx.z * p.KC + kc) * TC_BK;
     }
   };
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmA);
     ptx::prefetch_tmap(&tmB);
-    for (int i = 0; i < 4; ++i) { ptx::mbar_init(&a_full[i], 1); ptx::mbar_init(&a_empty[i], 1); }
-    for (int i = 0; i < p.stages; ++i) { ptx::mbar_init(&b_full[i], 1); ptx::mbar_init(&b_empty[i], 1); }
-    for (int i = 0; i < 2; ++i) { ptx::mbar_init(&acc_full[i], 1); ptx::mbar_init(&acc_empty[i], EPI_WARPS); }
+    for (int i = 0; i < p.stages; ++i) { ptx::mbar_init(&full[i], 1); ptx::mbar_init(&empty[i], 1); }
+    ptx::mbar_init(acc_full, 1);
     ptx::fence_mbar_init();
   }
   if (warp == 1) {
@@ -449,153 +374,73 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const uint32_t tmem_base = *tmem_slot;
   // everything above (barriers, TMEM, descriptor prefetch) overlapped the previous kernel's tail
   ptx::grid_dep_launch();
-  // Linear layers: the A operand is a WEIGHT matrix, independent of the previous kernel -- its first ring-full of
-  // chunks is requested before waiting for the previous grid (the activations, operand B, follow after the wait).
-  int n_pre = 0;
-  if (EPI == EPI_LINEAR_T && warp == 0 && lane == 0) {
-    const int total = p.NT * p.KC;
-    n_pre = total < p.stages ? total : p.stages;
-    for (int i = 0; i < n_pre; ++i) {
-      const int kc = i % p.KC;
-      int kco, kcb;
-      kcoords(kc, kco, kcb);
-      ptx::mbar_expect_tx(&b_full[i], (uint32_t)b_stage_bytes);
-      ptx::tma_load_2d(sB + i * b_stage_bytes, &tmA, &b_full[i], kco, (int)blockIdx.x * TC_BM);
+  // The A operand is a WEIGHT matrix, independent of the previous kernel: its first ring-full of chunks is
+  // requested before waiting for the previous grid (the activations, operand B, follow after the wait).
+  const int n_pre = p.KC < p.stages ? p.KC : p.stages;
+  if (warp == 0 && lane == 0)
+    for (int kc = 0; kc < n_pre; ++kc) {
+      int ka, kb;
+      kcoords(kc, ka, kb);
+      ptx::mbar_expect_tx(&full[kc], (uint32_t)stage_bytes);
+      ptx::tma_load_2d(smem + kc * stage_bytes, &tmA, &full[kc], ka, (int)blockIdx.x * TC_BM);
     }
-  }
   ptx::grid_dep_wait();
 
   if (warp == 0) {
     if (lane == 0) {
-      // ---------------- TMA producer
-      // A chunk = 128 rows x 64 K: an NCHW operand comes as two (64 px x 64 ch) boxes, an
-      // activation operand as one (64 k x 128 rows) box; 16 KB either way.
-      int m_tile = 0, batch = 0;
-      auto load_a = [&](uint8_t* dst, uint64_t* bar, int kc) {
-        int kco, kcb;
-        kcoords(kc, kco, kcb);
-        if (A_KMAJOR) {
-          ptx::tma_load_2d(dst, &tmA, bar, kco, m_tile * TC_BM);
-        } else {
-          for (int g = 0; g < 2; ++g)
-            ptx::tma_load_3d(dst + g * (A_CHUNK_BYTES / 2), &tmA, bar, m_tile * TC_BM + g * 64, kco, batch);
+      // ---------------- TMA producer: a chunk is (64 k x 128 features) of A and (64 k x N_TILE tokens) of B
+      for (int kc = 0; kc < p.KC; ++kc) {
+        const int s = kc % p.stages;
+        uint8_t* stage = smem + s * stage_bytes;
+        int ka, kb;
+        kcoords(kc, ka, kb);
+        if (kc >= n_pre) {
+          ptx::mbar_wait(&empty[s], ((uint32_t)(kc / p.stages) & 1u) ^ 1u);
+          ptx::mbar_expect_tx(&full[s], (uint32_t)stage_bytes);
+          ptx::tma_load_2d(stage, &tmA, &full[s], ka, (int)blockIdx.x * TC_BM);
         }
-      };
-      int it = 0, tl = 0;
-      for (int w = w_first; w < n_work; w += w_stride, ++tl) {
-       tile_of(w, m_tile, batch);
-       if (A_RESIDENT && tl == 0)
-         for (int kc = 0; kc < p.KC; ++kc) {
-           ptx::mbar_expect_tx(&a_full[kc], (uint32_t)A_CHUNK_BYTES);
-           load_a(sA + kc * A_CHUNK_BYTES, &a_full[kc], kc);
-         }
-       for (int t = 0; t < p.NT; ++t)
-        for (int kc = 0; kc < p.KC; ++kc, ++it) {
-          if (A_RESIDENT && t == 0 && tl > 0) {
-            // the previous work item's last N tile has finished reading chunk kc: refill it while that
-            // tile's remaining MMAs and epilogue still run
-            ptx::mbar_wait(&a_empty[kc], (uint32_t)(tl & 1) ^ 1u);
-            ptx::mbar_expect_tx(&a_full[kc], (uint32_t)A_CHUNK_BYTES);
-            load_a(sA + kc * A_CHUNK_BYTES, &a_full[kc], kc);
-          }
-          const int s = it % p.stages;
-          const uint32_t ph = (uint32_t)(it / p.stages) & 1u;
-          uint8_t* stage = sB + s * b_stage_bytes;
-          if (it >= n_pre) {      // (the first n_pre stages of a linear layer already have their weights on the way)
-            ptx::mbar_wait(&b_empty[s], ph ^ 1u);
-            ptx::mbar_expect_tx(&b_full[s], (uint32_t)b_stage_bytes);
-            if (!A_RESIDENT) load_a(stage, &b_full[s], kc);
-          }
-          int kca, kcb;
-          kcoords(kc, kca, kcb);
-          ptx::tma_load_2d(stage + a_in_stage, &tmB, &b_full[s], kcb, batch * p.b_rows_per_batch + p.b_row0 + t * p.N_TILE);
-        }
+        ptx::tma_load_2d(stage + A_CHUNK_BYTES, &tmB, &full[s], kb, (int)blockIdx.y * p.N_TILE);
       }
     }
   } else if (warp == 1) {
     // ---------------- MMA issuer: the whole warp walks the loop (uniform control flow keeps the descriptors in
     // uniform registers), one elected lane issues.  Descriptors = base + constant increments of the 14-bit
-    // address field (16-byte units).
-    //   A, MN-major SW128: 16 channel rows of 128 B per MMA; pixel groups 8 KB apart (LBO), 8-row groups 1 KB apart (SBO).
-    //   A / B, K-major SW128: 32 B along K per MMA, SBO 1 KB.
-    const uint32_t idesc = ptx::umma_idesc_bf16(TC_BM, p.N_TILE, /*A MN-major*/ !A_KMAJOR, /*B K-major*/ false, p.f16 != 0);
-    const uint64_t ad0 = A_KMAJOR ? ptx::umma_desc_sw128(ptx::smem_u32(A_RESIDENT ? sA : sB), 16, 1024)
-                                  : ptx::umma_desc_sw128(ptx::smem_u32(A_RESIDENT ? sA : sB), A_CHUNK_BYTES / 2, 1024);
-    const uint64_t bd0 = ptx::umma_desc_sw128(ptx::smem_u32(sB + a_in_stage), 16, 1024);
-    const uint32_t a_step = A_KMAJOR ? 2u : (2048u >> 4);
-    const uint32_t stage16 = (uint32_t)b_stage_bytes >> 4;
-    int it = 0, g = 0, tl = 0;
-    for (int w = w_first; w < n_work; w += w_stride, ++tl)
-      for (int t = 0; t < p.NT; ++t, ++g) {
-        const int buf = g & 1;
-        const uint32_t use = (uint32_t)(g >> 1);
-        ptx::mbar_wait(&acc_empty[buf], (use & 1u) ^ 1u);
-        ptx::tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(buf * p.acc_stride);
-        for (int kc = 0; kc < p.KC; ++kc, ++it) {
-          const int s = it % p.stages;
-          const uint32_t ph = (uint32_t)(it / p.stages) & 1u;
-          if (A_RESIDENT && t == 0) ptx::mbar_wait(&a_full[kc], (uint32_t)(tl & 1));
-          ptx::mbar_wait(&b_full[s], ph);
-          ptx::tc_fence_after();
-          if (ptx::elect_one()) {
-            const uint64_t ad = ad0 + (uint64_t)(A_RESIDENT ? (uint32_t)kc * (A_CHUNK_BYTES >> 4) : (uint32_t)s * stage16);
-            const uint64_t bd = bd0 + (uint64_t)((uint32_t)s * stage16);
+    // address field (16-byte units); K-major SW128: 32 B along K per MMA, SBO 1 KB.
+    const uint32_t idesc = ptx::umma_idesc_bf16(TC_BM, p.N_TILE, /*A MN-major*/ false, /*B K-major*/ false, p.f16 != 0);
+    const uint64_t ad0 = ptx::umma_desc_sw128(ptx::smem_u32(smem), 16, 1024);
+    const uint64_t bd0 = ptx::umma_desc_sw128(ptx::smem_u32(smem + A_CHUNK_BYTES), 16, 1024);
+    const uint32_t stage16 = (uint32_t)stage_bytes >> 4;
+    for (int kc = 0; kc < p.KC; ++kc) {
+      const int s = kc % p.stages;
+      ptx::mbar_wait(&full[s], (uint32_t)(kc / p.stages) & 1u);
+      ptx::tc_fence_after();
+      if (ptx::elect_one()) {
+        const uint64_t off = (uint64_t)((uint32_t)s * stage16);
 #pragma unroll
-            for (int k = 0; k < TC_BK / 16; ++k)
-              ptx::mma_bf16_ss(d_tmem, ad + (uint64_t)(k * a_step), bd + (uint64_t)(k * 2), idesc, (kc | k) != 0 ? 1u : 0u);
-            ptx::mma_commit(&b_empty[s]);      // frees the B stage when these MMAs retire
-            if (A_RESIDENT && t == p.NT - 1) ptx::mma_commit(&a_empty[kc]);
-            if (kc == p.KC - 1) ptx::mma_commit(&acc_full[buf]);     // accumulator tile complete
-          }
-          __syncwarp();
-        }
+        for (int k = 0; k < TC_BK / 16; ++k)
+          ptx::mma_bf16_ss(tmem_base, ad0 + off + (uint64_t)(k * 2), bd0 + off + (uint64_t)(k * 2), idesc,
+                           (kc | k) != 0 ? 1u : 0u);
+        ptx::mma_commit(&empty[s]);                        // frees the stage when these MMAs retire
+        if (kc == p.KC - 1) ptx::mma_commit(acc_full);     // accumulator tile complete
       }
+      __syncwarp();
+    }
   } else {
     // ---------------- epilogue: EPI_WARPS warps, EPI_WARPS/4 per TMEM lane quarter; each warp takes
-    // every (EPI_WARPS/4)-th 16-column chunk.  One lean, specialised loop per epilogue kind.
+    // every (EPI_WARPS/4)-th 16-column chunk
     const int quarter = warp & 3;
-    const int part = (warp - 2) >> 2;                       // which share of the chunks
-    if (EPI == EPI_ROWMAJOR) {
-      for (int i = threadIdx.x - 64; i < p.NT * p.N_TILE; i += EPI_WARPS * 32) sBias[i] = __ldg(p.bias + i);
-      asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
-    }
-    int g = 0;
-    for (int w = w_first; w < n_work; w += w_stride) {
-    int m_tile, batch;
-    tile_of(w, m_tile, batch);
-    const bool last_work = w + w_stride >= n_work;
-    const int m = m_tile * TC_BM + quarter * 32 + lane;     // TMEM lane -> pixel / key / feature index
-    const bool m_ok = m < p.M_valid;
+    const int m = (int)blockIdx.x * TC_BM + quarter * 32 + lane;    // TMEM lane -> output feature
     EpiCtx ctx;
-    ctx.lane = lane; ctx.m = m; ctx.m_ok = m_ok; ctx.batch = batch; ctx.part = part;
-    ctx.chunks = p.N_TILE / 16; ctx.wi = (m_tile * TC_BM + quarter * 32) >> 5;
+    ctx.lane = lane; ctx.m = m; ctx.m_ok = true; ctx.batch = blockIdx.y; ctx.part = (warp - 2) >> 2;
+    ctx.chunks = p.N_TILE / 16; ctx.wi = 0; ctx.col0 = 0;
+    ctx.taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
     LinCtx lin;
     LinPre pre;
-    const bool use_pre = EPI == EPI_LINEAR_T && p.NT == 1;
-    if (EPI == EPI_LINEAR_T) {
-      lin.init(p, m);
-      if (use_pre) lin_prefetch(p, ctx, lin, pre);
-    }
-    for (int t = 0; t < p.NT; ++t, ++g) {
-      const int buf = g & 1;
-      const uint32_t use = (uint32_t)(g >> 1);
-      ptx::mbar_wait(&acc_full[buf], use & 1u);
-      ptx::tc_fence_after();
-      ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
-      ctx.col0 = t * p.N_TILE;
-      const bool last = last_work && t == p.NT - 1;
-      if (EPI == EPI_MASK_T) epi_mask_t(p, ctx, sStage, &tmC, warp == 2, last, m_tile, &acc_empty[buf], false);
-      else if (EPI == EPI_ROWMAJOR) epi_rowmajor(p, ctx, sStage, sBias, &tmC, warp == 2, last, m_tile, &acc_empty[buf]);
-      else if (EPI == EPI_BITS) epi_bits(p, ctx);
-      else epi_linear_dispatch(p, ctx, lin, use_pre ? &pre : nullptr);
-      if (EPI != EPI_MASK_T && EPI != EPI_ROWMAJOR) {   // (those epilogues release the accumulator themselves, as soon as it is in registers)
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
-      }
-    }
-    }
+    lin.init(p, m);
+    lin_prefetch(p, ctx, lin, pre);
+    ptx::mbar_wait(acc_full, 0);
+    ptx::tc_fence_after();
+    epi_linear_dispatch(p, ctx, lin, pre);
   }
   ptx::tc_fence_before();
   __syncthreads();
@@ -609,15 +454,16 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 // The mask einsum with cta_group::2 MMAs (M = 256: two 128-pixel tiles, one per CTA of the pair; N =
 // N_TILE).  Each CTA streams only HALF of every B chunk (N_TILE/2 mask-embedding rows), which makes room
 // for TWO whole N tiles of B in shared memory (2 x 4 chunks).  That matters because the single MMA-issuing
-// thread, not the tensor pipe, paces the single-CTA kernel: every tcgen05.commit costs it ~300-400
+// thread, not the tensor pipe, paces a single-CTA kernel: every tcgen05.commit costs it ~300-400
 // cycles, and a 4-stage ring needs one per chunk.  Here ONE commit per N tile (acc_full) tells the
-// epilogue "accumulator ready" and the producer "these four B slots are free".
-// Otherwise the same persistent pipeline as tc_gemm_kernel<EPI_MASK_T>: A tile resident and refilled chunk
-// by chunk under the last N tile, double-buffered accumulators, staged TMA-store epilogue (each CTA stores
-// its own 128 pixels).
+// epilogue "accumulator ready" and the producer "these four B slots are free".  An N tile never spans two
+// head calls.  Persistent pairs: A tile resident and refilled chunk by chunk under the last N tile,
+// double-buffered accumulators, staged TMA-store epilogue (each CTA stores its own 128 pixels).
+// Work items of all three pair kernels are ceil(m_tiles / 2) tile pairs per image: with an odd tile count the
+// rank-1 tile of the last pair lies wholly past the end, TMA loads it as zeros and clips its stores.
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                      const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcGemmP p) {
+                      const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcPairP p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int KC = 4;
@@ -637,7 +483,7 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = ptx::cluster_ctarank();          // 0 = leader
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  const int mt2 = p.m_tiles >> 1;                         // pixel-tile pairs per image
+  const int mt2 = p.m_pairs;                              // pixel-tile pairs per image
   const int n_work = mt2 * p.n_batch;
 
   if (warp == 0 && lane == 0) {
@@ -734,7 +580,7 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
       const bool last_work = w + n_pairs >= n_work;
       const int m = m_tile * TC_BM + quarter * 32 + lane;
       EpiCtx ctx;
-      ctx.lane = lane; ctx.m = m; ctx.m_ok = m < p.M_valid; ctx.batch = batch; ctx.part = part;
+      ctx.lane = lane; ctx.m = m; ctx.m_ok = true; ctx.batch = batch; ctx.part = part;
       ctx.chunks = p.N_TILE / 16; ctx.wi = 0;
       for (int t = 0; t < p.NT; ++t, ++g) {
         const int buf = g & 1;
@@ -743,7 +589,7 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
         ptx::tc_fence_after();
         ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
         ctx.col0 = t * p.N_TILE;
-        epi_mask_t(p, ctx, sStage, &tmC, warp == 2, last_work && t == p.NT - 1, m_tile, &acc_empty[buf], true);
+        epi_mask_t(p, ctx, sStage, &tmC, warp == 2, last_work && t == p.NT - 1, m_tile, &acc_empty[buf]);
       }
     }
   }
@@ -755,12 +601,12 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
 
 // ------------------------------------------------------------------- K4, CTA-pair variant
 // K/V projection with cta_group::2 MMAs: M = 256 = two 128-token tiles (one per CTA, resident, refilled chunk by
-// chunk under the last N tile), N = N_TILE weight rows of which each CTA streams HALF per chunk.  The single-CTA
+// chunk under the last N tile), N = N_TILE weight rows of which each CTA streams HALF per chunk.  A single-CTA
 // kernel is bound by that stream (128 KB of weights per N tile through a two-stage ring); halving it per CTA and
 // doubling the ring depth moves the kernel to its HBM-write / epilogue bound.  Epilogue = epi_rowmajor.
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                  const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcGemmP p) {
+                  const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcPairP p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int KC = 4;
@@ -782,7 +628,7 @@ tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = ptx::cluster_ctarank();
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  const int mt2 = p.m_tiles >> 1;
+  const int mt2 = p.m_pairs;
   const int n_work = mt2 * p.n_batch;
 
   if (warp == 0 && lane == 0) {
@@ -869,7 +715,7 @@ tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       const int batch = w / mt2, m_tile = (w - batch * mt2) * 2 + (int)rank;
       const bool last_work = w + n_pairs >= n_work;
       EpiCtx ctx;
-      ctx.lane = lane; ctx.m = m_tile * TC_BM + quarter * 32 + lane; ctx.m_ok = ctx.m < p.M_valid; ctx.batch = batch;
+      ctx.lane = lane; ctx.m = m_tile * TC_BM + quarter * 32 + lane; ctx.m_ok = true; ctx.batch = batch;
       ctx.part = part; ctx.chunks = p.N_TILE / 16; ctx.wi = 0;
       for (int t = 0; t < p.NT; ++t, ++g) {
         const int buf = g & 1;
@@ -877,7 +723,7 @@ tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         ptx::tc_fence_after();
         ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
         ctx.col0 = t * p.N_TILE;
-        epi_rowmajor(p, ctx, sStage, sBias, &tmC, warp == 2, last_work && t == p.NT - 1, m_tile, &acc_empty[buf], true);
+        epi_rowmajor(ctx, sStage, sBias, &tmC, warp == 2, last_work && t == p.NT - 1, m_tile, &acc_empty[buf]);
       }
     }
   }
@@ -900,7 +746,7 @@ tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 //   signals "accumulator ready" + "ring slots free".  Both accumulators (2 x 256 columns) fill the TMEM.
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_einsum_t_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constant__ CUtensorMap tmE,
-                   const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcGemmP p) {
+                   const __grid_constant__ CUtensorMap tmC, const __grid_constant__ TcPairP p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int KC = 4;
@@ -920,7 +766,7 @@ tc_einsum_t_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = ptx::cluster_ctarank();          // 0 = leader
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  const int mt2 = p.m_tiles >> 1;                         // 256-pixel tiles per image
+  const int mt2 = p.m_pairs;                              // 256-pixel tiles per image
   const int n_work = mt2 * p.n_batch;
   const int NS = p.ein_split ? p.n_calls : (p.n_calls + 1) >> 1;   // steps: two head calls each (or one, split over the pair)
   const int q0 = p.ein_split ? (int)rank * p.q_rows : 0;  // first query row of this CTA within its call
@@ -1077,7 +923,8 @@ tc_einsum_t_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
 // ------------------------------------------------------------------- K3, persistent variant
 // Attention-mask bits with the B operand RESIDENT: the head call's mask embeddings (fp16, 4 chunks of
 // N_TILE x 64) are loaded once per CTA and stay in shared memory while the CTA walks its share of the
-// image's 128-key tiles; per tile only the resampled features (fp16, 4 chunks) stream in.
+// image's 128-key tiles; per tile only the resampled features (fp16, 4 chunks) stream in.  Above 256 queries
+// the queries are split into gridDim.z slices of N_TILE: slice z holds rows z*N_TILE.. of the head call.
 // Both operands are IEEE half: the resampled features are means of four bf16 values (10 significand bits,
 // exact in fp16 for 3 of 4 values), and rounding the mask embeddings to 11 bits flips 0.02 % of the bits --
 // plain bf16 operands flip 0.12 %, outside the 99.9 % bar (CPU study in DESIGN.md).
@@ -1128,7 +975,7 @@ tc_bits_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (lane == 0) {
       ptx::mbar_expect_tx(b_res_full, (uint32_t)(4 * bt));
       for (int j = 0; j < 4; ++j)      // the fp16 copy of the mask embeddings sits in columns [C, 2C) of the rows
-        ptx::tma_load_3d(sBres + j * bt, &tmB, b_res_full, p.C + j * TC_BK, p.b_row, batch);
+        ptx::tma_load_3d(sBres + j * bt, &tmB, b_res_full, p.C + j * TC_BK, p.b_row + (int)blockIdx.z * p.N_TILE, batch);
       int it = 0;
       for (int mt = blockIdx.x; mt < p.m_tiles; mt += gridDim.x)
         for (int j2 = 0; j2 < 2; ++j2, ++it) {
@@ -1181,7 +1028,8 @@ tc_bits_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   } else {
     const int quarter = warp & 3;
     EpiCtx ctx;
-    ctx.lane = lane; ctx.batch = batch; ctx.part = (warp - 2) >> 2; ctx.chunks = p.N_TILE / 16; ctx.col0 = 0;
+    ctx.lane = lane; ctx.batch = batch; ctx.part = (warp - 2) >> 2; ctx.chunks = p.N_TILE / 16;
+    ctx.col0 = (int)blockIdx.z * p.N_TILE;       // first query of this slice
     int t = 0;
     for (int mt = blockIdx.x; mt < p.m_tiles; mt += gridDim.x, ++t) {
       const int buf = t & 1;
@@ -1191,7 +1039,7 @@ tc_bits_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       ctx.m_ok = ctx.m < p.K_valid;
       ctx.wi = (mt * TC_BM + quarter * 32) >> 5;
       ctx.taddr = tmem_base + (uint32_t)(buf * p.acc_stride) + ((uint32_t)(quarter * 32) << 16);
-      epi_bits_impl(p.Q, p.W32, p.bitmap, ctx);
+      epi_bits(p.Q, p.W32, p.bitmap, ctx);
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
@@ -1345,46 +1193,20 @@ int make_map_B(TcState* t, CUtensorMap* m, const void* base, long rows, int C, i
   return CGG_OK;
 }
 
-// cta_cap > 0: the persistent (A-resident) kinds run on at most that many CTAs, leaving SMs to a concurrent
-// latency-bound chain
-int launch_tc_gemm(TcState* t, const CUtensorMap& mA, const CUtensorMap& mB, TcGemmP p, int m_tiles, int batch,
-                   cudaStream_t s, const CUtensorMap* mC = nullptr, int kparts = 1, int cta_cap = 0) {
-  if (p.N_TILE % 16 != 0 || p.N_TILE < 16 || p.N_TILE > 256) return tc_fail(t, CGG_ERR_BAD_SHAPE, "bad N tile");
-  p.acc_stride = p.N_TILE <= 128 ? 128 : 256;
-  if (p.N_TILE <= 32) p.acc_stride = 32; else if (p.N_TILE <= 64) p.acc_stride = 64;
-  p.tmem_cols = 2 * p.acc_stride;
-  const size_t a_bytes = p.a_resident ? (size_t)p.KC * A_CHUNK_BYTES : 0;
-  const size_t b_stage = (size_t)p.N_TILE * 128 + (p.a_resident ? 0 : A_CHUNK_BYTES);
-  if (p.KC > 12 && !p.k_identity && p.split_cpc == 0) return tc_fail(t, CGG_ERR_BAD_SHAPE, "too many K chunks");
-  const size_t stage_bytes = (p.epi == EPI_MASK_T || p.epi == EPI_ROWMAJOR)
-                                 ? (size_t)p.N_TILE * TC_BM * 2 + 1024 + (p.epi == EPI_ROWMAJOR ? (size_t)p.NT * p.N_TILE * 4 : 0) : 0;
-  const size_t budget = (size_t)204 * 1024 - stage_bytes;
-  int stages = (int)((budget - a_bytes) / b_stage);
-  if (stages > 8) stages = 8;
-  if (stages > p.NT * p.KC) stages = p.NT * p.KC;
-  if (stages < 2) return tc_fail(t, CGG_ERR_BAD_SHAPE, "tile does not fit shared memory");
-  p.stages = stages;
-  const size_t smem = 1024 + a_bytes + stages * b_stage + (8 + 2 * stages + 4) * 8 + 64 + stage_bytes;
-  // the kernel instantiation fixes the A-operand layout / residency: check the caller agrees
-  const bool want_res = (p.epi == EPI_MASK_T || p.epi == EPI_ROWMAJOR), want_km = (p.epi == EPI_LINEAR_T);
-  if (want_res && p.KC > 4) return tc_fail(t, CGG_ERR_BAD_SHAPE, "resident A tile limited to 4 K chunks");
-  if ((p.a_resident != 0) != want_res || (p.a_kmajor != 0) != want_km)
-    return tc_fail(t, CGG_ERR_BAD_SHAPE, "operand layout does not match the kernel specialisation");
-  dim3 grid(m_tiles, batch, kparts);
-  const dim3 block(TC_THREADS);
-  p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-  if (want_res) {
-    int ctas = p.n_work < t->num_sms ? p.n_work : t->num_sms;
-    if (cta_cap > 0 && ctas > cta_cap) ctas = cta_cap;
-    grid = dim3(ctas, 1, 1);
-  }
-  const CUtensorMap& mCC = mC ? *mC : mB;
-  switch (p.epi) {
-    case EPI_MASK_T: TCU(launch_pdl(tc_gemm_kernel<EPI_MASK_T>, grid, block, smem, s, mA, mB, mCC, p)); break;
-    case EPI_ROWMAJOR: TCU(launch_pdl(tc_gemm_kernel<EPI_ROWMAJOR>, grid, block, smem, s, mA, mB, mCC, p)); break;
-    case EPI_BITS: TCU(launch_pdl(tc_gemm_kernel<EPI_BITS>, grid, block, smem, s, mA, mB, mCC, p)); break;
-    default: TCU(launch_pdl(tc_gemm_kernel<EPI_LINEAR_T>, grid, block, smem, s, mA, mB, mCC, p)); break;
-  }
+// TMEM columns of one N_TILE-wide fp32 accumulator: a power of two >= 32
+int tmem_cols_for(int n_tile) { return n_tile <= 32 ? 32 : n_tile <= 64 ? 64 : n_tile <= 128 ? 128 : 256; }
+
+// Launches a CTA-pair kernel over the tile pairs of `pixels` per image: ceil(pixels / 256) work items per image,
+// at most one CTA per SM and, when cta_cap > 0, at most cta_cap CTAs (leaving SMs to a concurrent latency-bound chain).
+template <typename Kernel>
+int launch_pairs(TcState* t, Kernel kernel, size_t smem, cudaStream_t s, const CUtensorMap& mA, const CUtensorMap& mB,
+                 const CUtensorMap& mC, TcPairP p, long pixels, int batch, int cta_cap = 0) {
+  p.m_pairs = (int)((pixels + 2 * TC_BM - 1) / (2 * TC_BM)); p.n_batch = batch;
+  const int items = p.m_pairs * batch;
+  int pairs = t->num_sms / 2;
+  if (cta_cap > 0 && pairs > cta_cap / 2) pairs = cta_cap / 2;
+  if (pairs > items) pairs = items;
+  TCU(launch_pdl_cluster(2, kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mB, mC, p));
   count_launch();
   TCU(cudaGetLastError());
   return CGG_OK;
@@ -1404,26 +1226,34 @@ TcState* tc_create(const cgg_config& cfg) {
   };
   if (cudaGetDevice(&dev) != cudaSuccess ||
       cudaDeviceGetAttribute(&t->num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-      !max_smem(tc_gemm_kernel<EPI_MASK_T>) || !max_smem(tc_gemm_kernel<EPI_ROWMAJOR>) ||
-      !max_smem(tc_gemm_kernel<EPI_BITS>) || !max_smem(tc_gemm_kernel<EPI_LINEAR_T>) || !max_smem(tc_kv_pair_kernel) ||
-      !max_smem(tc_bits_kernel) || !max_smem(tc_einsum_t_kernel) || !max_smem(tc_einsum_pair_kernel) ||
+      !max_smem(tc_gemm_kernel) || !max_smem(tc_kv_pair_kernel) || !max_smem(tc_bits_kernel) ||
+      !max_smem(tc_einsum_t_kernel) || !max_smem(tc_einsum_pair_kernel) ||
       tc_attention_setup() != cudaSuccess) {
     delete t;
     return nullptr;
   }
   const int Q = cfg.num_queries, calls = cfg.num_layers + 1;
-  // N tiling: two head calls per 2*round8(Q)-wide tile when that fits one MMA (Q=100 -> 208, 4% pad);
-  // otherwise one call per round16(Q) tile; above 256 queries, two tiles per call.
-  if (2 * round_up(Q, 8) <= 256 && calls % 2 == 0) {
-    t->q_pad = round_up(Q, 8) < 16 ? 16 : round_up(Q, 8); t->ein_ntile = 2 * t->q_pad; t->ein_calls_per_tile = 2;
-  } else if (round_up(Q, 16) <= 256) {
-    t->q_pad = round_up(Q, 16); t->ein_ntile = t->q_pad; t->ein_calls_per_tile = 1;
+  // Mask-einsum routing.  Shared memory holds tc_einsum_t_kernel's query rows up to 104 per CTA and
+  // tc_einsum_pair_kernel's N tile up to 208 columns.  q_pad = B-operand rows per head call.
+  //   Q <= 104   einsum_t, q_pad = max(16, round8(Q)) rows per CTA, two head calls per step
+  //   105..128   pair kernel, one head call per N tile of round16(Q)
+  //   129..208   einsum_t, q_pad = round16(Q), one head call per step split over the pair
+  //   > 208      pair kernel, T = ceil(Q / 208) N tiles of round16(ceil(Q / T)) per head call
+  if (Q <= 104) {
+    t->q_pad = round_up(Q, 8) < 16 ? 16 : round_up(Q, 8);
+  } else if (Q <= 128) {
+    t->q_pad = t->ein_ntile = round_up(Q, 16);
+  } else if (Q <= 208) {
+    t->q_pad = round_up(Q, 16);
   } else {
-    t->q_pad = round_up(Q, 32); t->ein_ntile = t->q_pad / 2; t->ein_calls_per_tile = 0;  // 2 tiles per call
-    if (t->ein_ntile > 256) { delete t; return nullptr; }
+    const int T = (Q + 207) / 208;
+    t->ein_ntile = round_up((Q + T - 1) / T, 16);
+    t->q_pad = T * t->ein_ntile;
   }
+  // attention-mask bits: one N tile of round16(Q) queries, above 256 queries two slices of round32(Q) / 2
   if (round_up(Q, 16) <= 256) { t->bits_ntile = round_up(Q, 16); t->bits_nt = 1; }
   else { t->bits_ntile = round_up(Q, 32) / 2; t->bits_nt = 2; }
+  if (t->bits_ntile > 256) { delete t; return nullptr; }
   t->rows_per_batch = calls * t->q_pad;
   t->live_bytes = 1 << 20;
   if (cudaMalloc(&t->live_buf, t->live_bytes) != cudaSuccess) { delete t; return nullptr; }
@@ -1462,8 +1292,6 @@ const void* tc_key_bias_table(const TcState* t, int level, long* cols) {
   if (cols) *cols = 2L * t->nl[level] * t->cfg.embed_dim;   // [hi | lo]
   return t->rk[level];
 }
-int tc_rows_per_batch(const TcState* t) { return t ? t->rows_per_batch : 0; }
-int tc_q_pad(const TcState* t) { return t ? t->q_pad : 0; }
 
 int tc_prepare(TcState* t, const cgg_weights* w, int H4, int W4, const int* lh, const int* lw, const int* nl,
                float* const* wkv_f32, float* const* rk_f32, float* const* bkv_f32, cudaStream_t s) {
@@ -1513,20 +1341,14 @@ int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* 
   }
   int st = make_map_A(t, &mA, mem_bf16, K, C, batch, pitch);
   if (st != CGG_OK) return st;
-  TcGemmP p = {};
+  TcPairP p = {};
   p.N_TILE = 256;
   if (N % p.N_TILE != 0) return tc_fail(t, CGG_ERR_BAD_SHAPE, "K/V width not a multiple of 256");
-  st = make_map_B(t, &mB, t->wkv[level], N, C, p.N_TILE);
+  st = make_map_B(t, &mB, t->wkv[level], N, C, p.N_TILE / 2);     // each CTA of the pair loads half of a B chunk
   if (st != CGG_OK) return st;
-  p.NT = N / p.N_TILE; p.KC = C / TC_BK;
-  p.a_resident = 1;
-  for (int kc = 0; kc < p.KC; ++kc) p.a_kcoord[kc] = p.b_kcoord[kc] = kc * TC_BK;
-  p.b_row0 = 0; p.b_rows_per_batch = 0;
-  p.epi = EPI_ROWMAJOR; p.M_valid = K;
-  p.out_rows = static_cast<__nv_bfloat16*>(kv_bf16); p.ld_out = N; p.out_rows_batch_stride = (long)K * N;
+  p.NT = N / p.N_TILE;
   // the key-bias table (pos / level / bk through Wk) is NOT added here: the attention kernel adds Q R^T
-  p.bias = t->bkv[level]; p.R = t->rk[level]; p.ldr = (long)t->nl[level] * C; p.r_ncols = 0;
-  if (p.N_TILE % 64 != 0) return tc_fail(t, CGG_ERR_BAD_SHAPE, "K/V tile width must be a multiple of 64");
+  p.bias = t->bkv[level];
   CUtensorMap mC;
   {
     const cuuint64_t dims[3] = {(cuuint64_t)N, (cuuint64_t)K, (cuuint64_t)batch};
@@ -1536,30 +1358,15 @@ int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* 
                            CU_TENSOR_MAP_L2_PROMOTION_NONE, "kv out", &t->err))
       return CGG_ERR_CUDA;
   }
-  const int m_tiles = (K + TC_BM - 1) / TC_BM;
-  if (m_tiles % 2 == 0 && K % TC_BM == 0 && p.KC == 4) {
-    CUtensorMap mBh;
-    st = make_map_B(t, &mBh, t->wkv[level], N, C, p.N_TILE / 2);
-    if (st != CGG_OK) return st;
-    p.acc_stride = 256; p.tmem_cols = 512;
-    p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-    const size_t stage_bytes = (size_t)p.N_TILE * TC_BM * 2, bias_bytes = (size_t)p.NT * p.N_TILE * 4;
-    const size_t b_stage = (size_t)(p.N_TILE / 2) * 128;
-    int stages = (int)((224 * 1024 - 4 * A_CHUNK_BYTES - stage_bytes - bias_bytes - 512) / b_stage);
-    if (stages > 8) stages = 8;
-    if (stages >= 3) {
-      p.stages = stages;
-      const size_t smem = 1024 + 4 * A_CHUNK_BYTES + stages * b_stage + stage_bytes + bias_bytes + (8 + 2 * stages + 4) * 8 + 64;
-      int pairs = t->num_sms / 2;
-      if (cta_cap > 0 && pairs > cta_cap / 2) pairs = cta_cap / 2;
-      if (pairs > p.n_work / 2) pairs = p.n_work / 2;
-      TCU(launch_pdl_cluster(2, tc_kv_pair_kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mBh, mC, p));
-      count_launch();
-      TCU(cudaGetLastError());
-      return CGG_OK;
-    }
-  }
-  return launch_tc_gemm(t, mA, mB, p, m_tiles, batch, s, &mC, 1, cta_cap);
+  p.acc_stride = tmem_cols_for(p.N_TILE); p.tmem_cols = 2 * p.acc_stride;
+  const size_t stage_bytes = (size_t)p.N_TILE * TC_BM * 2, bias_bytes = (size_t)p.NT * p.N_TILE * 4;
+  const size_t b_stage = (size_t)(p.N_TILE / 2) * 128;
+  int stages = (int)((224 * 1024 - 4 * A_CHUNK_BYTES - stage_bytes - bias_bytes - 512) / b_stage);
+  if (stages > 8) stages = 8;
+  if (stages < 3) return tc_fail(t, CGG_ERR_BAD_SHAPE, "K/V projection: weight ring does not fit shared memory");
+  p.stages = stages;
+  const size_t smem = 1024 + 4 * A_CHUNK_BYTES + stages * b_stage + stage_bytes + bias_bytes + (8 + 2 * stages + 4) * 8 + 64;
+  return launch_pairs(t, tc_kv_pair_kernel, smem, s, mA, mB, mC, p, K, batch, cta_cap);
 }
 
 int tc_downsample(TcState* t, int batch, const void* mask_features_bf16, void* ws, cudaStream_t s) {
@@ -1602,62 +1409,34 @@ int tc_mask_bits(TcState* t, int batch, int call_idx, int level, uint32_t* bitma
   // logits = F_ds . me with both operands in IEEE half (fp32 accumulate)
   int st = make_map_A(t, &mA, base + w.fds[level], K, C, batch, pitch8(K));
   if (st != CGG_OK) return st;
-  // rows beyond the buffer's logical end are covered by the 64 KB slack of me_all (finite garbage,
-  // columns >= Q are never stored)
-  st = make_map_B(t, &mB, base + w.me_all, (long)batch * t->rows_per_batch + 128, 2 * C, t->bits_ntile);
-  if (st != CGG_OK) return st;
-  if (t->bits_nt == 1 && 4 * t->bits_ntile * 128 + 4 * A_CHUNK_BYTES <= 200 * 1024) {
-    // persistent, B-resident variant (Q <= 128)
-    TcBitsP bp = {};
-    bp.N_TILE = t->bits_ntile; bp.b_row = 0; bp.m_tiles = (K + TC_BM - 1) / TC_BM; bp.K_valid = K; bp.Q = Q;
-    bp.W32 = (K + 31) / 32; bp.C = C; bp.bitmap = bitmap;
-    bp.acc_stride = bp.N_TILE <= 32 ? 32 : bp.N_TILE <= 64 ? 64 : 128;
-    bp.tmem_cols = 2 * bp.acc_stride;
-    bp.stages = (int)((225 * 1024 - 4 * bp.N_TILE * 128) / (2 * A_CHUNK_BYTES));   // stages of two feature chunks
-    if (bp.stages > 4) bp.stages = 4;
-    // per-image B rows differ: one map per launch over all rows, row coordinate = image base + call offset
-    // (blockIdx.y = image) -> the kernel needs the per-image row: pass through b_row and rows_per_batch
-    bp.b_row = call_idx * t->q_pad;
-    const size_t smem = 1024 + 4 * (size_t)bp.N_TILE * 128 + (size_t)bp.stages * 2 * A_CHUNK_BYTES + (1 + 2 * bp.stages + 4) * 8 + 64;
-    int gx = t->num_sms / batch;
-    if (gx < 1) gx = 1;
-    if (gx > bp.m_tiles) gx = bp.m_tiles;
-    bp.m_tiles = bp.m_tiles;
-    // B map: rows of ONE image only (the image's row block is selected by offsetting the base pointer per launch
-    // would need one map per image) -> use a 3-D map (k, row-in-image, image)
-    CUtensorMap mB3;
-    {
-      const cuuint64_t dims[3] = {(cuuint64_t)(2 * C), (cuuint64_t)t->rows_per_batch, (cuuint64_t)batch};
-      const cuuint64_t strides[2] = {(cuuint64_t)(2 * C) * 2, (cuuint64_t)t->rows_per_batch * (2 * C) * 2};
-      const cuuint32_t box[3] = {64, (cuuint32_t)bp.N_TILE, 1};
-      if (!encode_tensor_map(&mB3, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base + w.me_all, dims, strides, box,
-                             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "me", &t->err))
-        return CGG_ERR_CUDA;
-    }
-    TCU(launch_pdl(tc_bits_kernel, dim3(gx, batch), dim3(TC_THREADS), smem, s, mA, mB3, bp));
-    count_launch();
-    TCU(cudaGetLastError());
-    const int rows = batch * Q;
-    TCU(launch_pdl(all_masked_kernel, dim3((rows + 7) / 8), dim3(256), 0, s, (const uint32_t*)bitmap, rows, bp.W32, K, all_masked));
-    count_launch();
-    TCU(cudaGetLastError());
-    return CGG_OK;
+  TcBitsP bp = {};
+  bp.N_TILE = t->bits_ntile; bp.m_tiles = (K + TC_BM - 1) / TC_BM; bp.K_valid = K; bp.Q = Q;
+  bp.W32 = (K + 31) / 32; bp.C = C; bp.bitmap = bitmap;
+  bp.acc_stride = tmem_cols_for(bp.N_TILE);
+  bp.tmem_cols = 2 * bp.acc_stride;
+  bp.stages = (int)((225 * 1024 - 4 * bp.N_TILE * 128) / (2 * A_CHUNK_BYTES));   // stages of two feature chunks
+  if (bp.stages > 4) bp.stages = 4;
+  bp.b_row = call_idx * t->q_pad;
+  const size_t smem = 1024 + 4 * (size_t)bp.N_TILE * 128 + (size_t)bp.stages * 2 * A_CHUNK_BYTES + (1 + 2 * bp.stages + 4) * 8 + 64;
+  // about one wave: (key-tile walkers) x images x query slices
+  int gx = t->num_sms / (batch * t->bits_nt);
+  if (gx < 1) gx = 1;
+  if (gx > bp.m_tiles) gx = bp.m_tiles;
+  // B map (k, row in image, image): the image's row block is selected by blockIdx.y; rows past the image's
+  // block (the last call's second slice) load as zeros and their queries are not stored
+  {
+    const cuuint64_t dims[3] = {(cuuint64_t)(2 * C), (cuuint64_t)t->rows_per_batch, (cuuint64_t)batch};
+    const cuuint64_t strides[2] = {(cuuint64_t)(2 * C) * 2, (cuuint64_t)t->rows_per_batch * (2 * C) * 2};
+    const cuuint32_t box[3] = {64, (cuuint32_t)bp.N_TILE, 1};
+    if (!encode_tensor_map(&mB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base + w.me_all, dims, strides, box,
+                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "me", &t->err))
+      return CGG_ERR_CUDA;
   }
-  TcGemmP p = {};
-  p.N_TILE = t->bits_ntile; p.NT = t->bits_nt; p.KC = C / TC_BK;
-  p.a_resident = 0;
-  p.f16 = 1;                                       // both operands are IEEE half
-  for (int kc = 0; kc < p.KC; ++kc) {
-    p.a_kcoord[kc] = kc * TC_BK;                   // resampled features (fp16 planes)
-    p.b_kcoord[kc] = C + kc * TC_BK;               // fp16 copy of the mask embeddings: columns [C, 2C) of the rows
-  }
-  p.b_row0 = call_idx * t->q_pad; p.b_rows_per_batch = t->rows_per_batch;
-  p.epi = EPI_BITS; p.M_valid = K; p.Q = Q;
-  p.bitmap = bitmap; p.W32 = (K + 31) / 32;
-  st = launch_tc_gemm(t, mA, mB, p, (K + TC_BM - 1) / TC_BM, batch, s);
-  if (st != CGG_OK) return st;
+  TCU(launch_pdl(tc_bits_kernel, dim3(gx, batch, t->bits_nt), dim3(TC_THREADS), smem, s, mA, mB, bp));
+  count_launch();
+  TCU(cudaGetLastError());
   const int rows = batch * Q;
-  TCU(launch_pdl(all_masked_kernel, dim3((rows + 7) / 8), dim3(256), 0, s, (const uint32_t*)bitmap, rows, p.W32, K, all_masked));
+  TCU(launch_pdl(all_masked_kernel, dim3((rows + 7) / 8), dim3(256), 0, s, (const uint32_t*)bitmap, rows, bp.W32, K, all_masked));
   count_launch();
   TCU(cudaGetLastError());
   return CGG_OK;
@@ -1670,103 +1449,51 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
   const int C = t->cfg.embed_dim, Q = t->cfg.num_queries;
   const long HW = (long)t->H4 * t->W4;
   char* base = static_cast<char*>(ws);
-  CUtensorMap mA, mB;
-  int st = make_map_A(t, &mA, mask_features_bf16, (int)HW, C, batch);
-  if (st != CGG_OK) return st;
-  TcGemmP p = {};
-  p.KC = C / TC_BK;
-  p.a_resident = 1;
-  for (int kc = 0; kc < p.KC; ++kc) p.a_kcoord[kc] = p.b_kcoord[kc] = kc * TC_BK;
-  p.b_row0 = first_call * t->q_pad; p.b_rows_per_batch = t->rows_per_batch;
-  p.epi = EPI_MASK_T; p.M_valid = (int)HW; p.Q = Q; p.q_pad = t->q_pad; p.n_calls = num_calls;
-  p.out_mask = static_cast<__nv_bfloat16*>(mask_bf16);
-  p.out_call_stride = call_stride; p.out_batch_stride = (long)Q * HW; p.HW = HW;
-  if (t->ein_calls_per_tile == 2 && num_calls % 2 == 0) {
-    p.N_TILE = t->ein_ntile; p.NT = num_calls / 2;
-  } else if (t->ein_calls_per_tile == 0) {
-    p.N_TILE = t->ein_ntile; p.NT = 2 * num_calls;
-  } else {
-    // one call per tile; a tile may read past this call's rows (next call / slack), never stored
-    p.N_TILE = round_up(t->q_pad, 16); p.NT = num_calls;
-    if (p.N_TILE != t->q_pad && num_calls > 1) {
-      // q_pad is a multiple of 8 only: walk call by call so tiles start on call boundaries
-      for (int c = 0; c < num_calls; ++c) {
-        st = tc_mask_einsum(t, batch, first_call + c, 1, mask_features_bf16,
-                            static_cast<__nv_bfloat16*>(mask_bf16) + (long)c * call_stride, call_stride, ws, s);
-        if (st != CGG_OK) return st;
-      }
-      return CGG_OK;
-    }
-  }
-  st = make_map_B(t, &mB, base + w.me_all, (long)batch * t->rows_per_batch + 128, 2 * C, p.N_TILE);
-  if (st != CGG_OK) return st;
-  // output map: (pixels, q, call*B + image); one (128 px x min(q_pad, N_TILE) rows) box per store
   if (num_calls > 1 && call_stride != (long)batch * Q * HW)
     return tc_fail(t, CGG_ERR_BAD_SHAPE, "mask outputs of consecutive head calls must be contiguous");
-  CUtensorMap mC;
-  {
-    const cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
-    const cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
-    const cuuint32_t box[3] = {(cuuint32_t)TC_BM, (cuuint32_t)(t->q_pad < p.N_TILE ? t->q_pad : p.N_TILE), 1};
-    if (!encode_tensor_map(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out", &t->err))
-      return CGG_ERR_CUDA;
-  }
-  const int m_tiles = (int)((HW + TC_BM - 1) / TC_BM);
-  const bool t_split = t->q_pad > 128;      // one head call per step, its rows split over the CTA pair (Q up to 256)
-  const int t_rows = t_split ? t->q_pad / 2 : t->q_pad;
-  if (m_tiles % 2 == 0 && HW % (2 * TC_BM) == 0 && t->q_pad <= 256 && t_rows % 8 == 0 && t_rows <= 128 && p.KC == 4 && C == 256) {
+  CUtensorMap mA, mB, mC;
+  int st = make_map_A(t, &mA, mask_features_bf16, (int)HW, C, batch);
+  if (st != CGG_OK) return st;
+  TcPairP p = {};
+  p.b_row0 = first_call * t->q_pad; p.b_rows_per_batch = t->rows_per_batch;
+  p.q_pad = t->q_pad; p.n_calls = num_calls;
+  // B rows up to 128 past the last call of the last image fall in the slack of me_all (finite, never stored)
+  const long b_rows = (long)batch * t->rows_per_batch + 128;
+  // output map (pixels, q, call*B + image): rows q >= Q and pixels >= HW of a store box are clipped
+  const cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
+  const cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
+  if (t->ein_ntile == 0) {
     // transposed CTA-pair kernel: queries on the TMEM lanes, pixels on the columns
-    const size_t e_chunk = (size_t)t_rows * 128;
-    const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * e_chunk + 4 * e_chunk + 24 * 8 + 64;
-    if (smem <= 227 * 1024) {
-      CUtensorMap mE, mCt;
-      st = make_map_B(t, &mE, base + w.me_all, (long)batch * t->rows_per_batch + 128, 2 * C, t_rows);
-      if (st != CGG_OK) return st;
-      {
-        const cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)Q, (cuuint64_t)num_calls * batch};
-        const cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)Q * HW * 2};
-        const cuuint32_t box[3] = {64, (cuuint32_t)t_rows, 1};
-        if (!encode_tensor_map(&mCt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box,
-                               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out, swizzled", &t->err))
-          return CGG_ERR_CUDA;
-      }
-      p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-      p.ein_split = t_split ? 1 : 0; p.q_rows = t_rows;
-      int pairs = t->num_sms / 2;
-      if (pairs > p.n_work / 2) pairs = p.n_work / 2;
-      TCU(launch_pdl_cluster(2, tc_einsum_t_kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mE, mCt, p));
-      count_launch();
-      TCU(cudaGetLastError());
-      return CGG_OK;
-    }
-  }
-  if (m_tiles % 2 == 0 && HW % TC_BM == 0 && p.N_TILE % 16 == 0 && p.KC == 4) {
-    // CTA-pair kernel: each CTA loads N_TILE/2 rows of every B chunk
-    st = make_map_B(t, &mB, base + w.me_all, (long)batch * t->rows_per_batch + 128, 2 * C, p.N_TILE / 2);
+    p.ein_split = t->q_pad > 104 ? 1 : 0;     // one head call per step, its rows split over the CTA pair
+    p.q_rows = p.ein_split ? t->q_pad / 2 : t->q_pad;
+    st = make_map_B(t, &mB, base + w.me_all, b_rows, 2 * C, p.q_rows);
     if (st != CGG_OK) return st;
-    p.acc_stride = p.N_TILE <= 128 ? 128 : 256;
-    p.tmem_cols = 2 * p.acc_stride;
-    p.m_tiles = m_tiles; p.n_batch = batch; p.n_work = m_tiles * batch;
-    const size_t stage_bytes = (size_t)p.N_TILE * TC_BM * 2 + 1024;
-    const size_t b_chunk = (size_t)(p.N_TILE / 2) * 128;
-    const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * b_chunk + 24 * 8 + 64 + stage_bytes;
-    if (smem <= 227 * 1024) {
-      p.stages = 8;
-      int pairs = t->num_sms / 2;
-      if (pairs > p.n_work / 2) pairs = p.n_work / 2;
-      TCU(launch_pdl_cluster(2, tc_einsum_pair_kernel, dim3(2 * pairs), dim3(TC_THREADS), smem, s, mA, mB, mC, p));
-      count_launch();
-      TCU(cudaGetLastError());
-      return CGG_OK;
-    }
+    const cuuint32_t box[3] = {64, (cuuint32_t)p.q_rows, 1};
+    if (!encode_tensor_map(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box,
+                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out, swizzled", &t->err))
+      return CGG_ERR_CUDA;
+    const size_t e_chunk = (size_t)p.q_rows * 128;
+    const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * e_chunk + 4 * e_chunk + 24 * 8 + 64;
+    return launch_pairs(t, tc_einsum_t_kernel, smem, s, mA, mB, mC, p, HW, batch);
   }
-  return launch_tc_gemm(t, mA, mB, p, m_tiles, batch, s, &mC);
+  // pixel-on-lane CTA-pair kernel: q_pad / N_TILE tiles per head call, each CTA loads N_TILE/2 rows of every B chunk
+  p.N_TILE = t->ein_ntile; p.NT = num_calls * (t->q_pad / t->ein_ntile);
+  p.acc_stride = tmem_cols_for(p.N_TILE); p.tmem_cols = 2 * p.acc_stride;
+  st = make_map_B(t, &mB, base + w.me_all, b_rows, 2 * C, p.N_TILE / 2);
+  if (st != CGG_OK) return st;
+  const cuuint32_t box[3] = {(cuuint32_t)TC_BM, (cuuint32_t)p.N_TILE, 1};
+  if (!encode_tensor_map(&mC, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, mask_bf16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out", &t->err))
+    return CGG_ERR_CUDA;
+  const size_t stage_bytes = (size_t)p.N_TILE * TC_BM * 2 + 1024;
+  const size_t b_chunk = (size_t)(p.N_TILE / 2) * 128;
+  const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * b_chunk + 24 * 8 + 64 + stage_bytes;
+  return launch_pairs(t, tc_einsum_pair_kernel, smem, s, mA, mB, mC, p, HW, batch);
 }
 
 // ------------------------------------------------------------------ small-M linear layers
 // y = A[M,K] W[N,K]^T (+ bias ...) with both operands bf16 K-major through TMA.  Rows are the
-// flattened (image, query) pairs; 128 rows per CTA, N walked in tiles of <= 256.
+// flattened (image, query) pairs, in tiles of <= 128; 128 output features per CTA.
 namespace {
 int make_map_act(TcState* t, CUtensorMap* m, const void* base, long rows, int K) {
   const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
@@ -1792,8 +1519,8 @@ int tc_linear(TcState* t, const __nv_bfloat16* A, int M, int K, const __nv_bfloa
   for (int i = 0; i < nsegs; ++i)
     if (segs[i].col0 % 32 != 0) return tc_fail(t, CGG_ERR_BAD_SHAPE, "segment start must be a multiple of 32");
   const int row_len = split_k ? 2 * K : K;
-  TcGemmP p = {};
-  // token tile: as few CTAs-worth of padding as possible with N <= 256 (multiple of 16)
+  TcLinP p = {};
+  // token tile: as few CTAs-worth of padding as possible with N <= 128 (multiple of 16)
   const int tok_cap = 128;   // tokens per tile; measured best (3.93 vs 4.29 ms/step at 256)
   const int n_tok_tiles = (M + tok_cap - 1) / tok_cap;
   p.N_TILE = ((M + n_tok_tiles - 1) / n_tok_tiles + 15) / 16 * 16;
@@ -1802,17 +1529,22 @@ int tc_linear(TcState* t, const __nv_bfloat16* A, int M, int K, const __nv_bfloa
   if (st != CGG_OK) return st;
   st = make_map_B(t, &mX, A, M, row_len, p.N_TILE);          // B operand: (64 k x N_TILE tokens) boxes
   if (st != CGG_OK) return st;
-  p.NT = 1; p.KC = K / TC_BK / kparts; p.kpart_stride = kpart_stride;
-  p.a_kmajor = 1; p.k_identity = 1; p.a_resident = 0;
-  if (split_k) {
-    p.k_identity = 0; p.split_cpc = K / TC_BK / kparts; p.split_K = K; p.KC = 3 * p.split_cpc;
-  }
-  p.b_row0 = 0; p.b_rows_per_batch = p.N_TILE;       // blockIdx.y = token tile
-  p.epi = EPI_LINEAR_T; p.M_valid = n_padded; p.n_tokens = M;
+  p.KC = K / TC_BK / kparts; p.kpart_stride = kpart_stride;
+  if (split_k) { p.split_cpc = p.KC; p.split_K = K; p.KC = 3 * p.split_cpc; }
+  p.n_tokens = M;
   p.f16 = f16 ? 1 : 0;
   p.nseg = nsegs; p.lin_bias = bias;
   for (int i = 0; i < nsegs; ++i) p.seg[i] = segs[i];
-  return launch_tc_gemm(t, mW, mX, p, n_padded / TC_BM, n_tok_tiles, s, nullptr, kparts);
+  p.tmem_cols = tmem_cols_for(p.N_TILE);
+  const size_t stage_bytes = A_CHUNK_BYTES + (size_t)p.N_TILE * 128;
+  p.stages = (int)(204 * 1024 / stage_bytes);
+  if (p.stages > 8) p.stages = 8;
+  if (p.stages > p.KC) p.stages = p.KC;
+  const size_t smem = 1024 + p.stages * stage_bytes + (2 * p.stages + 1) * 8 + 64;
+  TCU(launch_pdl(tc_gemm_kernel, dim3(n_padded / TC_BM, n_tok_tiles, kparts), dim3(TC_THREADS), smem, s, mW, mX, p));
+  count_launch();
+  TCU(cudaGetLastError());
+  return CGG_OK;
 }
 
 }  // namespace cgg

@@ -29,15 +29,13 @@ void tc_destroy(TcState* t);
 const char* tc_last_error(const TcState* t);
 size_t tc_workspace_bytes(const TcState* t, int batch);  // t may be null (fp32 mode) -> 0
 size_t tc_workspace_offset(const TcState* t, int batch, const char* what);  // (size_t)-1 if unknown
-int tc_rows_per_batch(const TcState* t);
-int tc_q_pad(const TcState* t);
 
 // bf16 copies of the K/V projection weights and key-bias tables for the given sizes.
 int tc_prepare(TcState* t, const cgg_weights* w, int H4, int W4, const int* lh, const int* lw, const int* nl,
                float* const* wkv_f32, float* const* rk_f32, float* const* bkv_f32, cudaStream_t s);
 
 // K4: kv[b, key, :] = mem[b, :, key]^T Wkv^T + bias tables, bf16 out (B, K_l, nl*2C)
-// cta_cap > 0: run on at most that many (persistent) CTAs, for launches that overlap a latency-bound chain
+// cta_cap > 0: run on at most that many CTAs, for launches that overlap a latency-bound chain
 int tc_kv_project(TcState* t, int level, int batch, const void* mem_bf16, void* kv_bf16, void* ws, cudaStream_t s,
                   int cta_cap = 0);
 

@@ -15,8 +15,9 @@ struct TcState {
   __nv_bfloat16* wkv[3] = {nullptr, nullptr, nullptr};   // (nl*2C, C) bf16
   __nv_bfloat16* rk[3] = {nullptr, nullptr, nullptr};    // (K_l, nl*C) bf16 key-bias table
   const float* bkv[3] = {nullptr, nullptr, nullptr};     // (nl*2C) fp32, owned by the handle
-  // N tiling of the mask einsum / bits GEMMs
-  int q_pad = 0, ein_ntile = 0, ein_calls_per_tile = 0, bits_ntile = 0, bits_nt = 0;
+  // N tiling of the mask einsum / bits GEMMs (tc_create): q_pad = B-operand rows per head call;
+  // ein_ntile = N tile of tc_einsum_pair_kernel, 0 when the mask einsum runs on tc_einsum_t_kernel
+  int q_pad = 0, ein_ntile = 0, bits_ntile = 0, bits_nt = 0;
   int rows_per_batch = 0;
   // bf16 copies of the small-M weights (path_bf16.cu)
   struct LayerW {

@@ -38,10 +38,12 @@ def _setup(Q, B, H, W, pseed, iseed):
     return sd, mf, mems, head
 
 
-# the last two have key counts that are not multiples of 8 (11x9, 22x18; 33x25, 66x50 = the reference demo's 1056x800):
-# those levels are re-pitched for TMA inside cgg_kv_project
+# 352x288 and 1056x800 have key counts that are not multiples of 8 (11x9, 22x18; 33x25, 66x50 = the reference demo's
+# 1056x800): those levels are re-pitched for TMA inside cgg_kv_project.  Odd tile counts (256x256: the 8x8 level is one
+# 128-key tile; 352x288) leave the second CTA of the last pair wholly past the end.  Q = 128 and 240 take the pixel-on-lane
+# pair einsum (one and two N tiles per head call), Q = 300 also two attention-mask query slices.
 @pytest.mark.parametrize('Q,B,H,W', [(100, 2, 256, 256), (37, 1, 256, 320), (200, 1, 256, 256), (300, 1, 256, 256),
-                                     (100, 2, 352, 288), (100, 1, 1056, 800)])
+                                     (100, 2, 352, 288), (100, 1, 1056, 800), (128, 1, 256, 256), (240, 1, 256, 256)])
 def test_bf16_teacher_forced_layers(Q, B, H, W):
     sd, mf, mems, head = _setup(Q, B, H, W, 31, 7)
     ref = O.decoder_forward(sd, mf, mems)
@@ -205,9 +207,8 @@ def test_bf16_final_mask_only_matches_full_forward():
         assert torch.equal(a, b)
 
 
-def test_bf16_batched_einsum_equals_per_call_einsum():
-    """The all-calls-in-one-pass einsum (A tile resident) must equal the per-call stage output."""
-    Q, B, H, W = 100, 2, 256, 256
+def _batched_einsum_check(Q, H, W):
+    B = 2
     sd, mf, mems, head = _setup(Q, B, H, W, 35, 11)
     mfd, memd = mf.to(DEV).bfloat16(), [m.to(DEV).bfloat16() for m in mems]
     cls, emb, mask, dbg = head.decoder_forward(mfd, memd, return_debug=True)
@@ -215,6 +216,26 @@ def test_bf16_batched_einsum_equals_per_call_einsum():
     for j in (0, 3, 9):
         _, _, m1, _, _, _ = rt.head_call(dbg['x'][j].contiguous(), mfd, j % 3, want_bits=False)
         assert torch.equal(m1, mask[j]), j
+    # head calls 1..3 of the forward still have their mask embeddings in the workspace (head_call writes call slot 0):
+    # one batched call over an odd number of head calls that does not start at call 0
+    odd = torch.empty((3,) + tuple(mask[0].shape), dtype=torch.bfloat16, device=DEV)
+    rt.mask_einsum(mfd, odd, first_call=1, num_calls=3)
+    torch.cuda.synchronize()
+    for i in range(3):
+        assert torch.equal(odd[i], mask[1 + i]), 1 + i
+
+
+def test_bf16_batched_einsum_equals_per_call_einsum():
+    """The all-calls-in-one-pass einsum (A tile resident) must equal the per-call stage output, as must a pass over an
+    odd number of head calls."""
+    _batched_einsum_check(100, 256, 256)
+
+
+@pytest.mark.parametrize('Q,H,W', [(100, 352, 288), (128, 256, 256), (240, 256, 256), (300, 256, 256)])
+def test_bf16_batched_einsum_equals_per_call_einsum_other_routes(Q, H, W):
+    """The same with a partial last pixel tile (352x288: 88x72 = 6336 mask pixels) and on the pixel-on-lane pair einsum
+    (Q = 128: one N tile per head call; Q = 240, 300: two)."""
+    _batched_einsum_check(Q, H, W)
 
 
 def test_bf16_full_size_1024_properties():
