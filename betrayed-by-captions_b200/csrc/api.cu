@@ -1,6 +1,7 @@
 // C-ABI layer + host-side orchestration of the decoder-head path (include/cgg_b200.h).
 // Everything here only enqueues kernels on the caller's stream.
 #include "../../include/cgg_b200.h"
+#include "common.cuh"
 #include "kernels.h"
 #include "gemm_tc.h"
 #include "gemm_tf32.h"
@@ -80,8 +81,6 @@ int fail(cgg_handle* h, int code, const std::string& msg) {
     if (s__ != CGG_OK) return fail(h, s__, std::string(#call) + ": " + tc_last_error(t));   \
   } while (0)
 
-inline size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
-
 // Workspace carving shared by cgg_workspace_bytes and the entry points.
 struct Workspace {
   size_t total = 0;
@@ -90,7 +89,7 @@ struct Workspace {
   void carve(const cgg_handle* h, int B) {
     const cgg_config& c = h->cfg;
     size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes); return o; };
+    auto take = [&](size_t bytes) { size_t o = off; off += align256(bytes); return o; };
     const size_t kv_elt = (c.precision == CGG_BF16) ? 2 : 4;
     for (int l = 0; l < CGG_NUM_LEVELS; ++l)
       kv[l] = take((size_t)B * h->lh[l] * h->lw[l] * h->nl[l] * 2 * c.embed_dim * kv_elt);
@@ -585,8 +584,6 @@ extern "C" int cgg_similarity(cgg_handle* h, const float* a, const float* b, int
 
 namespace {
 
-inline int round_up_i(int x, int m) { return (x + m - 1) / m * m; }
-
 template <typename T>
 int grow(cgg_handle* h, T** p, size_t* have, size_t want_elems, cudaStream_t s, bool zero) {
   if (*have >= want_elems) return CGG_OK;
@@ -610,7 +607,7 @@ int k7_similarity(cgg_handle* h, const float* pred, const float* cap, int Bg, in
     if (!h->tc_aux) return fail(h, CGG_ERR_CUDA, "tc_create (grounding) failed");
     t = h->tc_aux;
   }
-  const int rows_p = Bg * Q, rows_c = Bg * T, np = round_up_i(rows_p, 128);
+  const int rows_p = Bg * Q, rows_c = Bg * T, np = round_up(rows_p, 128);
   ST(grow(h, &h->k7.pred_hl, &h->k7.n_pred, (size_t)np * 2 * D, s, true));      // pad rows stay zero
   ST(grow(h, &h->k7.cap_hl, &h->k7.n_cap, (size_t)rows_c * 2 * D, s, false));
   ST(grow(h, &h->k7.S, &h->k7.n_S, (size_t)rows_c * rows_p, s, false));
@@ -673,7 +670,7 @@ extern "C" int cgg_grounding_loss_backward(cgg_handle* h, const float* pred, con
     // tensor-core mode: S once (tcgen05), pair kernels on S, then dpred[(j,q), :] = sum_(i,t) dS[(j,q), (i,t)] cap[(i,t), :]
     // as a second split-precision tcgen05 GEMM (M = Bg*Q tokens, N = D, K = Bg*T padded to 64)
     ST(k7_similarity(h, pred, cap, Bg, Q, T, D, temperature, s));
-    const int rows_p = Bg * Q, rows_c = Bg * T, Kp = round_up_i(rows_c, 64), nd = round_up_i(D, 128);
+    const int rows_p = Bg * Q, rows_c = Bg * T, Kp = round_up(rows_c, 64), nd = round_up(D, 128);
     ST(grow(h, &h->k7.dst_hl, &h->k7.n_dst, (size_t)rows_p * 2 * Kp, s, true));    // pad columns stay zero
     ST(grow(h, &h->k7.capT_hl, &h->k7.n_capT, (size_t)nd * 2 * Kp, s, true));
     CU(launch_grounding_pairs(pred, cap, cap_mask, Bg, Q, T, D, temperature, g1, g2, s, h->k7.S));

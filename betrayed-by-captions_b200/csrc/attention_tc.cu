@@ -109,15 +109,6 @@ __device__ __forceinline__ float fast_exp2(float x) {
   return y;
 }
 
-// Shared-memory descriptor with an explicit layout type (0 = no swizzle / core-matrix interleave,
-// 4 = SWIZZLE_64B); same bit layout as ptx::umma_desc_sw128.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t addr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-  return (uint64_t)((addr >> 4) & 0x3FFFu) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | (1ull << 46) | ((uint64_t)layout << 61);
-}
-
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 __device__ __forceinline__ int next_live(const uint8_t* live, int t, int n) {
   while (t < n && !live[t]) ++t;
   return t;
@@ -291,7 +282,7 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
       }
       *reinterpret_cast<uint4*>(sQ + (row >> 3) * 512 + c * 128 + (row & 7) * 16) = pk;
     }
-    fence_async_smem();
+    ptx::fence_proxy_async_smem();
   }
   ptx::tc_fence_before();
   __syncthreads();
@@ -358,9 +349,9 @@ masked_attention_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid
     for (int t = 0; t < p.ntiles; ++t) n_live += live[t] ? 1 : 0;
     // descriptors: base + constant increments of the 14-bit address field (16-byte units); the smem window is
     // < 256 KB so the field never carries
-    const uint64_t qd0 = umma_desc(ptx::smem_u32(sQ), 128, 512, 0);                        // Q: core matrices
-    const uint64_t kd0 = umma_desc(ptx::smem_u32(sKV), 16, 512, 4);                       // K / R tiles: SW64, K-major
-    const uint64_t vd0 = umma_desc(ptx::smem_u32(sKV + AT_KV_TILE_BYTES), 1024, 512, 4);  // V: SW64, N-major (one N group)
+    const uint64_t qd0 = ptx::umma_desc(ptx::smem_u32(sQ), 128, 512, ptx::UMMA_INTERLEAVE);             // Q: core matrices
+    const uint64_t kd0 = ptx::umma_desc(ptx::smem_u32(sKV), 16, 512, ptx::UMMA_SW64);                   // K / R tiles, K-major
+    const uint64_t vd0 = ptx::umma_desc(ptx::smem_u32(sKV + AT_KV_TILE_BYTES), 1024, 512, ptx::UMMA_SW64);  // V, N-major (one N group)
     auto wait_kv = [&](int j) {
       ptx::mbar_wait(&kv_full[j % AT_STAGES], (uint32_t)(j / AT_STAGES) & 1u);
       ptx::tc_fence_after();

@@ -12,6 +12,7 @@
 // box with zeros and clips stores at the tensor's extent.
 //   warp 0 : TMA producer (one lane)        warp 1 : TMEM alloc + tcgen05.mma issue (one lane)
 //   warps 2..17 : epilogue (tcgen05.ld -> registers -> global), 4 warps per TMEM lane quarter
+#include "common.cuh"
 #include "gemm_tc.h"
 #include "kernels.h"
 #include <cuda_fp16.h>
@@ -56,11 +57,6 @@ struct TcPairP {
   int q_pad, n_calls;    // K2: rows per head call in the B operand, head calls of the launch
   const float* bias;     // K4: bias of all NT * N_TILE output columns
 };
-
-__device__ __forceinline__ bool masked_from_logit(float d) {
-  // same expression as the fp32 path / torch: sigmoid(d) < 0.5
-  return (1.0f / (1.0f + expf(-d))) < 0.5f;
-}
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
@@ -190,8 +186,7 @@ __device__ __forceinline__ void epi_rowmajor(const EpiCtx& c, uint8_t* sStage, c
   }
 }
 
-// K3 epilogue: threshold + ballot = 32 consecutive key bits of one query per warp instruction.
-// sigmoid(x) < 0.5 in fp32 holds exactly for x <= -1.7881392e-07 (SURVEY.md section 7.2).
+// K3 epilogue: threshold (common.cuh) + ballot = 32 consecutive key bits of one query per warp instruction.
 __device__ __forceinline__ void epi_bits(int Q, int W32, uint32_t* bitmap, const EpiCtx& c) {
   uint32_t* brow = bitmap + (long)c.batch * Q * W32 + c.wi;
   const bool w_ok = c.wi < W32;
@@ -201,7 +196,7 @@ __device__ __forceinline__ void epi_bits(int Q, int W32, uint32_t* bitmap, const
     const int q0 = c.col0 + ch * 16;
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
-      const uint32_t word = __ballot_sync(0xffffffffu, c.m_ok && v[i] <= -1.7881392e-07f);
+      const uint32_t word = __ballot_sync(0xffffffffu, c.m_ok && v[i] <= MASKED_LOGIT_MAX);
       if (c.lane == 0 && w_ok && q0 + i < Q) brow[(long)(q0 + i) * W32] = word;
     }
   }
@@ -407,8 +402,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // uniform registers), one elected lane issues.  Descriptors = base + constant increments of the 14-bit
     // address field (16-byte units); K-major SW128: 32 B along K per MMA, SBO 1 KB.
     const uint32_t idesc = ptx::umma_idesc_bf16(TC_BM, p.N_TILE, /*A MN-major*/ false, /*B K-major*/ false, p.f16 != 0);
-    const uint64_t ad0 = ptx::umma_desc_sw128(ptx::smem_u32(smem), 16, 1024);
-    const uint64_t bd0 = ptx::umma_desc_sw128(ptx::smem_u32(smem + A_CHUNK_BYTES), 16, 1024);
+    const uint64_t ad0 = ptx::umma_desc(ptx::smem_u32(smem), 16, 1024, ptx::UMMA_SW128);
+    const uint64_t bd0 = ptx::umma_desc(ptx::smem_u32(smem + A_CHUNK_BYTES), 16, 1024, ptx::UMMA_SW128);
     const uint32_t stage16 = (uint32_t)stage_bytes >> 4;
     for (int kc = 0; kc < p.KC; ++kc) {
       const int s = kc % p.stages;
@@ -541,9 +536,9 @@ tc_einsum_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
       uint64_t adesc0[KC], bdesc0[2 * KC];
 #pragma unroll
       for (int kc = 0; kc < KC; ++kc)
-        adesc0[kc] = ptx::umma_desc_sw128(ptx::smem_u32(sA + kc * A_CHUNK_BYTES), A_CHUNK_BYTES / 2, 1024);
+        adesc0[kc] = ptx::umma_desc(ptx::smem_u32(sA + kc * A_CHUNK_BYTES), A_CHUNK_BYTES / 2, 1024, ptx::UMMA_SW128);
 #pragma unroll
-      for (int i = 0; i < 2 * KC; ++i) bdesc0[i] = ptx::umma_desc_sw128(ptx::smem_u32(sB + i * b_chunk_bytes), 16, 1024);
+      for (int i = 0; i < 2 * KC; ++i) bdesc0[i] = ptx::umma_desc(ptx::smem_u32(sB + i * b_chunk_bytes), 16, 1024, ptx::UMMA_SW128);
       int g = 0, tl = 0;
       for (int w = pair; w < n_work; w += n_pairs, ++tl)
         for (int t = 0; t < p.NT; ++t, ++g) {
@@ -676,8 +671,8 @@ tc_kv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   } else if (warp == 1) {
     if (rank == 0) {
       const uint32_t idesc = ptx::umma_idesc_bf16(2 * TC_BM, p.N_TILE, /*A MN-major*/ true, /*B K-major*/ false);
-      const uint64_t ad0 = ptx::umma_desc_sw128(ptx::smem_u32(sA), A_CHUNK_BYTES / 2, 1024);
-      const uint64_t bd0 = ptx::umma_desc_sw128(ptx::smem_u32(sB), 16, 1024);
+      const uint64_t ad0 = ptx::umma_desc(ptx::smem_u32(sA), A_CHUNK_BYTES / 2, 1024, ptx::UMMA_SW128);
+      const uint64_t bd0 = ptx::umma_desc(ptx::smem_u32(sB), 16, 1024, ptx::UMMA_SW128);
       const uint32_t stage16 = (uint32_t)b_stage_bytes >> 4;
       int it = 0, g = 0, tl = 0;
       for (int w = pair; w < n_work; w += n_pairs, ++tl)
@@ -822,8 +817,8 @@ tc_einsum_t_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
     if (rank == 0) {
       // ---------------- MMA issuer: the leader CTA's warp walks the loop, one elected lane drives both SMs
       const uint32_t idesc = ptx::umma_idesc_bf16(2 * TC_BM, 256, /*A = E, K-major*/ false, /*B = F, MN-major*/ true);
-      const uint64_t ed0 = ptx::umma_desc_sw128(ptx::smem_u32(sE), 16, 1024);
-      const uint64_t fd0 = ptx::umma_desc_sw128(ptx::smem_u32(sF), A_CHUNK_BYTES / 2, 1024);
+      const uint64_t ed0 = ptx::umma_desc(ptx::smem_u32(sE), 16, 1024, ptx::UMMA_SW128);
+      const uint64_t fd0 = ptx::umma_desc(ptx::smem_u32(sF), A_CHUNK_BYTES / 2, 1024, ptx::UMMA_SW128);
       const uint32_t e16 = (uint32_t)e_chunk_bytes >> 4;
       int g = 0, tl = 0;
       for (int w = pair; w < n_work; w += n_pairs, ++tl)
@@ -996,8 +991,8 @@ tc_bits_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const uint32_t idesc = ptx::umma_idesc_bf16(TC_BM, p.N_TILE, true, false, /*f16*/ true);
     ptx::mbar_wait(b_res_full, 0);
     ptx::tc_fence_after();
-    const uint64_t ad0 = ptx::umma_desc_sw128(ptx::smem_u32(sA), A_CHUNK_BYTES / 2, 1024);
-    const uint64_t bd0 = ptx::umma_desc_sw128(ptx::smem_u32(sBres), 16, 1024);
+    const uint64_t ad0 = ptx::umma_desc(ptx::smem_u32(sA), A_CHUNK_BYTES / 2, 1024, ptx::UMMA_SW128);
+    const uint64_t bd0 = ptx::umma_desc(ptx::smem_u32(sBres), 16, 1024, ptx::UMMA_SW128);
     const uint32_t bt16 = (uint32_t)bt >> 4;
     int it = 0, t = 0;
     for (int mt = blockIdx.x; mt < p.m_tiles; mt += gridDim.x, ++t) {
@@ -1145,7 +1140,10 @@ __global__ void store_me_kernel(const float* __restrict__ me, __nv_bfloat16* __r
   reinterpret_cast<__half*>(row)[C + c] = __float2half_rn(me[i]);        // columns [C,2C): fp16, read by the attention-mask GEMM
 }
 
-// all_masked[row] = (popcount of the row's bitmap == K)
+}  // namespace
+
+// all_masked[row] = (popcount of the row's bitmap == K).  The fp32 route launches it without PDL, where the two
+// griddepcontrol instructions do nothing.
 __global__ void __launch_bounds__(256) all_masked_kernel(const uint32_t* __restrict__ bitmap, int rows, int W32, int K,
                                                          uint8_t* __restrict__ all_masked) {
   ptx::grid_dep_launch();
@@ -1158,11 +1156,6 @@ __global__ void __launch_bounds__(256) all_masked_kernel(const uint32_t* __restr
   for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
   if (lane == 0) all_masked[row] = (cnt == K) ? 1 : 0;
 }
-
-inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
-inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
-}  // namespace
 
 namespace {
 

@@ -24,6 +24,7 @@
 // shared-memory row.  conv_cin turns the A loads into the nine taps of a 3x3 convolution over a token-major image (the TMA
 // unit's out-of-bounds zero fill is the padding); a weight matrix shared by every batch entry is a tensor map without
 // batch dimensions.
+#include "common.cuh"
 #include "tc_ptx.cuh"
 #include "kernels.h"
 #include "gemm_tf32.h"
@@ -64,25 +65,11 @@ struct Tf32P {
   int w_shared;                // the W operand has no batch stride (one weight matrix for every batch entry)
 };
 
-__device__ __forceinline__ void mma_tf32_ss(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // kind::tf32 instruction descriptor: c_format F32 (1) at [4,6), a/b format TF32 (2) at [7,10)/[10,13), operand majors at
 // 15 / 16 (1 = MN-major), N>>3 at [17,23), M>>4 at [24,29)  (cute::UMMA::InstrDescriptor).
 __host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N, bool a_mn, bool b_mn) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-// matrix descriptor with layout type 1 (SWIZZLE_128B_BASE32B), otherwise as ptx::umma_desc_sw128
-__device__ __forceinline__ uint64_t umma_desc_sw128_32b(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | (1ull << 61);
 }
 
 __device__ __forceinline__ float epi_value(const Tf32P& p, float acc, int b, int gm, int gn) {
@@ -181,12 +168,13 @@ __global__ void __launch_bounds__(THREADS) gemm_tf32_kernel(const __grid_constan
           ptx::mbar_wait(&full[st], (it / (uint32_t)p.stages) & 1u);
           ptx::tc_fence_after();
           const uint32_t sA = ptx::smem_u32(smem + (size_t)st * stage_bytes);
-          const uint64_t ad = p.a_mn ? umma_desc_sw128_32b(sA, 4096, 512) : ptx::umma_desc_sw128(sA, 16, 1024);
-          const uint64_t bd = p.b_mn ? umma_desc_sw128_32b(sA + A_STAGE_BYTES, 4096, 512)
-                                     : ptx::umma_desc_sw128(sA + A_STAGE_BYTES, 16, 1024);
+          const uint64_t ad = p.a_mn ? ptx::umma_desc(sA, 4096, 512, ptx::UMMA_SW128_BASE32B)
+                                     : ptx::umma_desc(sA, 16, 1024, ptx::UMMA_SW128);
+          const uint64_t bd = p.b_mn ? ptx::umma_desc(sA + A_STAGE_BYTES, 4096, 512, ptx::UMMA_SW128_BASE32B)
+                                     : ptx::umma_desc(sA + A_STAGE_BYTES, 16, 1024, ptx::UMMA_SW128);
 #pragma unroll
           for (int kk = 0; kk < BK / 8; ++kk)
-            mma_tf32_ss(d_tmem, ad + (uint64_t)(kk * a_step), bd + (uint64_t)(kk * b_step), idesc, (c > c0 || kk > 0) ? 1u : 0u);
+            ptx::mma_tf32_ss(d_tmem, ad + (uint64_t)(kk * a_step), bd + (uint64_t)(kk * b_step), idesc, (c > c0 || kk > 0) ? 1u : 0u);
           ptx::mma_commit(&empty[st]);
         }
         ptx::mma_commit(&acc_full[buf]);
@@ -402,8 +390,6 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const Tf32P p) {
   float* c = p.C + (long)(b / p.batch_inner) * p.sCb + (long)(b % p.batch_inner) * p.sCb2 + (long)gm * p.sCm + (long)gn * p.sCn;
   *c = epi_value(p, acc, b, gm, gn) + (p.accumulate ? *c : 0.f);
 }
-
-inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // operand X[b, r, k] with element strides (sb, sr, sk): 0 = K-major, 1 = MN-major, -1 = TMA cannot describe it
 int operand_major(const float* base, long sb, long sb2, long sr, long sk, int rows, int K, int batch, int batch_inner) {

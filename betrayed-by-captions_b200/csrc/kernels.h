@@ -54,6 +54,11 @@ cudaError_t launch_pos_level(const float* level_embed, float* out, int h, int w,
 // K3: mask logits (B*Q rows of H4*W4 fp32) -> bitmap words + all_masked flags for target (th,tw)
 cudaError_t launch_mask_bits(const float* mask_pred, int rows, int H4, int W4, int th, int tw,
                              uint32_t* bitmap, uint8_t* all_masked, cudaStream_t s);
+// all_masked[row] = every one of the row's K keys is masked (the reference's all-masked-row fallback,
+// mask2former_head.py:825-826).  One warp per row, 256 threads per block; defined in gemm_tc.cu, where the bf16 route
+// launches it with programmatic dependent launch.
+__global__ void all_masked_kernel(const uint32_t* __restrict__ bitmap, int rows, int W32, int K,
+                                  uint8_t* __restrict__ all_masked);
 
 // K5/K6 attention core, fp32 SIMT flash-style (K/V fp32 or bf16).  q (B,Q,H*32) pre-scaled; k,v rows of H*32 at
 // (b*kv_bstride + key*kv_stride); bitmap (B,Q,ceil(K/32)) or nullptr.

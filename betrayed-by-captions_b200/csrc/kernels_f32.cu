@@ -2,6 +2,7 @@
 // these, and the throughput mode (CGG_BF16) keeps using them for the latency-bound small-M
 // work.  No fast-math: the sigmoid threshold and the softmax follow IEEE expf / division so the
 // attention-mask bits match the PyTorch CUDA reference (SURVEY.md section 7, hard part 2).
+#include "common.cuh"
 #include "kernels.h"
 #include <cuda_fp16.h>
 #include <math.h>
@@ -12,17 +13,6 @@ namespace cgg {
 static std::atomic<unsigned long long> g_launches{0};
 void count_launch(int n) { g_launches.fetch_add((unsigned long long)n, std::memory_order_relaxed); }
 unsigned long long launch_count() { return g_launches.load(std::memory_order_relaxed); }
-
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 
 // ------------------------------------------------------------------------------- GEMM
 template <bool A_MMAJOR, bool C_MMAJOR>
@@ -185,27 +175,8 @@ cudaError_t launch_pos_level(const float* level_embed, float* out, int h, int w,
 }
 
 // ---------------------------------------------------------------- K3: attention-mask bits
-// F.interpolate(bilinear, align_corners=False) -> sigmoid() < 0.5 -> bit-pack, one warp per
-// (image, query) row.  Source index / weights follow ATen's upsample_bilinear2d:
-// src = scale*(dst+0.5)-0.5 clamped at 0;  v = h0*(w0*a + w1*b) + h1*(w0*c + w1*d).
-__device__ __forceinline__ void src_index(float scale, int dst, int in_size, int& i0, int& i1,
-                                          float& l0, float& l1) {
-  float src = scale * ((float)dst + 0.5f) - 0.5f;
-  if (src < 0.f) src = 0.f;
-  i0 = (int)src;
-  if (i0 > in_size - 1) i0 = in_size - 1;
-  i1 = i0 + ((i0 < in_size - 1) ? 1 : 0);
-  l1 = src - (float)i0;
-  l0 = 1.f - l1;
-}
-
-__device__ __forceinline__ bool masked_from_logit(float d) {
-  // torch: sigmoid(d) < 0.5 with sigmoid = 1/(1+exp(-d)) in fp32 (not a sign test:
-  // true only for d <= -1.7881392e-07)
-  const float sg = 1.0f / (1.0f + expf(-d));
-  return sg < 0.5f;
-}
-
+// F.interpolate(bilinear, align_corners=False) -> sigmoid() < 0.5 -> bit-pack, with the index math and threshold of
+// common.cuh; all_masked_kernel (gemm_tc.cu) then flags the rows that are masked at every key.
 // one warp per (row, 32-key word): 400 rows alone would leave most of the machine idle
 __global__ void __launch_bounds__(256) mask_bits_kernel(const float* __restrict__ mask_pred, long words, int W32,
                                                         int H4, int W4, int th, int tw,
@@ -222,28 +193,14 @@ __global__ void __launch_bounds__(256) mask_bits_kernel(const float* __restrict_
   bool m = false;
   if (key < K) {
     const int r = key / tw, c = key % tw;
-    int r0, r1, c0, c1;
-    float h0, h1, w0, w1;
-    src_index(sh, r, H4, r0, r1, h0, h1);
-    src_index(sw, c, W4, c0, c1, w0, w1);
-    const float a = mp[(long)r0 * W4 + c0], bq = mp[(long)r0 * W4 + c1];
-    const float cq = mp[(long)r1 * W4 + c0], dq = mp[(long)r1 * W4 + c1];
-    const float d = h0 * (w0 * a + w1 * bq) + h1 * (w0 * cq + w1 * dq);
+    const BilinearAxis y = bilinear_src(sh, r, H4), x = bilinear_src(sw, c, W4);
+    const float a = mp[(long)y.i0 * W4 + x.i0], bq = mp[(long)y.i0 * W4 + x.i1];
+    const float cq = mp[(long)y.i1 * W4 + x.i0], dq = mp[(long)y.i1 * W4 + x.i1];
+    const float d = y.l0 * (x.l0 * a + x.l1 * bq) + y.l1 * (x.l0 * cq + x.l1 * dq);
     m = masked_from_logit(d);
   }
   const uint32_t word = __ballot_sync(0xffffffffu, m);
   if (lane == 0) bitmap[wid] = word;
-}
-// all_masked[row] = every key of the row is masked (mask2former_head.py:825-826 fallback)
-__global__ void __launch_bounds__(256) mask_rows_full_kernel(const uint32_t* __restrict__ bitmap, int rows, int W32, int K,
-                                                             uint8_t* __restrict__ all_masked) {
-  const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (row >= rows) return;
-  int cnt = 0;
-  for (int i = lane; i < W32; i += 32) cnt += __popc(bitmap[(long)row * W32 + i]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-  if (lane == 0) all_masked[row] = (cnt == K) ? 1 : 0;
 }
 cudaError_t launch_mask_bits(const float* mask_pred, int rows, int H4, int W4, int th, int tw,
                              uint32_t* bitmap, uint8_t* all_masked, cudaStream_t s) {
@@ -251,7 +208,7 @@ cudaError_t launch_mask_bits(const float* mask_pred, int rows, int H4, int W4, i
   const int K = th * tw, W32 = (K + 31) / 32;
   const long words = (long)rows * W32;
   mask_bits_kernel<<<(unsigned)((words + 7) / 8), 256, 0, s>>>(mask_pred, words, W32, H4, W4, th, tw, bitmap);
-  mask_rows_full_kernel<<<(rows + 7) / 8, 256, 0, s>>>(bitmap, rows, W32, K, all_masked);
+  all_masked_kernel<<<(rows + 7) / 8, 256, 0, s>>>(bitmap, rows, W32, K, all_masked);
   count_launch(2);
   return cudaGetLastError();
 }

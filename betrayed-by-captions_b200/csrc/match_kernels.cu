@@ -2,6 +2,7 @@
 // masks, the Hungarian cost matrix, the point-sampled dice + BCE losses and the class-weighted cross entropy of
 // `loss_single` (open_set/models/mask2former_head.py:464-629; targets :320-390; assigner
 // open_set/assigners/mask_hungarian_assigner.py:98-125).  All fp32; HBM / latency bound gathers and reductions.
+#include "common.cuh"
 #include "kernels.h"
 
 #include <math.h>
@@ -9,19 +10,9 @@
 namespace cgg {
 namespace {
 
-__device__ __forceinline__ float warp_sum_f(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max_f(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 // block-wide sum of up to 3 values (blockDim = 256); result valid in every thread
 __device__ __forceinline__ void block_sum3(float& a, float& b, float& c, float (*sh)[3]) {
-  a = warp_sum_f(a); b = warp_sum_f(b); c = warp_sum_f(c);
+  a = warp_sum(a); b = warp_sum(b); c = warp_sum(c);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   __syncthreads();
   if (lane == 0) { sh[warp][0] = a; sh[warp][1] = b; sh[warp][2] = c; }
@@ -85,7 +76,6 @@ __global__ void __launch_bounds__(256) point_sample_bwd_kernel(const float* __re
 }
 
 __device__ __forceinline__ float softplus_f(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
-__device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-x)); }
 
 // ---- cost matrix, stage 1: per query row  sp = sum softplus(x), sg = sum sigmoid(x), log-sum-exp of the class rows;
 // per ground-truth row  gs = sum g.   One CTA per row (rows 0..Q-1 queries, Q..Q+G-1 ground truths).
@@ -96,7 +86,7 @@ __global__ void __launch_bounds__(256) match_rowstats_kernel(const float* __rest
   const int r = blockIdx.x, t = threadIdx.x;
   if (r < Q) {
     float sp = 0.f, sg = 0.f, z = 0.f;
-    for (int p = t; p < P; p += 256) { const float v = x[(long)r * P + p]; sp += softplus_f(v); sg += sigmoid_f(v); }
+    for (int p = t; p < P; p += 256) { const float v = x[(long)r * P + p]; sp += softplus_f(v); sg += sigmoid_f32(v); }
     block_sum3(sp, sg, z, sh);
     if (t == 0) { stats[r * 4 + 0] = sp; stats[r * 4 + 1] = sg; }
     if (t < 64) {                                            // warp 0: lse of cls, warp 1: lse of emb
@@ -106,10 +96,10 @@ __global__ void __launch_bounds__(256) match_rowstats_kernel(const float* __rest
         row += (long)r * C1;
         float m = -INFINITY;
         for (int c = lane; c < C1; c += 32) m = fmaxf(m, row[c]);
-        m = warp_max_f(m);
+        m = warp_max(m);
         float s = 0.f;
         for (int c = lane; c < C1; c += 32) s += expf(row[c] - m);
-        s = warp_sum_f(s);
+        s = warp_sum(s);
         if (lane == 0) stats[r * 4 + (t < 32 ? 2 : 3)] = m + logf(s);
       }
     }
@@ -140,10 +130,10 @@ __global__ void __launch_bounds__(256) match_pairs_kernel(const float* __restric
   for (int p = lane; p < P; p += 32) {
     const float v = xr[p], t = gr[p];
     xg = fmaf(v, t, xg);
-    sgd = fmaf(sigmoid_f(v), t, sgd);
+    sgd = fmaf(sigmoid_f32(v), t, sgd);
   }
-  xg = warp_sum_f(xg);
-  sgd = warp_sum_f(sgd);
+  xg = warp_sum(xg);
+  sgd = warp_sum(sgd);
   if (lane == 0) {
     const int64_t lab = labels[gi];
     float c = 0.f;
@@ -165,7 +155,7 @@ __global__ void __launch_bounds__(256) point_losses_kernel(const float* __restri
   float a = 0.f, b = 0.f, c = 0.f, e = 0.f;
   for (int p = threadIdx.x; p < P; p += 256) {
     const float v = x[n * P + p], tt = t[n * P + p];
-    const float s = sigmoid_f(v);
+    const float s = sigmoid_f32(v);
     a = fmaf(s, tt, a); b += s; c += tt;
     e += fmaxf(v, 0.f) - v * tt + log1pf(expf(-fabsf(v)));
   }
@@ -190,7 +180,7 @@ __global__ void __launch_bounds__(256) point_losses_bwd_kernel(const float* __re
   const float a = abc[n * 3], b = abc[n * 3 + 1], c = abc[n * 3 + 2];
   const float den = b + c + eps, num = 2.f * a + eps;
   const float v = x[n * P + p], tt = t[n * P + p];
-  const float s = sigmoid_f(v);
+  const float s = sigmoid_f32(v);
   const float dd_ds = (2.f * tt * den - num) / (den * den);      // d d_row / d s_p
   dx[n * P + p] = g_dice * (-dd_ds) * s * (1.f - s) + g_bce * (s - tt);
 }
@@ -206,10 +196,10 @@ __global__ void __launch_bounds__(256) weighted_ce_kernel(const float* __restric
   const float* row = logits + (long)r * C1;
   float m = -INFINITY;
   for (int c = lane; c < C1; c += 32) m = fmaxf(m, row[c]);
-  m = warp_max_f(m);
+  m = warp_max(m);
   float s = 0.f;
   for (int c = lane; c < C1; c += 32) s += expf(row[c] - m);
-  s = warp_sum_f(s);
+  s = warp_sum(s);
   if (lane == 0) {
     const int64_t lab = labels[r];
     const float l = m + logf(s), w = cw[lab];

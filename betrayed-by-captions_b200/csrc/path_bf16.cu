@@ -3,6 +3,7 @@
 // K-major activations through TMA; bias / scale / ReLU / residual + LayerNorm live in the GEMM
 // epilogues.  The decoder state x stays fp32 between layers (residual stream); only GEMM operands
 // are rounded to bf16.
+#include "common.cuh"
 #include "gemm_tc.h"
 #include "kernels.h"
 #include "tc_ptx.cuh"
@@ -15,8 +16,6 @@
 namespace cgg {
 
 namespace {
-
-inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // hi/lo bf16 pair of a float pair, packed
 __device__ __forceinline__ void split_pack(float a, float b, uint32_t& hi, uint32_t& lo) {

@@ -13,6 +13,7 @@
 // The contractions (1x1 convs, the 3x3 output conv as an implicit GEMM over 9 taps, every linear layer of the encoder) are
 // calls of cgg_gemm_f32 (gemm_tf32.cu: tcgen05 kind::tf32 fed by TMA, zero-filled out-of-bounds taps; kernels_f32.cu in the
 // fp32 parity mode).
+#include "common.cuh"
 #include "kernels.h"
 #include <math.h>
 
@@ -405,18 +406,6 @@ __global__ void __launch_bounds__(256) gn_bwd_apply_kernel(const float* __restri
 }
 
 // ------------------------------------------------------------------------------------- FPN top-down step
-// ATen upsample_bilinear2d(align_corners=False) source index: max(0, (dst + 0.5) * in/out - 0.5)
-__device__ __forceinline__ void src_index(int dst, int in, int out, int& i0, int& i1, float& l0, float& l1) {
-  const float scale = (float)in / (float)out;
-  float src = ((float)dst + 0.5f) * scale - 0.5f;
-  if (src < 0.f) src = 0.f;
-  i0 = (int)src;
-  if (i0 > in - 1) i0 = in - 1;
-  i1 = i0 + (i0 < in - 1 ? 1 : 0);
-  l1 = src - (float)i0;
-  l0 = 1.f - l1;
-}
-
 // out[b,y,x,:] = lat[b,y,x,:] + bilinear(prev[b,:,:,:])(y,x);  lat/out (B, H*W, C), prev (B, h*w, C) with batch stride pbs
 __global__ void __launch_bounds__(256) upsample_add_kernel(const float* __restrict__ lat, const float* __restrict__ prev, long pbs,
                                                            float* __restrict__ out, long total4, int H, int W, int h, int w, int C) {
@@ -428,21 +417,18 @@ __global__ void __launch_bounds__(256) upsample_add_kernel(const float* __restri
   const int x = (int)(row % W); row /= W;
   const int y = (int)(row % H);
   const int b = (int)(row / H);
-  int y0, y1, x0, x1;
-  float ly0, ly1, lx0, lx1;
-  src_index(y, h, H, y0, y1, ly0, ly1);
-  src_index(x, w, W, x0, x1, lx0, lx1);
+  const BilinearAxis ay = bilinear_src((float)h / (float)H, y, h), ax = bilinear_src((float)w / (float)W, x, w);
   const float* pb = prev + (long)b * pbs + cv * 4;
-  const float4 v00 = *reinterpret_cast<const float4*>(pb + ((long)y0 * w + x0) * C);
-  const float4 v01 = *reinterpret_cast<const float4*>(pb + ((long)y0 * w + x1) * C);
-  const float4 v10 = *reinterpret_cast<const float4*>(pb + ((long)y1 * w + x0) * C);
-  const float4 v11 = *reinterpret_cast<const float4*>(pb + ((long)y1 * w + x1) * C);
+  const float4 v00 = *reinterpret_cast<const float4*>(pb + ((long)ay.i0 * w + ax.i0) * C);
+  const float4 v01 = *reinterpret_cast<const float4*>(pb + ((long)ay.i0 * w + ax.i1) * C);
+  const float4 v10 = *reinterpret_cast<const float4*>(pb + ((long)ay.i1 * w + ax.i0) * C);
+  const float4 v11 = *reinterpret_cast<const float4*>(pb + ((long)ay.i1 * w + ax.i1) * C);
   const float4 l = reinterpret_cast<const float4*>(lat)[i];
   float4 o;
-  o.x = l.x + (ly0 * (lx0 * v00.x + lx1 * v01.x) + ly1 * (lx0 * v10.x + lx1 * v11.x));
-  o.y = l.y + (ly0 * (lx0 * v00.y + lx1 * v01.y) + ly1 * (lx0 * v10.y + lx1 * v11.y));
-  o.z = l.z + (ly0 * (lx0 * v00.z + lx1 * v01.z) + ly1 * (lx0 * v10.z + lx1 * v11.z));
-  o.w = l.w + (ly0 * (lx0 * v00.w + lx1 * v01.w) + ly1 * (lx0 * v10.w + lx1 * v11.w));
+  o.x = l.x + (ay.l0 * (ax.l0 * v00.x + ax.l1 * v01.x) + ay.l1 * (ax.l0 * v10.x + ax.l1 * v11.x));
+  o.y = l.y + (ay.l0 * (ax.l0 * v00.y + ax.l1 * v01.y) + ay.l1 * (ax.l0 * v10.y + ax.l1 * v11.y));
+  o.z = l.z + (ay.l0 * (ax.l0 * v00.z + ax.l1 * v01.z) + ay.l1 * (ax.l0 * v10.z + ax.l1 * v11.z));
+  o.w = l.w + (ay.l0 * (ax.l0 * v00.w + ax.l1 * v01.w) + ay.l1 * (ax.l0 * v10.w + ax.l1 * v11.w));
   reinterpret_cast<float4*>(out)[i] = o;
 }
 
@@ -457,16 +443,13 @@ __global__ void __launch_bounds__(256) upsample_add_bwd_kernel(const float* __re
   const int x = (int)(row % W); row /= W;
   const int y = (int)(row % H);
   const int b = (int)(row / H);
-  int y0, y1, x0, x1;
-  float ly0, ly1, lx0, lx1;
-  src_index(y, h, H, y0, y1, ly0, ly1);
-  src_index(x, w, W, x0, x1, lx0, lx1);
+  const BilinearAxis ay = bilinear_src((float)h / (float)H, y, h), ax = bilinear_src((float)w / (float)W, x, w);
   const float4 d = reinterpret_cast<const float4*>(dout)[i];
   float* pb = dprev + (long)b * h * w * C + cv * 4;
   auto add = [&](int yy, int xx, float wgt) {
     atomicAdd(reinterpret_cast<float4*>(pb + ((long)yy * w + xx) * C), make_float4(wgt * d.x, wgt * d.y, wgt * d.z, wgt * d.w));
   };
-  add(y0, x0, ly0 * lx0); add(y0, x1, ly0 * lx1); add(y1, x0, ly1 * lx0); add(y1, x1, ly1 * lx1);
+  add(ay.i0, ax.i0, ay.l0 * ax.l0); add(ay.i0, ax.i1, ay.l0 * ax.l1); add(ay.i1, ax.i0, ay.l1 * ax.l0); add(ay.i1, ax.i1, ay.l1 * ax.l1);
 }
 
 // ------------------------------------------------------------------------------------- layout changes

@@ -7,6 +7,7 @@
 // instance_mask_stats_kernel does all of it in ONE pass that reads only the (B, Q, H/4, W/4) logits: the full-resolution
 // logits are never written.  Both resampling stages follow ATen's upsample_bilinear2d index math and operation order
 // (src = scale (dst + 0.5) - 0.5 clamped at 0; v = h0 (w0 a + w1 b) + h1 (w0 c + w1 d)), evaluated in fp32.
+#include "common.cuh"
 #include "kernels.h"
 #include <cuda_bf16.h>
 #include <limits.h>
@@ -16,27 +17,13 @@ namespace cgg {
 
 namespace {
 
-struct Axis { int i0, i1; float l0, l1; };
-
-__device__ __forceinline__ Axis src_axis(float scale, int dst, int in_size) {
-  float src = scale * ((float)dst + 0.5f) - 0.5f;
-  if (src < 0.f) src = 0.f;
-  Axis a;
-  a.i0 = (int)src;
-  if (a.i0 > in_size - 1) a.i0 = in_size - 1;
-  a.i1 = a.i0 + ((a.i0 < in_size - 1) ? 1 : 0);
-  a.l1 = src - (float)a.i0;
-  a.l0 = 1.f - a.l1;
-  return a;
-}
-
 template <typename T> __device__ __forceinline__ float ldf(const T* p);
 template <> __device__ __forceinline__ float ldf<float>(const float* p) { return __ldg(p); }
 template <> __device__ __forceinline__ float ldf<__nv_bfloat16>(const __nv_bfloat16* p) { return __bfloat162float(*p); }
 
 // value of the first-stage upsample (logits (h4, w4) -> (up_h, up_w)) at (y, x) given precomputed axes
 template <typename T>
-__device__ __forceinline__ float up1(const T* __restrict__ src, int w4, const Axis& ay, const Axis& ax) {
+__device__ __forceinline__ float up1(const T* __restrict__ src, int w4, const BilinearAxis& ay, const BilinearAxis& ax) {
   const float a = ldf(src + (long)ay.i0 * w4 + ax.i0), b = ldf(src + (long)ay.i0 * w4 + ax.i1);
   const float c = ldf(src + (long)ay.i1 * w4 + ax.i0), d = ldf(src + (long)ay.i1 * w4 + ax.i1);
   return ay.l0 * (ax.l0 * a + ax.l1 * b) + ay.l1 * (ax.l0 * c + ax.l1 * d);
@@ -45,8 +32,9 @@ __device__ __forceinline__ float up1(const T* __restrict__ src, int w4, const Ax
 // value of the two-stage resample (logits -> (up_h, up_w) -> crop -> (out_h, out_w)) at an output pixel whose second-stage
 // axes are (by, bx) and whose first-stage axes at the two source rows / columns are (ay0, ay1) / (ax0, ax1)
 template <typename T>
-__device__ __forceinline__ float up2(const T* __restrict__ src, int w4, const Axis& by, const Axis& ay0, const Axis& ay1,
-                                     const Axis& bx, const Axis& ax0, const Axis& ax1) {
+__device__ __forceinline__ float up2(const T* __restrict__ src, int w4, const BilinearAxis& by, const BilinearAxis& ay0,
+                                     const BilinearAxis& ay1, const BilinearAxis& bx, const BilinearAxis& ax0,
+                                     const BilinearAxis& ax1) {
   const float a = up1(src, w4, ay0, ax0), bb = up1(src, w4, ay0, ax1);
   const float c = up1(src, w4, ay1, ax0), d = up1(src, w4, ay1, ax1);
   return by.l0 * (bx.l0 * a + bx.l1 * bb) + by.l1 * (bx.l0 * c + bx.l1 * d);
@@ -60,10 +48,10 @@ __global__ void __launch_bounds__(256) upsample_kernel(const T* __restrict__ log
   const long plane = blockIdx.z;
   if (x >= up_w) return;
   const float sy = (float)h4 / (float)up_h, sx = (float)w4 / (float)up_w;
-  const Axis ax = src_axis(sx, x, w4);
+  const BilinearAxis ax = bilinear_src(sx, x, w4);
   const T* src = logits + plane * (long)h4 * w4;
   for (int y = y0; y < y0 + 8 && y < up_h; ++y) {
-    const Axis ay = src_axis(sy, y, h4);
+    const BilinearAxis ay = bilinear_src(sy, y, h4);
     out[(plane * up_h + y) * (long)up_w + x] = up1(src, w4, ay, ax);
   }
 }
@@ -89,27 +77,27 @@ __global__ void __launch_bounds__(256) instance_mask_stats_kernel(const T* __res
   const bool x_ok = x < out_w;
   const int xc = x_ok ? x : out_w - 1;
   // x axes: second stage (out -> crop) and, for its two source columns, first stage (up -> logits)
-  Axis bx = {xc, xc, 1.f, 0.f};
-  if (rescale) bx = src_axis(s2x, xc, crop_w);
-  const Axis ax0 = src_axis(s1x, bx.i0, w4), ax1 = src_axis(s1x, bx.i1, w4);
+  BilinearAxis bx = {xc, xc, 1.f, 0.f};
+  if (rescale) bx = bilinear_src(s2x, xc, crop_w);
+  const BilinearAxis ax0 = bilinear_src(s1x, bx.i0, w4), ax1 = bilinear_src(s1x, bx.i1, w4);
   const T* src = logits + (long)plane * h4 * w4;
   int cnt = 0, xmin = INT_MAX, xmax = -1, ymin = INT_MAX, ymax = -1;
   float ssum = 0.f;
   for (int y = y_begin; y < y_begin + ROWS_PER_BLOCK && y < out_h; ++y) {
     float v;
     if (rescale) {
-      const Axis by = src_axis(s2y, y, crop_h);
-      const Axis ay0 = src_axis(s1y, by.i0, h4), ay1 = src_axis(s1y, by.i1, h4);
+      const BilinearAxis by = bilinear_src(s2y, y, crop_h);
+      const BilinearAxis ay0 = bilinear_src(s1y, by.i0, h4), ay1 = bilinear_src(s1y, by.i1, h4);
       v = up2(src, w4, by, ay0, ay1, bx, ax0, ax1);
     } else {
-      v = up1(src, w4, src_axis(s1y, y, h4), ax0);
+      v = up1(src, w4, bilinear_src(s1y, y, h4), ax0);
     }
     const bool pos = x_ok && v > 0.f;
     const uint32_t word = __ballot_sync(0xffffffffu, pos);
     if (bits && lane == 0) bits[(long)plane * bits_plane + (long)y * bits_w32 + strip] = word;
     if (pos) {
       ++cnt;
-      ssum += 1.0f / (1.0f + expf(-v));
+      ssum += sigmoid_f32(v);
       xmin = min(xmin, x); xmax = max(xmax, x);
       ymin = min(ymin, y); ymax = max(ymax, y);
     }
@@ -261,10 +249,10 @@ __global__ void __launch_bounds__(256) pan_pixel_kernel(const T* __restrict__ lo
   const int x = x0 + lane;
   const bool x_ok = x < out_w;
   const int xc = x_ok ? x : out_w - 1;
-  Axis bx = {xc, xc, 1.f, 0.f};
-  if (rescale) bx = src_axis(s2x, xc, crop_w);
-  const Axis ax0 = src_axis(s1x, bx.i0, w4), ax1 = src_axis(s1x, bx.i1, w4);
-  Axis by[PAN_ROWS], ay0[PAN_ROWS], ay1[PAN_ROWS];
+  BilinearAxis bx = {xc, xc, 1.f, 0.f};
+  if (rescale) bx = bilinear_src(s2x, xc, crop_w);
+  const BilinearAxis ax0 = bilinear_src(s1x, bx.i0, w4), ax1 = bilinear_src(s1x, bx.i1, w4);
+  BilinearAxis by[PAN_ROWS], ay0[PAN_ROWS], ay1[PAN_ROWS];
   bool ok[PAN_ROWS];
   float best[PAN_ROWS];
   int code[PAN_ROWS];
@@ -273,10 +261,10 @@ __global__ void __launch_bounds__(256) pan_pixel_kernel(const T* __restrict__ lo
     const int y = y0 + ty + 8 * r;
     ok[r] = x_ok && y < out_h;
     const int yc = y < out_h ? y : out_h - 1;
-    by[r] = Axis{yc, yc, 1.f, 0.f};
-    if (rescale) by[r] = src_axis(s2y, yc, crop_h);
-    ay0[r] = src_axis(s1y, by[r].i0, h4);
-    ay1[r] = src_axis(s1y, by[r].i1, h4);
+    by[r] = BilinearAxis{yc, yc, 1.f, 0.f};
+    if (rescale) by[r] = bilinear_src(s2y, yc, crop_h);
+    ay0[r] = bilinear_src(s1y, by[r].i0, h4);
+    ay1[r] = bilinear_src(s1y, by[r].i1, h4);
     best[r] = -1.f;
     code[r] = -1;
   }
@@ -287,7 +275,7 @@ __global__ void __launch_bounds__(256) pan_pixel_kernel(const T* __restrict__ lo
 #pragma unroll
     for (int r = 0; r < PAN_ROWS; ++r) {
       const float v = rescale ? up2(src, w4, by[r], ay0[r], ay1[r], bx, ax0, ax1) : up1(src, w4, ay0[r], ax0);
-      const float sg = 1.0f / (1.0f + expf(-v));
+      const float sg = sigmoid_f32(v);
       const float p = sc * sg;
       const bool half = sg >= 0.5f;
       if (p > best[r]) { best[r] = p; code[r] = k | (half ? PAN_FLAG : 0); }

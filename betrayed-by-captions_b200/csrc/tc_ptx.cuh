@@ -184,6 +184,15 @@ __device__ __forceinline__ void mma_bf16_ss(uint32_t d_tmem, uint64_t adesc, uin
       ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// the same with fp32 operands read as tf32 (kind::tf32)
+__device__ __forceinline__ void mma_tf32_ss(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                            uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n"
+      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // mbarrier arrives when every previously issued tcgen05.mma of this thread has completed
 // (implies tcgen05.fence::before_thread_sync).
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
@@ -272,10 +281,15 @@ __device__ __forceinline__ void mma_commit_2sm(uint64_t* bar) {
 // ------------------------------------------------------------------ UMMA descriptors
 // Shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout): start address
 // [0,14) >>4, leading byte offset [16,30) >>4, stride byte offset [32,46) >>4, version=1 at
-// [46,48), layout type [61,64) (2 = SWIZZLE_128B).
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+// [46,48), layout type [61,64).
+constexpr uint32_t UMMA_INTERLEAVE = 0;      // no swizzle: 8 x 16-byte core matrices
+constexpr uint32_t UMMA_SW128_BASE32B = 1;   // 128-byte swizzle with 32-byte atoms (32-bit MN-major operands)
+constexpr uint32_t UMMA_SW128 = 2;
+constexpr uint32_t UMMA_SW64 = 4;
+__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes,
+                                              uint32_t layout) {
   return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | (2ull << 61);
+         ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | ((uint64_t)layout << 61);
 }
 // Instruction descriptor for kind::f16 (cute::UMMA::InstrDescriptor): c_format F32 (1) at [4,6),
 // a/b format BF16 (1) at [7,10)/[10,13), a_major at 15, b_major at 16 (1 = MN-major),

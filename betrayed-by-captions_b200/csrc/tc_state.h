@@ -1,5 +1,6 @@
 // Internal state of the bf16 / tcgen05 side (shared by gemm_tc.cu and attention_tc.cu).
 #pragma once
+#include "common.cuh"
 #include "gemm_tc.h"
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -52,7 +53,7 @@ struct TcWs {
   size_t me_all, fds[3], memp[3], xqb, xb, ob, fb, zb, h1b, h2b, qf, qs, kvs, x1, x2, t1, total;
   void carve(const TcState* t, int B) {
     size_t off = 0;
-    auto take = [&](size_t b) { size_t o = off; off += (b + 255) & ~(size_t)255; return o; };
+    auto take = [&](size_t b) { size_t o = off; off += align256(b); return o; };
     const int C = t->cfg.embed_dim;
     const size_t M = (size_t)B * t->cfg.num_queries;
     me_all = take((size_t)B * t->rows_per_batch * 2 * C * 2 + 128 * 1024);   // [hi|lo] rows + 128 slack rows

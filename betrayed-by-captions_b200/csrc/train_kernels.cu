@@ -4,18 +4,13 @@
 // two gradients of the mask einsum, the K/V in-projection) go through the generic strided GEMM of kernels_f32.cu;
 // this file holds what is not a GEMM: LayerNorm backward, the masked-attention backward, ReLU masking, and the
 // forward attention variant that also returns the row log-sum-exp.
+#include "common.cuh"
 #include "kernels.h"
 #include <math.h>
 
 namespace cgg {
 
 namespace {
-
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 
 // ----------------------------------------------------------------------------------------------- LayerNorm
 // y = (x - mu) * rstd * w + b  (torch.nn.LayerNorm, biased variance).  One warp per row:
