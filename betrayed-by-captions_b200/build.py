@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libcgg_b200.so')
-SOURCES = ['kernels_f32.cu', 'train_kernels.cu', 'post_kernels.cu', 'match_kernels.cu', 'pixdec_kernels.cu', 'gemm_tc.cu', 'gemm_tf32.cu', 'attention_tc.cu', 'path_bf16.cu', 'api.cu']
+SOURCES = ['kernels_f32.cu', 'train_kernels.cu', 'post_kernels.cu', 'match_kernels.cu', 'caption_kernels.cu', 'pixdec_kernels.cu', 'gemm_tc.cu', 'gemm_tf32.cu', 'attention_tc.cu', 'path_bf16.cu', 'api.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC']
 

@@ -8,8 +8,10 @@ The module carries the reference's state_dict keys (checkpoints load unchanged);
 kernels of the C-ABI library through the autograd nodes of train.py -- every linear layer a `cgg_gemm_f32` call (tcgen05
 kind::tf32 in the tf32 training mode, fp32 FMA otherwise), the attention as the (image, head)-batched products with the
 row-softmax kernels (`_AttentionViews`: 8 heads x 96, causal + key-padding masks as a bitmap), LayerNorm, broadcast adds.
-The beam search keeps the reference's control flow (host-side candidate bookkeeping, top-k over the flattened beams) and
-runs the network in fp32 FMA mode, so that the token sequences are the reference's."""
+The beam search (`beam_search_batch`) runs every image of a batch at once on the device: the network in fp32 FMA mode with
+the self-attention keys / values of earlier tokens cached per beam, and the reference's candidate bookkeeping (top-k
+over the flattened beams, finished list, max_idx) in the kernels of csrc/caption_kernels.cu, so that each image's token
+sequences are the ones the reference's search produces for it alone."""
 import math
 
 import numpy as np
@@ -18,7 +20,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import lib as _lib
-from .train import _K, _Linear, _LayerNorm, _AddRows, _AttentionViews
+from .train import _K, _Linear, _LayerNorm, _AddRows, _AttentionViews, _p
 
 BOS_TOKEN, EOS_TOKEN = 101, 102             # bert-base-uncased [CLS] / [SEP] (mask2former_head.py:30-31)
 
@@ -114,6 +116,8 @@ class CaptionTransformerB200(nn.Module):
         like caption_tranformer.py:38-43.  `exact`: fp32 FMA contractions whatever the training precision (beam search)."""
         if memory_mask is not None or memory_key_padding_mask is not None or tgt_mask is not None:
             raise _lib.CggError('only the causal tgt mask + tgt_key_padding_mask form the reference uses is built')
+        if memory.shape[0] != tgt.shape[0]:
+            raise _lib.CggError('memory has %d images, tgt %d' % (memory.shape[0], tgt.shape[0]))
         if not tgt.is_cuda:
             raise _lib.CggError('the caption transformer runs on CUDA only (no CPU fallback)')
         k = self._k(tgt.device, exact)
@@ -196,65 +200,124 @@ def caption_generation_loss(head, cls_emb_preds, gt_caption_ids_list, gt_caption
     return loss_weight * row_loss.sum() / gt.numel()
 
 
+def _pow32(x, alpha):
+    """x ** alpha as the reference applies it to an fp32 tensor: the power in double, rounded to fp32."""
+    return float(np.float32(x ** alpha))
+
+
 @torch.no_grad()
-def beam_search(head, memory, BOS=BOS_TOKEN, EOS=EOS_TOKEN, max_len=35, beam_width=7, alpha=0.7, tokenizer=None):
-    """inference.py:84-157 with the same candidate bookkeeping: returns (best sentence token ids, score, all finished
-    (ids, score) pairs); with a `tokenizer` (bert-base-uncased) also the decoded sentence as the reference returns it."""
+def _search_device(head, memory, BOS, EOS, max_len, beam_width, alpha):
+    """Issues the batched search on the current stream without waiting for the device.  Every step runs all B * W rows:
+    the new token's embedding, the decoder blocks with the self-attention keys / values of earlier positions cached per
+    beam, the generator on every block's output, the beam scores and the selection.  The host reads the done-image count
+    back asynchronously and stops issuing steps once it sees every image done.  Returns (state tensors, steps issued)."""
     gen = head.caption_generator
+    psne = gen.position_encoder.psne_layer
+    npos = psne.shape[0]
+    if memory.dim() != 3 or memory.shape[0] < 1:
+        raise _lib.CggError('memory must be (B, Q, dim) with B >= 1')
+    if not 1 <= beam_width <= 32:
+        raise _lib.CggError('beam_width must be in 1..32')
+    if not 1 <= max_len <= npos:
+        raise _lib.CggError('max_len must be in 1..%d (the position table)' % npos)
+    if not memory.is_cuda:
+        raise _lib.CggError('the caption beam search runs on CUDA only (no CPU fallback)')
     dev = memory.device
+    k = gen._k(dev, True)
+    blocks = gen.transformer_decoder.decoders
+    B, Q, W = memory.shape[0], memory.shape[1], beam_width
+    nb, D, H = len(blocks), gen.hidden_dim, gen.nb_heads
+    d, n = D // H, B * W
+    scale = 1.0 / math.sqrt(d)
+    # the BOS step, then passes while a beam may continue (length + 1 < max_len - 1): pass s sees sequences of length s + 1
+    steps = max(2, max_len - 2)
+    T = steps + 1                                                   # the longest sequence, EOS included
+    lin = lambda x, m, res=None, relu=False: _Linear.apply(k, x, m.weight, m.bias, res, 1.0, relu)     # noqa: E731
+    ln = lambda x, m: x if isinstance(m, nn.Identity) else _LayerNorm.apply(k, x, m.weight, m.bias, m.eps)   # noqa: E731
+    mem = memory.float().contiguous().view(B * Q, -1)
+    if not isinstance(gen.adapter, nn.Identity):
+        mem = lin(mem, gen.adapter)
+    # cross-attention keys / values: once per image and block, shared by the image's beams
+    kv_mem = [(lin(mem, b.crx_layer.to_key).view(B, Q, H, d), lin(mem, b.crx_layer.to_val).view(B, Q, H, d)) for b in blocks]
+    cache = [k.new(nb, 2, n, steps, D) for _ in range(2)]          # double-buffered (block, k / v, row, position, D)
+    i32 = dict(dtype=torch.int32, device=dev)
+    st = dict(tokens=torch.full((B, W, T), BOS, **i32), weights=k.new(B, W).zero_(), n_active=torch.zeros(B, **i32),
+              parent=torch.zeros((B, W), **i32), next_ids=torch.full((B, W), BOS, dtype=torch.int64, device=dev),
+              fin_tokens=torch.zeros((B, W, T), **i32), fin_len=torch.zeros((B, W), **i32), fin_score=k.new(B, W).zero_(),
+              n_fin=torch.zeros(B, **i32), max_idx=torch.zeros(B, **i32), done=torch.zeros(B, **i32),
+              n_done=torch.zeros(1, **i32))
+    state = _lib.BeamState(token_cap=T, **{name: t.data_ptr() for name, t in st.items()})
+    cand_val, cand_col = k.new(n, W), torch.empty((n, W), **i32)
+    n_done = torch.zeros(steps, dtype=torch.int32, pin_memory=True)
+    events, checked = [], 0
+    be = head.bert_embeddings
+    for s in range(steps):
+        x = head.extract_word_embeddings(be.word_embeddings.weight, be.LayerNorm.weight, be.LayerNorm.bias,
+                                         st['next_ids'].view(n), eps=be.LayerNorm.eps)
+        x = _AddRows.apply(k, x.view(n, 1, D), psne[s:s + 1], n).view(n, D)
+        kc = cache[s % 2]
+        outs = []
+        for i, blk in enumerate(blocks):
+            nz, ca = blk.layer_normalz, blk.crx_layer
+            tmp = ln(x, nz['mha'][0])
+            qkv = lin(tmp, blk.mha_layer.qkv_layer)
+            o = k.new(n, D)
+            k.chk(k.lib.cgg_caption_self_attn_step(k.h, _p(qkv), _p(kc[i, 0]), _p(kc[i, 1]), _p(o), n, H, d, s, steps, scale,
+                                                   k.s()), 'cgg_caption_self_attn_step')
+            x = ln(lin(o, blk.mha_layer.out_layer, res=tmp), nz['mha'][1])
+            tmp = ln(x, nz['crx'][0])
+            o = _AttentionViews.apply(k, lin(tmp, ca.to_qry).view(B, W, H, d), kv_mem[i][0], kv_mem[i][1], None, scale)
+            x = ln(lin(o.view(n, D), ca.to_out, res=tmp), nz['crx'][1])
+            tmp = ln(x, nz['ffn'][0])
+            f0, f1 = blk.ffn_layer.linears[0], blk.ffn_layer.linears[1]
+            x = ln(lin(lin(x, f0[0], relu=True), f1[0], res=tmp), nz['ffn'][1])
+            outs.append(x)
+        logits = lin(torch.stack(outs, 0).view(nb * n, D), gen.generator)        # the generator on every block's rows
+        first, length = int(s == 0), s + 1
+        pw, pw1 = _pow32(length, alpha), _pow32(length + 1, alpha)
+        k.chk(k.lib.cgg_caption_beam_scores(k.h, _p(logits), nb, B, W, logits.shape[1], first, state, pw,
+                                            _p(cand_val), _p(cand_col), k.s()), 'cgg_caption_beam_scores')
+        k.chk(k.lib.cgg_caption_beam_select(k.h, _p(cand_val), _p(cand_col), B, W, first, length, max_len, npos, pw, pw1,
+                                            EOS, state, k.s()), 'cgg_caption_beam_select')
+        if s + 1 < steps:
+            k.chk(k.lib.cgg_caption_cache_reorder(k.h, _p(kc), _p(cache[(s + 1) % 2]), _p(st['parent']), nb, B, W, steps,
+                                                  s + 1, D, k.s()), 'cgg_caption_cache_reorder')
+        n_done[s].copy_(st['n_done'][0], non_blocking=True)
+        events.append(torch.cuda.Event())
+        events[-1].record(torch.cuda.current_stream(dev))
+        while checked <= s and events[checked].query():
+            if int(n_done[checked]) == B:
+                return st, s + 1
+            checked += 1
+    return st, steps
 
-    def embed(ids):
-        be = head.bert_embeddings
-        return head.extract_word_embeddings(be.word_embeddings.weight, be.LayerNorm.weight, be.LayerNorm.bias, ids.to(dev),
-                                            eps=be.LayerNorm.eps)
 
-    def step_logits(batch_emb, mem):
-        outs = gen(batch_emb, mem, exact=True)[0]
-        k = gen._k(dev, True)
-        rows = torch.stack([o[:, -1, :] for o in outs], 0)                                   # (layers, n, C)
-        nl, n, C = rows.shape
-        lg = _Linear.apply(k, rows.reshape(nl * n, C).contiguous(), gen.generator.weight, gen.generator.bias, None, 1.0, False)
-        return lg.view(nl, n, -1).mean(0)                                                    # mean over the blocks' logits
+def _search_results(st, tokenizer=None):
+    """The one synchronisation of a search: its state as one dict per image (the shape `beam_search` returns)."""
+    torch.cuda.current_stream(st['n_fin'].device).synchronize()
+    n_fin, max_idx = st['n_fin'].tolist(), st['max_idx'].tolist()
+    fin_len, fin_tokens, fin_score = st['fin_len'].tolist(), st['fin_tokens'].cpu(), st['fin_score'].tolist()
+    results = []
+    for b in range(len(n_fin)):
+        finished = [(fin_tokens[b, j, :fin_len[b][j]].tolist(), fin_score[b][j]) for j in range(n_fin[b])]
+        best = finished[max_idx[b]] if finished else (None, None)
+        text = None
+        if tokenizer is not None and finished:
+            text = tokenizer.decode(best[0])[1:-1]                                           # inference.py:149-154
+        results.append(dict(ids=best[0], score=best[1], finished=finished, text=text))
+    return results
 
-    target = torch.tensor([[BOS]])
-    logits = step_logits(embed(target).view(1, 1, -1), memory)[0]
-    scaled = torch.log_softmax(logits[None, :], dim=1).cpu().squeeze(0)
-    weights, candidates = torch.topk(scaled, k=beam_width, largest=True)
-    finished, active = [], [torch.cat([target, torch.tensor([[int(i)]])], dim=1) for i in candidates]
-    max_idx = 0
-    while True:
-        max_score, max_idx = -100, 0      # reset on EVERY pass, as the reference does (inference.py:117-118): the sentence
-        #                                   returned is the best one finished in the last pass (the first one if none was)
-        batch = torch.vstack(active)
-        n = batch.shape[0]
-        mem = torch.cat([m.repeat(n, 1, 1) for m in memory], dim=0)
-        scaled = torch.log_softmax(step_logits(embed(batch).view(n, batch.shape[1], -1), mem), dim=1).cpu()
-        length, vocab = batch.shape[1], scaled.shape[1]
-        weighted = (scaled + weights[:, None]) / length ** alpha
-        weights, candidates = torch.topk(torch.flatten(weighted), k=beam_width, largest=True)
-        weights = weights * length ** alpha
-        w_next, s_next, stop = [], [], False
-        for idx, pos in enumerate(candidates):
-            row = int(torch.div(pos, vocab, rounding_mode='floor'))
-            col = int(pos % vocab)
-            seq = torch.cat([active[row], torch.tensor([[col]])], dim=1)
-            if col == EOS:
-                flat = torch.flatten(seq).tolist()
-                score = weights[idx] / len(flat) ** alpha
-                finished.append((flat, float(score)))
-                if score > max_score:
-                    max_score, max_idx = score, len(finished) - 1
-                if len(finished) == beam_width:
-                    stop = True
-                    break
-            elif seq.shape[1] < max_len - 1:
-                w_next.append(weights[row])
-                s_next.append(seq)
-        if stop or not s_next:
-            break
-        weights, active = torch.tensor(w_next), s_next
-    best = finished[max_idx] if finished else (None, None)
-    text = None
-    if tokenizer is not None and finished:
-        text = tokenizer.decode(best[0])[1:-1]                                               # inference.py:149-154
-    return dict(ids=best[0], score=best[1], finished=finished, text=text)
+
+def beam_search_batch(head, memory, BOS=BOS_TOKEN, EOS=EOS_TOKEN, max_len=35, beam_width=7, alpha=0.7, tokenizer=None):
+    """inference.py:84-157 for every image of memory (B, Q, dim) at once, on the device: one dict per image with the best
+    sentence's token ids, its score, all finished (ids, score) pairs in the reference's order and, with a `tokenizer`
+    (bert-base-uncased), the decoded sentence -- for each image what the reference's beam search returns for it alone."""
+    st, _ = _search_device(head, memory, BOS, EOS, max_len, beam_width, alpha)
+    return _search_results(st, tokenizer)
+
+
+def beam_search(head, memory, BOS=BOS_TOKEN, EOS=EOS_TOKEN, max_len=35, beam_width=7, alpha=0.7, tokenizer=None):
+    """The beam search of one image (memory (1, Q, dim)): `beam_search_batch(...)[0]`."""
+    if memory.dim() != 3 or memory.shape[0] != 1:
+        raise _lib.CggError('beam_search takes one image (memory (1, Q, dim)); use beam_search_batch for a batch')
+    return beam_search_batch(head, memory, BOS, EOS, max_len, beam_width, alpha, tokenizer)[0]

@@ -1061,3 +1061,68 @@ extern "C" int cgg_nchw_to_tokens(cgg_handle* h, const float* in, float* tokens,
   CU(launch_nchw_to_tokens(in, tokens, token_batch_stride, batch, pixels, channels, accumulate != 0, (cudaStream_t)stream));
   return CGG_OK;
 }
+
+// ====================================================================== test-time caption generation (beam search)
+namespace {
+int check_beam_state(cgg_handle* h, const cgg_beam_state* st) {
+  if (!st || !st->tokens || !st->weights || !st->n_active || !st->parent || !st->next_ids || !st->fin_tokens ||
+      !st->fin_len || !st->fin_score || !st->n_fin || !st->max_idx || !st->done || !st->n_done)
+    return CGG_ERR_NULL;
+  if (st->token_cap < 2) return fail(h, CGG_ERR_BAD_SHAPE, "token_cap must be at least 2");
+  return CGG_OK;
+}
+int check_beams(cgg_handle* h, int batch, int beam_width) {
+  if (beam_width < 1 || beam_width > 32) return fail(h, CGG_ERR_BAD_SHAPE, "beam_width must be in 1..32");
+  if (batch < 1 || (long)batch * beam_width > 65535) return fail(h, CGG_ERR_BAD_SHAPE, "bad batch");
+  return CGG_OK;
+}
+}  // namespace
+
+extern "C" int cgg_caption_self_attn_step(cgg_handle* h, const float* qkv, float* k_cache, float* v_cache, float* out,
+                                          int rows, int heads, int head_dim, int t, int cache_len, float scale,
+                                          void* stream) {
+  if (!h || !qkv || !k_cache || !v_cache || !out) return CGG_ERR_NULL;
+  if (rows < 1 || rows > 0x7fffffff / 2 || heads < 1 || heads > 65535 || head_dim < 1 || cache_len < 1 || t < 0 ||
+      t >= cache_len || head_dim + cache_len > 12288)
+    return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  CU(launch_caption_self_attn(qkv, k_cache, v_cache, out, rows, heads, head_dim, t, cache_len, scale, (cudaStream_t)stream));
+  return CGG_OK;
+}
+
+extern "C" int cgg_caption_cache_reorder(cgg_handle* h, const float* src, float* dst, const int* parent, int blocks, int batch,
+                                         int beam_width, int cache_len, int positions, int dim, void* stream) {
+  if (!h || !src || !dst || !parent) return CGG_ERR_NULL;
+  ST(check_beams(h, batch, beam_width));
+  if (blocks < 1 || 2 * blocks > 65535 || cache_len < 1 || positions < 1 || positions > cache_len || dim < 4 || dim % 4)
+    return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  CU(launch_caption_cache_reorder(src, dst, parent, blocks, batch * beam_width, beam_width, cache_len, positions, dim,
+                                  (cudaStream_t)stream));
+  return CGG_OK;
+}
+
+extern "C" int cgg_caption_beam_scores(cgg_handle* h, float* logits, int blocks, int batch, int beam_width, int vocab,
+                                       int first, const cgg_beam_state* state, float pow_len, float* cand_val, int* cand_col,
+                                       void* stream) {
+  if (!h || !logits || !cand_val || !cand_col) return CGG_ERR_NULL;
+  ST(check_beam_state(h, state));
+  ST(check_beams(h, batch, beam_width));
+  if (blocks < 1 || vocab < beam_width) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  CU(launch_beam_scores(logits, blocks, batch * beam_width, vocab, beam_width, first != 0, *state, pow_len, cand_val, cand_col,
+                        (cudaStream_t)stream));
+  return CGG_OK;
+}
+
+extern "C" int cgg_caption_beam_select(cgg_handle* h, const float* cand_val, const int* cand_col, int batch, int beam_width,
+                                       int first, int length, int max_len, int num_positions, float pow_len, float pow_len1,
+                                       int eos, const cgg_beam_state* state, void* stream) {
+  if (!h || !cand_val || !cand_col) return CGG_ERR_NULL;
+  ST(check_beam_state(h, state));
+  ST(check_beams(h, batch, beam_width));
+  if (max_len < 1 || num_positions < 1 || max_len > num_positions)
+    return fail(h, CGG_ERR_BAD_SHAPE, "max_len must be in 1..num_positions (the position table's rows)");
+  if (length < 1 || length + 1 > state->token_cap || beam_width * state->token_cap > BEAM_SELECT_MAX_TOKENS)
+    return fail(h, CGG_ERR_BAD_SHAPE, "bad length / token_cap");
+  CU(launch_beam_select(cand_val, cand_col, batch, beam_width, first != 0, length, max_len, pow_len, pow_len1, eos, *state,
+                        (cudaStream_t)stream));
+  return CGG_OK;
+}

@@ -5,6 +5,8 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+struct cgg_beam_state;   // include/cgg_b200.h
+
 namespace cgg {
 
 // launch counter (cgg_launch_count)
@@ -156,6 +158,22 @@ cudaError_t launch_panoptic_fuse(const void* logits, bool bf16, const float* pro
                                  int num_things, int h4, int w4, int up_h, int up_w, int max_out_h, int max_out_w,
                                  double object_mask_thr, double iou_thr, bool filter_low_score, int* pan, int* mask_area,
                                  int* original_area, int* seg_value, void* scratch, cudaStream_t s);
+
+// ---- test-time caption beam search (caption_kernels.cu)
+// cached self-attention step: qkv (rows, heads x [q | k | v]), caches (rows, cache_len, heads * hd), new key at position t
+cudaError_t launch_caption_self_attn(const float* qkv, float* k_cache, float* v_cache, float* out, int rows, int heads, int hd,
+                                     int t, int cache_len, float scale, cudaStream_t s);
+// caches (blocks, 2, rows, cache_len, dim): positions [0, positions) of each row copied from its parent beam's row
+cudaError_t launch_caption_cache_reorder(const float* src, float* dst, const int* parent, int blocks, int rows, int W,
+                                         int cache_len, int positions, int dim, cudaStream_t s);
+cudaError_t launch_beam_scores(float* logits, int blocks, int rows, int V, int W, bool first, const cgg_beam_state& st,
+                               float pow_len, float* cand_val, int* cand_col, cudaStream_t s);
+// beam_select_kernel stages beam_width * token_cap ints in dynamic shared memory; with its static shared memory (at most
+// BEAM_SELECT_STATIC_SMEM bytes) that stays within the default 48 KiB a launch may use without an opt-in
+constexpr int BEAM_SELECT_STATIC_SMEM = 1024;
+constexpr int BEAM_SELECT_MAX_TOKENS = (48 * 1024 - BEAM_SELECT_STATIC_SMEM) / 4;
+cudaError_t launch_beam_select(const float* cand_val, const int* cand_col, int B, int W, bool first, int length, int max_len,
+                               float pow_len, float pow_len1, int eos, const cgg_beam_state& st, cudaStream_t s);
 
 // fp32 (rows, cols) -> bf16 (rows, 2*cols) hi/lo pairs: [hi | lo] per row
 cudaError_t launch_cast_bf16_split(const float* in, __nv_bfloat16* out, int rows, int cols, cudaStream_t s);

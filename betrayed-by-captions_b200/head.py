@@ -303,7 +303,8 @@ class Mask2FormerHeadOpenB200(nn.Module):
         input size, optional query x noun attention `att`, optional test-time label assignment (`gt_labels` / `gt_masks`:
         the Hungarian assignment of `_get_target_single`, cgg_b200/matching.py) and caption generation (`with_caption` /
         'cap_results': the beam search of cgg_b200/caption.py; the sentence text when `self.tokenizer` is set -- the
-        reference downloads bert-base-uncased's tokenizer for that -- otherwise its token ids)."""
+        reference downloads bert-base-uncased's tokenizer for that -- otherwise its token ids; for a batch of B > 1
+        images, a list of B such results)."""
         from .postprocess import upsample_masks
         all_cls_scores, all_cls_emb_preds, all_mask_preds = self(feats, img_metas)
         mask_cls_results, mask_cls_emb_results, mask_pred_results = all_cls_scores[-1], all_cls_emb_preds[-1], all_mask_preds[-1]
@@ -329,9 +330,11 @@ class Mask2FormerHeadOpenB200(nn.Module):
         if kwargs.get('with_caption', False) or 'cap_results' in self.test_cfg.get('eval_types', []):     # :966-970
             if self.caption_generator is None:
                 raise _lib.CggError('with_caption needs a head built with caption_generator=dict(...)')
-            from .caption import beam_search
-            res = beam_search(self, mask_cls_emb_results.float(), max_len=35, beam_width=7, tokenizer=self.tokenizer)
-            caption_generation_results = res['text'] if self.tokenizer is not None else res['ids']
+            from .caption import beam_search_batch
+            res = beam_search_batch(self, mask_cls_emb_results.float(), max_len=35, beam_width=7, tokenizer=self.tokenizer)
+            caption_generation_results = [r['text'] if self.tokenizer is not None else r['ids'] for r in res]
+            if len(res) == 1:                          # one image: the reference's return value
+                caption_generation_results = caption_generation_results[0]
         att = None
         if kwargs.get('with_att', False):                                                               # :973-978
             ids = kwargs['nouns_ids']

@@ -23,7 +23,8 @@ EXPORTS = ['cgg_create', 'cgg_destroy', 'cgg_last_error', 'cgg_version', 'cgg_la
            'cgg_matching_cost', 'cgg_point_losses', 'cgg_point_losses_backward', 'cgg_weighted_ce', 'cgg_weighted_ce_backward',
            # test-time step after the path
            'cgg_upsample_masks', 'cgg_instance_mask_stats', 'cgg_softmax_rows', 'cgg_panoptic_scratch_bytes',
-           'cgg_panoptic_fuse',
+           'cgg_panoptic_fuse', 'cgg_caption_self_attn_step', 'cgg_caption_cache_reorder', 'cgg_caption_beam_scores',
+           'cgg_caption_beam_select',
            # the pixel decoder before the path
            'cgg_ms_deform_attn', 'cgg_ms_deform_attn_backward', 'cgg_group_norm_scratch_bytes', 'cgg_group_norm_tokens',
            'cgg_group_norm_tokens_backward', 'cgg_upsample_add_tokens', 'cgg_upsample_add_tokens_backward',
@@ -60,6 +61,13 @@ class GemmDesc(C.Structure):
                 ('M', C.c_int), ('N', C.c_int), ('K', C.c_int), ('batch', C.c_int),
                 ('relu', C.c_int), ('alpha', C.c_float), ('a_mmajor', C.c_int), ('c_mmajor', C.c_int), ('tf32', C.c_int),
                 ('batch_inner', C.c_int), ('sAb2', C.c_long), ('sWb2', C.c_long), ('sCb2', C.c_long), ('accumulate', C.c_int), ('slot', C.c_int), ('conv_cin', C.c_int)]
+
+
+class BeamState(C.Structure):
+    """cgg_beam_state (include/cgg_b200.h): device pointers of a batched caption beam search"""
+    _fields_ = [('tokens', C.c_void_p), ('token_cap', C.c_int)] + \
+               [(n, C.c_void_p) for n in ('weights', 'n_active', 'parent', 'next_ids', 'fin_tokens', 'fin_len', 'fin_score',
+                                         'n_fin', 'max_idx', 'done', 'n_done')]
 
 
 class CggError(RuntimeError):
@@ -141,6 +149,11 @@ def load():
     lib.cgg_panoptic_scratch_bytes.restype = sz
     dbl = C.c_double
     lib.cgg_panoptic_fuse.argtypes = [vp, vp, i, vp, vp, i, i, i, i, i, i, i, i, i, i, dbl, dbl, i, vp, vp, vp, vp, vp, sz, vp]
+    bs = C.POINTER(BeamState)
+    lib.cgg_caption_self_attn_step.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, i, f32, vp]
+    lib.cgg_caption_cache_reorder.argtypes = [vp, vp, vp, vp, i, i, i, i, i, i, vp]
+    lib.cgg_caption_beam_scores.argtypes = [vp, vp, i, i, i, i, i, bs, f32, vp, vp, vp]
+    lib.cgg_caption_beam_select.argtypes = [vp, vp, vp, i, i, i, i, i, i, f32, f32, i, bs, vp]
     ip = C.POINTER(C.c_int)
     lib.cgg_ms_deform_attn.argtypes = [vp, vp, lg, vp, lg, vp, lg, vp, i, i, i, i, i, ip, ip, vp]
     lib.cgg_ms_deform_attn_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, ip, ip, vp]

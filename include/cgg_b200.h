@@ -380,6 +380,58 @@ int cgg_panoptic_fuse(cgg_handle *h, const void *logits, int is_bf16, const floa
                       int *mask_area, int *original_area, int *seg_value, void *scratch, size_t scratch_bytes,
                       void *stream);
 
+/* ---- test-time caption generation: the beam search of open_set/utils/eval/inference.py:84-157 ---------------------
+ * For `batch` images at once, W = beam_width beams each (1..32), rows = batch * W in (image, beam) order.  The caller runs
+ * the decoder blocks with cgg_gemm_f32 / cgg_layernorm and these four stages; nothing here synchronises with the host.
+ * Search state, device arrays (T = token_cap, the longest sequence the search can produce):
+ *   tokens (batch, W, T) int32   the active beams' token ids, BOS first
+ *   weights (batch, W) fp32      the beams' weights;  n_active (batch) int32;  parent (batch, W) int32: beam of the previous
+ *                                step each beam continues;  next_ids (batch, W) int64: the token each beam feeds next
+ *   fin_tokens (batch, W, T) int32, fin_len (batch, W) int32, fin_score (batch, W) fp32, n_fin (batch) int32: finished
+ *                                sequences in the order the reference appends them
+ *   max_idx (batch) int32: the reference's max_idx of the image's last pass (its result is fin[max_idx], if n_fin > 0)
+ *   done (batch) int32: the image's search has ended (later calls leave its state unchanged);  n_done (1) int32: count of
+ *                                done images (each image adds 1 once)
+ * A new search starts from tokens[:, :, 0] = BOS, n_fin = done = n_done = 0. */
+typedef struct cgg_beam_state {
+  int *tokens;
+  int token_cap;
+  float *weights;
+  int *n_active, *parent;
+  int64_t *next_ids;
+  int *fin_tokens, *fin_len;
+  float *fin_score;
+  int *n_fin, *max_idx, *done, *n_done;
+} cgg_beam_state;
+
+/* cgg_caption_self_attn_step: masked self-attention of one new position t with cached keys: per row and head, k and v of
+ *   qkv (rows, heads x [q | k | v] of head_dim each, the caption transformer's fused qkv_layer output) are stored at
+ *   position t of k_cache / v_cache (rows, cache_len, heads * head_dim), then softmax(scale q k^T) v over positions 0..t
+ *   -> out (rows, heads * head_dim).  t < cache_len; head_dim + cache_len <= 12288.
+ * cgg_caption_cache_reorder: src / dst caches (blocks, 2 [k, v], rows, cache_len, dim): dst[., ., image * W + w, p] =
+ *   src[., ., image * W + parent[image * W + w], p] for p < positions (dim % 4 == 0).
+ * cgg_caption_beam_scores: logits (blocks, rows, vocab), the generator applied to every block's output.  For each row of
+ *   an image that is not done and a beam < n_active (first != 0: beam 0 only): logp = log_softmax(mean over blocks), the
+ *   score logp (first) or (logp + weights[row]) / pow_len, and the row's top W scores in torch.topk order (descending,
+ *   ties to the lower column) -> cand_val / cand_col (rows, W).  Overwrites block 0 of logits.  vocab >= W.
+ * cgg_caption_beam_select: per image, the flattened top W of its active rows' candidates (flat index row * vocab + col,
+ *   torch.topk order) and the reference's bookkeeping.  first != 0 (the BOS step, length 1): the W picks become the
+ *   beams [BOS, c] with weight log p.  Otherwise, with the picks' weights = score * pow_len and in rank order: EOS
+ *   appends (sequence + EOS, weights[k] / pow_len1) to the finished list, the walk stops at W finished; another token
+ *   continues if length + 1 < max_len - 1 with weight weights[parent row]; the image is done on the stop or when no
+ *   beam continues.  pow_len = fp32(length ** alpha), pow_len1 = fp32((length + 1) ** alpha), alpha in double as the
+ *   reference computes them.  max_len <= num_positions (the position table's rows), length + 1 <= token_cap,
+ *   W * token_cap <= 12032.  Bad sizes: CGG_ERR_BAD_SHAPE. */
+int cgg_caption_self_attn_step(cgg_handle *h, const float *qkv, float *k_cache, float *v_cache, float *out, int rows,
+                               int heads, int head_dim, int t, int cache_len, float scale, void *stream);
+int cgg_caption_cache_reorder(cgg_handle *h, const float *src, float *dst, const int *parent, int blocks, int batch,
+                              int beam_width, int cache_len, int positions, int dim, void *stream);
+int cgg_caption_beam_scores(cgg_handle *h, float *logits, int blocks, int batch, int beam_width, int vocab, int first,
+                            const cgg_beam_state *state, float pow_len, float *cand_val, int *cand_col, void *stream);
+int cgg_caption_beam_select(cgg_handle *h, const float *cand_val, const int *cand_col, int batch, int beam_width,
+                            int first, int length, int max_len, int num_positions, float pow_len, float pow_len1,
+                            int eos, const cgg_beam_state *state, void *stream);
+
 /* ---- the step before the path: mmdet MSDeformAttnPixelDecoder (SURVEY.md 8f rank 3) ------------------------------
  * `mask_features, multi_scale_memorys = self.pixel_decoder(feats)` (mask2former_head.py:787; configured at
  * configs/instance/coco_b48n17.py:38-70).  mmdet 2.28.2 / mmcv-full 1.7.1 are un-vendored dependencies of the reference;
