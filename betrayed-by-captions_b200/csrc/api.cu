@@ -871,6 +871,25 @@ extern "C" int cgg_point_sample_backward(cgg_handle* h, const float* dout, const
   return CGG_OK;
 }
 
+extern "C" int cgg_panoptic_stuff_labels(cgg_handle* h, const void* sem, int sem_is_i64, int batch, int hs, int ws,
+                                         int num_things, int num_classes, uint32_t* bitmap, int64_t* stuff_labels, int* counts,
+                                         void* stream) {
+  if (!h || !sem || !bitmap || !stuff_labels || !counts) return CGG_ERR_NULL;
+  if (batch < 1 || hs < 1 || ws < 1 || num_things < 0 || num_classes <= num_things || num_classes - num_things > 8192)
+    return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  CU(launch_panoptic_stuff_labels(sem, sem_is_i64 != 0, batch, (long)hs * ws, num_things, num_classes, bitmap, stuff_labels,
+                                  counts, (cudaStream_t)stream));
+  return CGG_OK;
+}
+
+extern "C" int cgg_gt_point_sample(cgg_handle* h, const cgg_gt_image* images, const int* rows, const float* coords, float* out,
+                                   int num_rows, int num_points, int coords_per_image, void* stream) {
+  if (!h || !images || !rows || !coords || !out) return CGG_ERR_NULL;
+  if (num_rows < 0 || num_points < 0) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  CU(launch_gt_point_sample(images, rows, coords, out, num_rows, num_points, coords_per_image != 0, (cudaStream_t)stream));
+  return CGG_OK;
+}
+
 extern "C" int cgg_matching_cost(cgg_handle* h, const float* mask_points, const float* gt_points, const float* cls_scores,
                                  const float* cls_emb_logits, const int64_t* gt_labels, int num_q, int num_gt, int classes_p1,
                                  int num_points, float w_cls, float w_cls_emb, float w_mask, float w_dice, float dice_eps,

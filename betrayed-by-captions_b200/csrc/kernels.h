@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 struct cgg_beam_state;   // include/cgg_b200.h
+struct cgg_gt_image;     // include/cgg_b200.h
 
 namespace cgg {
 
@@ -123,6 +124,12 @@ cudaError_t launch_point_losses(const float* x, const float* t, int N, int P, fl
                                 float* bce_rows, cudaStream_t s);
 cudaError_t launch_point_losses_bwd(const float* x, const float* t, const float* abc, int N, int P, float eps,
                                     const float* g_dice, const float* g_bce, float* dx, cudaStream_t s);
+// panoptic targets: ascending stuff labels (B, num_classes - num_things) and counts (B,) of the semantic maps (B, pixels);
+// bitmap: B * ceil(num_stuff / 32) words of scratch.  Ground-truth point samples of (image, target) rows -> out (R, P)
+cudaError_t launch_panoptic_stuff_labels(const void* sem, bool sem_i64, int B, long pixels, int num_things, int num_classes,
+                                         uint32_t* bitmap, int64_t* labels, int* counts, cudaStream_t s);
+cudaError_t launch_gt_point_sample(const cgg_gt_image* images, const int* rows, const float* coords, float* out, int R, int P,
+                                   bool coords_per_image, cudaStream_t s);
 cudaError_t launch_weighted_ce(const float* logits, const int64_t* labels, const float* cw, int R, int C1, float* row_loss,
                                float* row_w, float* lse, cudaStream_t s);
 cudaError_t launch_weighted_ce_bwd(const float* logits, const int64_t* labels, const float* cw, const float* lse, int R, int C1,

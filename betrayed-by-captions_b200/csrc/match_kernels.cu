@@ -2,10 +2,15 @@
 // masks, the Hungarian cost matrix, the point-sampled dice + BCE losses and the class-weighted cross entropy of
 // `loss_single` (open_set/models/mask2former_head.py:464-629; targets :320-390; assigner
 // open_set/assigners/mask_hungarian_assigner.py:98-125).  All fp32; HBM / latency bound gathers and reductions.
+// Panoptic training targets (mmdet MaskFormerHead.preprocess_gt) stay compact: the stuff labels of each semantic map are
+// found on the device, and ground-truth point samples are read from the unpadded things planes and the semantic map.
+#include "../../include/cgg_b200.h"
 #include "common.cuh"
 #include "kernels.h"
 
 #include <math.h>
+
+#include <algorithm>
 
 namespace cgg {
 namespace {
@@ -37,6 +42,18 @@ __device__ __forceinline__ Taps taps_of(float px, float py, int H, int W) {
   t.se = (ix - fx) * (iy - fy);
   return t;
 }
+// the zero-padded bilinear sum of the four taps in ATen's order; at(y, x) reads the plane inside (H, W)
+template <class At>
+__device__ __forceinline__ float sample_taps(const Taps& t, int H, int W, At at) {
+  const bool x0 = t.x0 >= 0 && t.x0 < W, x1 = t.x0 + 1 >= 0 && t.x0 + 1 < W;
+  const bool y0 = t.y0 >= 0 && t.y0 < H, y1 = t.y0 + 1 >= 0 && t.y0 + 1 < H;
+  float acc = 0.f;
+  if (y0 && x0) acc += at(t.y0, t.x0) * t.nw;
+  if (y0 && x1) acc += at(t.y0, t.x0 + 1) * t.ne;
+  if (y1 && x0) acc += at(t.y0 + 1, t.x0) * t.sw;
+  if (y1 && x1) acc += at(t.y0 + 1, t.x0 + 1) * t.se;
+  return acc;
+}
 __global__ void __launch_bounds__(256) point_sample_kernel(const float* __restrict__ in, const float* __restrict__ coords,
                                                            float* __restrict__ out, int N, int H, int W, int P,
                                                            int coords_shared) {
@@ -47,14 +64,7 @@ __global__ void __launch_bounds__(256) point_sample_kernel(const float* __restri
   const float* c = coords + ((coords_shared ? 0 : n) * P + p) * 2;
   const Taps t = taps_of(c[0], c[1], H, W);
   const float* plane = in + n * H * W;
-  const bool x0 = t.x0 >= 0 && t.x0 < W, x1 = t.x0 + 1 >= 0 && t.x0 + 1 < W;
-  const bool y0 = t.y0 >= 0 && t.y0 < H, y1 = t.y0 + 1 >= 0 && t.y0 + 1 < H;
-  float acc = 0.f;
-  if (y0 && x0) acc += plane[(long)t.y0 * W + t.x0] * t.nw;
-  if (y0 && x1) acc += plane[(long)t.y0 * W + t.x0 + 1] * t.ne;
-  if (y1 && x0) acc += plane[(long)(t.y0 + 1) * W + t.x0] * t.sw;
-  if (y1 && x1) acc += plane[(long)(t.y0 + 1) * W + t.x0 + 1] * t.se;
-  out[i] = acc;
+  out[i] = sample_taps(t, H, W, [&](int y, int x) { return plane[(long)y * W + x]; });
 }
 __global__ void __launch_bounds__(256) point_sample_bwd_kernel(const float* __restrict__ dout, const float* __restrict__ coords,
                                                                float* __restrict__ din, int N, int H, int W, int P,
@@ -73,6 +83,87 @@ __global__ void __launch_bounds__(256) point_sample_bwd_kernel(const float* __re
   if (y0 && x1) atomicAdd(plane + (long)t.y0 * W + t.x0 + 1, g * t.ne);
   if (y1 && x0) atomicAdd(plane + (long)(t.y0 + 1) * W + t.x0, g * t.sw);
   if (y1 && x1) atomicAdd(plane + (long)(t.y0 + 1) * W + t.x0 + 1, g * t.se);
+}
+
+// ---- panoptic training targets.  Stuff labels: presence bits of [num_things, num_classes) per CTA in shared memory,
+// OR-ed into the image's bitmap (one atomic per non-zero word); then one CTA per image writes the set bits in ascending
+// order.  grid (ctas_per_image, B); the semantic maps are contiguous (B, hs * ws), uint8 or int64.
+template <class T>
+__global__ void __launch_bounds__(256) stuff_presence_kernel(const T* __restrict__ sem, long pixels, int num_things,
+                                                             int num_classes, uint32_t* __restrict__ bitmap) {
+  extern __shared__ uint32_t bits[];
+  const int words = (num_classes - num_things + 31) >> 5;
+  for (int w = threadIdx.x; w < words; w += blockDim.x) bits[w] = 0u;
+  __syncthreads();
+  const T* img = sem + (long)blockIdx.y * pixels;
+  for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < pixels; p += (long)gridDim.x * blockDim.x) {
+    const long v = (long)img[p];
+    if (v >= num_things && v < num_classes) {
+      const int k = (int)(v - num_things);
+      const uint32_t bit = 1u << (k & 31);
+      if (!(bits[k >> 5] & bit)) atomicOr(&bits[k >> 5], bit);    // a read first: most pixels repeat a set bit
+    }
+  }
+  __syncthreads();
+  for (int w = threadIdx.x; w < words; w += blockDim.x)
+    if (bits[w]) atomicOr(&bitmap[(long)blockIdx.y * words + w], bits[w]);
+}
+// one warp per image: labels (B, num_stuff) ascending, -1 past the count; counts (B,)
+__global__ void __launch_bounds__(32) stuff_compact_kernel(const uint32_t* __restrict__ bitmap, int num_things,
+                                                          int num_classes, int64_t* __restrict__ labels,
+                                                          int* __restrict__ counts) {
+  const int num_stuff = num_classes - num_things, words = (num_stuff + 31) >> 5, lane = threadIdx.x;
+  const uint32_t* bm = bitmap + (long)blockIdx.x * words;
+  int64_t* out = labels + (long)blockIdx.x * num_stuff;
+  int base = 0;
+  for (int w0 = 0; w0 < words; w0 += 32) {
+    uint32_t word = (w0 + lane < words) ? bm[w0 + lane] : 0u;
+    const int n = __popc(word);
+    int incl = n;
+    for (int d = 1; d < 32; d <<= 1) {
+      const int o = __shfl_up_sync(0xffffffffu, incl, d);
+      if (lane >= d) incl += o;
+    }
+    int at = base + incl - n;
+    while (word) {
+      const int b = __ffs(word) - 1;
+      out[at++] = num_things + (w0 + lane) * 32 + b;
+      word &= word - 1;
+    }
+    base += __shfl_sync(0xffffffffu, incl, 31);
+  }
+  for (int k = base + lane; k < num_stuff; k += 32) out[k] = -1;
+  if (lane == 0) counts[blockIdx.x] = base;
+}
+
+// Ground-truth point samples, point_sample_kernel's arithmetic on implicit planes: row r = (image, target) of `rows`;
+// target g < num_things reads things plane g, 0 outside its (h, w) (the zero padding up to (pad_h, pad_w)); a stuff
+// target reads sem == stuff_labels[g - num_things].  coords (num_images, P, 2) per image or (rows, P, 2) per row.
+__device__ __forceinline__ float stuff_tap(const cgg_gt_image& im, int y, int x, int64_t label) {
+  const long at = (long)y * im.sem_stride + x;
+  const int64_t v = im.sem_is_i64 ? ((const int64_t*)im.sem)[at] : (int64_t)((const uint8_t*)im.sem)[at];
+  return v == label ? 1.f : 0.f;
+}
+__global__ void __launch_bounds__(256) gt_point_sample_kernel(const cgg_gt_image* __restrict__ images,
+                                                              const int* __restrict__ rows, const float* __restrict__ coords,
+                                                              float* __restrict__ out, int R, int P, int coords_per_image) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long)R * P) return;
+  const int p = (int)(i % P);
+  const long r = i / P;
+  const int img = rows[2 * r], g = rows[2 * r + 1];
+  const cgg_gt_image& im = images[img];
+  const float* c = coords + ((coords_per_image ? (long)img : r) * P + p) * 2;
+  const Taps t = taps_of(c[0], c[1], im.pad_h, im.pad_w);
+  if (g < im.num_things) {
+    const uint8_t* plane = im.things + (long)g * im.h * im.w;
+    out[i] = sample_taps(t, im.pad_h, im.pad_w, [&](int y, int x) {
+      return (y < im.h && x < im.w && plane[(long)y * im.w + x]) ? 1.f : 0.f;
+    });
+  } else {
+    const int64_t label = im.stuff_labels[g - im.num_things];
+    out[i] = sample_taps(t, im.pad_h, im.pad_w, [&](int y, int x) { return stuff_tap(im, y, x, label); });
+  }
 }
 
 __device__ __forceinline__ float softplus_f(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
@@ -276,6 +367,33 @@ cudaError_t launch_weighted_ce_bwd(const float* logits, const int64_t* labels, c
   const long total = (long)R * C1;
   if (total <= 0) return cudaSuccess;
   weighted_ce_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(logits, labels, cw, lse, R, C1, grow, dlogits);
+  count_launch();
+  return cudaGetLastError();
+}
+cudaError_t launch_panoptic_stuff_labels(const void* sem, bool sem_i64, int B, long pixels, int num_things, int num_classes,
+                                         uint32_t* bitmap, int64_t* labels, int* counts, cudaStream_t s) {
+  const int words = (num_classes - num_things + 31) / 32;
+  cudaError_t e = cudaMemsetAsync(bitmap, 0, (size_t)B * words * sizeof(uint32_t), s);
+  if (e != cudaSuccess) return e;
+  // enough CTAs to stream a 1024^2 map at full bandwidth, at least 4K pixels each
+  const long per_cta = 4096;
+  const int ctas = (int)std::min<long>(64, std::max<long>(1, (pixels + per_cta - 1) / per_cta));
+  const dim3 grid(ctas, B);
+  const size_t smem = (size_t)words * sizeof(uint32_t);
+  if (sem_i64)
+    stuff_presence_kernel<int64_t><<<grid, 256, smem, s>>>((const int64_t*)sem, pixels, num_things, num_classes, bitmap);
+  else
+    stuff_presence_kernel<uint8_t><<<grid, 256, smem, s>>>((const uint8_t*)sem, pixels, num_things, num_classes, bitmap);
+  stuff_compact_kernel<<<B, 32, 0, s>>>(bitmap, num_things, num_classes, labels, counts);
+  count_launch(2);
+  return cudaGetLastError();
+}
+cudaError_t launch_gt_point_sample(const cgg_gt_image* images, const int* rows, const float* coords, float* out, int R, int P,
+                                   bool coords_per_image, cudaStream_t s) {
+  const long total = (long)R * P;
+  if (total <= 0) return cudaSuccess;
+  gt_point_sample_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(images, rows, coords, out, R, P,
+                                                                         coords_per_image ? 1 : 0);
   count_launch();
   return cudaGetLastError();
 }

@@ -287,8 +287,11 @@ class Mask2FormerHeadOpenB200(nn.Module):
     def forward_train(self, feats, img_metas, gt_bboxes, gt_labels, gt_masks, gt_semantic_seg, gt_caption_ids,
                       gt_caption_mask, gt_caption_nouns_ids, gt_caption_nouns_mask, gt_bboxes_ignore=None, **kwargs):
         """head.py:851-921 (same signature): forward on the autograd-connected path, noun embeddings, losses.
-        `preprocess_gt` (mmdet, :903) only feeds the matching-based losses and is left to the `matching_losses` hook."""
+        mmdet's inputs (BitmapMasks, a gt_semantic_seg batch) go through `preprocess_gt` (:903) into compact targets; a
+        list of dense mask tensors without a semantic map is passed to the losses as it is."""
         assert gt_bboxes_ignore is None
+        if gt_masks is not None and (gt_semantic_seg is not None or not all(torch.is_tensor(m) for m in gt_masks)):
+            gt_labels, gt_masks = self.preprocess_gt(gt_labels, gt_masks, gt_semantic_seg, img_metas)
         all_cls_scores, all_cls_emb_preds, all_mask_preds = self(feats, img_metas)
         nouns_embs = nouns_mask = cap_embs = None
         if self.use_caption_generation:                                                                 # :905-908
@@ -297,6 +300,15 @@ class Mask2FormerHeadOpenB200(nn.Module):
             nouns_embs, nouns_mask = self.extract_caption_embeddings(gt_caption_nouns_ids, gt_caption_nouns_mask)
         return self.loss(all_cls_scores, all_cls_emb_preds, all_mask_preds, gt_labels, gt_masks, gt_caption_ids, cap_embs,
                          gt_caption_mask, gt_caption_nouns_ids, nouns_embs, nouns_mask, img_metas)
+
+    def preprocess_gt(self, gt_labels_list, gt_masks_list, gt_semantic_segs, img_metas):
+        """mmdet 2.28.2 MaskFormerHead.preprocess_gt (head.py:903): per image, things labels then the stuff labels present
+        in the semantic map (ascending) -> (labels_list, cgg_b200.matching.PanopticTargets).  The targets stay compact
+        (unpadded things masks, the semantic map and its stuff labels on the device); the matching losses point-sample
+        them as mmdet's dense padded int64 masks would be sampled."""
+        from .matching import preprocess_gt
+        return preprocess_gt(gt_labels_list, gt_masks_list, gt_semantic_segs, img_metas, self.num_things_classes,
+                             self.num_stuff_classes, self.query_feat.weight.device)
 
     def simple_test(self, feats, img_metas, **kwargs):
         """head.py:923-980 (same signature and return tuple): last head call's outputs, masks upsampled to the padded
@@ -315,15 +327,17 @@ class Mask2FormerHeadOpenB200(nn.Module):
             ml = getattr(self, 'matching_losses', None)
             if not isinstance(ml, MatchingLosses):
                 ml = MatchingLosses(self, train_cfg=self.train_cfg)
-            gm = kwargs['gt_masks'][0][0]
-            if not torch.is_tensor(gm):              # mmdet BitmapMasks
-                gm = gm.pad(img_metas[0]['pad_shape'][:2], pad_val=0).to_tensor(dtype=torch.long, device=mask_cls_results.device)
+            gl, gm = kwargs['gt_labels'][0][0], kwargs['gt_masks'][0][0]
+            if torch.is_tensor(gm):
+                gm = gm.to(mask_cls_results.device)
+            else:                                    # mmdet BitmapMasks: compact things targets
+                gl, gm = self.preprocess_gt([gl], [gm], None, img_metas[:1])
+                gl = gl[0]
             logits = None
             if self.use_class_emb:
                 logits = similarity(mask_cls_emb_results[0].float(), self.class_embs, 1.0 / float(self.softmax_temperature))
             assigned_labels = ml.get_target_single(mask_cls_results[0].float(), logits, mask_pred_results[0],
-                                                   kwargs['gt_labels'][0][0].to(mask_cls_results.device),
-                                                   gm.to(mask_cls_results.device))[0]
+                                                   gl.to(mask_cls_results.device), gm)[0]
         img_shape = kwargs.get('img_shape') or img_metas[0]['batch_input_shape']
         mask_pred_results = upsample_masks(self, mask_pred_results, (img_shape[0], img_shape[1]))      # :957-964
         caption_generation_results = None

@@ -20,7 +20,7 @@ EXPORTS = ['cgg_create', 'cgg_destroy', 'cgg_last_error', 'cgg_version', 'cgg_la
            'cgg_gemm_f32', 'cgg_layernorm', 'cgg_layernorm_bwd_scratch_bytes', 'cgg_layernorm_backward', 'cgg_relu_backward',
            'cgg_axpy', 'cgg_add_rows', 'cgg_sum_batch', 'cgg_colsum', 'cgg_mem_prep', 'cgg_mem_prep_backward', 'cgg_sine_pos',
            'cgg_attention_f32', 'cgg_attention_backward', 'cgg_attn_softmax_rows', 'cgg_attn_dscore', 'cgg_point_sample', 'cgg_point_sample_backward',
-           'cgg_matching_cost', 'cgg_point_losses', 'cgg_point_losses_backward', 'cgg_weighted_ce', 'cgg_weighted_ce_backward',
+           'cgg_matching_cost', 'cgg_panoptic_stuff_labels', 'cgg_gt_point_sample', 'cgg_point_losses', 'cgg_point_losses_backward', 'cgg_weighted_ce', 'cgg_weighted_ce_backward',
            # test-time step after the path
            'cgg_upsample_masks', 'cgg_instance_mask_stats', 'cgg_softmax_rows', 'cgg_panoptic_scratch_bytes',
            'cgg_panoptic_fuse', 'cgg_caption_self_attn_step', 'cgg_caption_cache_reorder', 'cgg_caption_beam_scores',
@@ -68,6 +68,12 @@ class BeamState(C.Structure):
     _fields_ = [('tokens', C.c_void_p), ('token_cap', C.c_int)] + \
                [(n, C.c_void_p) for n in ('weights', 'n_active', 'parent', 'next_ids', 'fin_tokens', 'fin_len', 'fin_score',
                                          'n_fin', 'max_idx', 'done', 'n_done')]
+
+
+class GtImage(C.Structure):
+    """cgg_gt_image (include/cgg_b200.h): one image's compact panoptic training targets (device pointers)"""
+    _fields_ = [('things', C.c_void_p), ('sem', C.c_void_p), ('stuff_labels', C.c_void_p), ('sem_stride', C.c_int64)] + \
+               [(n, C.c_int) for n in ('num_things', 'h', 'w', 'pad_h', 'pad_w', 'num_stuff', 'sem_is_i64', 'reserved')]
 
 
 class CggError(RuntimeError):
@@ -138,6 +144,8 @@ def load():
     lib.cgg_point_sample.argtypes = [vp, vp, vp, vp, i, i, i, i, i, vp]
     lib.cgg_point_sample_backward.argtypes = [vp, vp, vp, vp, i, i, i, i, i, vp]
     lib.cgg_matching_cost.argtypes = [vp, vp, vp, vp, vp, vp, i, i, i, i, f, f, f, f, f, vp, vp, vp]
+    lib.cgg_panoptic_stuff_labels.argtypes = [vp, vp, i, i, i, i, i, i, vp, vp, vp, vp]
+    lib.cgg_gt_point_sample.argtypes = [vp, vp, vp, vp, vp, i, i, i, vp]
     lib.cgg_point_losses.argtypes = [vp, vp, vp, i, i, f, vp, vp, vp, vp]
     lib.cgg_point_losses_backward.argtypes = [vp, vp, vp, vp, i, i, f, vp, vp, vp, vp]
     lib.cgg_weighted_ce.argtypes = [vp, vp, vp, vp, i, i, vp, vp, vp, vp]

@@ -10,10 +10,15 @@ backward are kernels of the C-ABI library (csrc/match_kernels.cu).  What stays w
 reference: the Hungarian solve (scipy's linear_sum_assignment on the (Q, G) cost matrix, assigner :127-134), the random
 point draws (torch.rand) and the top-k of the uncertainty sampling.
 
+Panoptic targets (mmdet MaskFormerHead.preprocess_gt, :903) are kept compact: `preprocess_gt` uploads the unpadded things
+masks and finds each semantic map's stuff labels on the device, and the targets are only ever point-sampled from there
+(`PanopticTargets`); no (G, Hp, Wp) mask tensor exists.
+
 `MatchingLosses` plugs into `Mask2FormerHeadOpenB200.matching_losses` (head.py `loss`), which merges its dict with the
 grounding terms: together they are the reference's full loss dict (caption generation excepted, row f4)."""
 import ctypes as C
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -149,6 +154,159 @@ def matching_cost(mask_points, gt_points, gt_labels, cls_scores=None, cls_emb_lo
     return cost
 
 
+class PanopticTargets:
+    """Compact panoptic training targets of a batch, from `preprocess_gt`: per image the unpadded things planes (uint8),
+    the semantic map and its stuff labels, described by one cgg_gt_image per image in device memory.  Target g of image i
+    is things plane g (zero outside the plane, up to the image's pad_shape) for g < num_things[i], else the stuff mask
+    `sem_i == stuff label`; targets are only ever point-sampled, bit for bit as `point_sample` samples the dense padded
+    masks of mmdet's preprocess_gt."""
+
+    def __init__(self, images, rows, num_gts, keep):
+        self.images = images            # B cgg_gt_image descriptors (device bytes)
+        self.rows = rows                # (sum G, 2) int32 (image, target), every target of the batch in image order
+        self.num_gts = num_gts          # per image, things + stuff (host ints)
+        self._keep = keep               # the buffers the descriptors point into
+
+    def __len__(self):
+        return len(self.num_gts)
+
+    def _sample(self, rows, coords, per_image):
+        c = coords.float().contiguous()
+        R, P = rows.shape[0], c.shape[1]
+        out = torch.empty((R, P), dtype=torch.float32, device=c.device)
+        if R == 0 or P == 0:
+            return out
+        lib, h, s = _ctx(c)
+        _lib.check(lib.cgg_gt_point_sample(h, _p(self.images), _p(rows), _p(c), _p(out), R, P, int(per_image), s), h,
+                   'cgg_gt_point_sample')
+        return out
+
+    def sample_shared(self, coords):
+        """Every target of image i at the points coords[i] (B, P, 2) -> (sum G, P), images in order (the cost matrices)."""
+        return self._sample(self.rows, coords, True)
+
+    def sample_rows(self, rows, coords):
+        """Row r of `rows` (N, 2) int32 = (image, target) at its own points coords[r] (N, P, 2) -> (N, P) (loss targets)."""
+        return self._sample(rows.int().contiguous(), coords, False)
+
+
+def _is_bitmap_masks(m):
+    return hasattr(m, 'masks') and hasattr(m, 'height') and hasattr(m, 'width')
+
+
+def check_stuff_extent(num_stuff, img_metas, sem_hw):
+    """mmdet concatenates the things masks (padded to pad_shape) with the stuff masks (the semantic map's shape): that
+    fails when the two extents differ and the image has a stuff target."""
+    for i, n in enumerate(num_stuff):
+        pad = tuple(int(v) for v in img_metas[i]['pad_shape'][:2])
+        if n > 0 and pad != tuple(sem_hw):
+            raise _lib.CggError('image %d: pad_shape %s differs from the semantic map %s, and it has %d stuff targets'
+                                % (i, pad, tuple(sem_hw), n))
+
+
+def stuff_labels(sem, num_things, num_stuff):
+    """The stuff labels present in each semantic map of sem (B, 1, Hs, Ws) (uint8 or int64, on the device), in
+    [num_things, num_things + num_stuff) -> (labels (B, num_stuff) int64 ascending, -1 past the count; counts (B,) int32)."""
+    sem = sem.contiguous()
+    B, Hs, Ws = sem.shape[0], sem.shape[-2], sem.shape[-1]
+    labels = torch.empty((B, num_stuff), dtype=torch.long, device=sem.device)
+    counts = torch.zeros((B,), dtype=torch.int32, device=sem.device)
+    if num_stuff == 0:
+        return labels, counts
+    bitmap = torch.empty((B * ((num_stuff + 31) // 32),), dtype=torch.int32, device=sem.device)
+    lib, h, s = _ctx(sem)
+    _lib.check(lib.cgg_panoptic_stuff_labels(h, _p(sem), int(sem.dtype == torch.int64), B, Hs, Ws, num_things,
+                                             num_things + num_stuff, _p(bitmap), _p(labels), _p(counts), s), h,
+               'cgg_panoptic_stuff_labels')
+    return labels, counts
+
+
+def preprocess_gt(gt_labels_list, gt_masks_list, gt_semantic_segs, img_metas, num_things, num_stuff, device):
+    """mmdet 2.28.2 MaskFormerHead.preprocess_gt / preprocess_panoptic_gt, compact: -> (labels_list, PanopticTargets).
+    labels: int64 on `device`, things then the stuff labels present in the semantic map, ascending.  gt_masks_list[i]:
+    mmdet BitmapMasks (anything with `.masks` (G, h, w), `.height`, `.width`; uploaded unpadded through one pinned
+    staging buffer) or a bool / uint8 (G, h, w) tensor; padded implicitly to img_metas[i]['pad_shape'].  gt_semantic_segs:
+    None (things only) or the (B, 1, Hs, Ws) batch (a list of (1, Hs, Ws) maps is stacked), uint8 or int64, pad value 255."""
+    B = len(gt_labels_list)
+    if len(gt_masks_list) != B or len(img_metas) != B:
+        raise _lib.CggError('preprocess_gt: %d label lists, %d mask lists, %d img_metas' % (B, len(gt_masks_list), len(img_metas)))
+    device = torch.device(device)
+    planes = []                                                    # per image: (numpy array or device tensor, G, h, w)
+    for i, (lab, m) in enumerate(zip(gt_labels_list, gt_masks_list)):
+        if _is_bitmap_masks(m):
+            arr = np.asarray(m.masks)
+            h, w = int(m.height), int(m.width)
+            arr = arr.reshape(-1, h, w) if arr.size else np.zeros((0, h, w), np.uint8)
+            arr = np.ascontiguousarray(arr if arr.dtype in (np.uint8, np.bool_) else arr != 0).view(np.uint8)
+        elif torch.is_tensor(m):
+            if m.dtype not in (torch.bool, torch.uint8) or m.dim() != 3:
+                raise _lib.CggError('image %d: a mask tensor must be bool or uint8 (G, h, w), got %s %s' % (i, m.dtype, tuple(m.shape)))
+            arr = m
+        else:
+            raise _lib.CggError('image %d: masks must be mmdet BitmapMasks or a (G, h, w) tensor, got %s' % (i, type(m).__name__))
+        G, h, w = (int(v) for v in arr.shape)
+        if G != int(lab.shape[0]):
+            raise _lib.CggError('image %d: %d masks for %d labels' % (i, G, int(lab.shape[0])))
+        pad_h, pad_w = (int(v) for v in img_metas[i]['pad_shape'][:2])
+        if h > pad_h or w > pad_w:
+            raise _lib.CggError('image %d: masks (%d, %d) larger than pad_shape (%d, %d)' % (i, h, w, pad_h, pad_w))
+        planes.append((arr, G, h, w, pad_h, pad_w))
+    sem = None
+    if gt_semantic_segs is not None:
+        sem = gt_semantic_segs if torch.is_tensor(gt_semantic_segs) else torch.stack([torch.as_tensor(x) for x in gt_semantic_segs])
+        if sem.dtype not in (torch.uint8, torch.int64):
+            raise _lib.CggError('gt_semantic_seg must be uint8 or int64, got %s' % sem.dtype)
+        if sem.dim() != 4 or sem.shape[0] != B or sem.shape[1] != 1:
+            raise _lib.CggError('gt_semantic_seg must be (B, 1, Hs, Ws), got %s' % (tuple(sem.shape),))
+    labels = [torch.as_tensor(x).to(device=device, dtype=torch.long) for x in gt_labels_list]
+    keep = []
+    n_stuff = [0] * B
+    if sem is not None:
+        sem = sem.to(device).contiguous()
+        Hs, Ws = int(sem.shape[2]), int(sem.shape[3])
+        stuff, counts = stuff_labels(sem, num_things, num_stuff)
+        n_stuff = counts.tolist()                                  # the batch's one read-back: it shapes the cost matrices
+        check_stuff_extent(n_stuff, img_metas, (Hs, Ws))
+        labels = [torch.cat((labels[i], stuff[i, :n_stuff[i]])) for i in range(B)]
+        keep += [sem, stuff]
+    # one staging buffer, one copy: B descriptors, the (image, target) table, then every host-side things plane
+    desc_bytes = B * C.sizeof(_lib.GtImage)
+    num_gts = [p[1] + n for p, n in zip(planes, n_stuff)]
+    rows = np.array([(i, g) for i in range(B) for g in range(num_gts[i])], dtype=np.int32).reshape(-1, 2)
+    at = desc_bytes + rows.nbytes
+    offsets = []
+    for arr, G, h, w, _, _ in planes:
+        offsets.append(at if isinstance(arr, np.ndarray) else None)
+        at += arr.nbytes if isinstance(arr, np.ndarray) else 0
+    buf = torch.empty((at,), dtype=torch.uint8, device=device)
+    staging = torch.empty((at,), dtype=torch.uint8, pin_memory=True)
+    st = staging.numpy()
+    descs = (_lib.GtImage * B)()
+    elem = sem.element_size() if sem is not None else 0
+    for i, ((arr, G, h, w, pad_h, pad_w), off) in enumerate(zip(planes, offsets)):
+        d = descs[i]
+        if off is not None:
+            st[off:off + arr.nbytes] = arr.reshape(-1)
+            d.things = buf.data_ptr() + off
+        else:
+            t = arr.to(device).contiguous().view(torch.uint8)
+            keep.append(t)
+            d.things = t.data_ptr()
+        d.num_things, d.h, d.w, d.pad_h, d.pad_w = G, h, w, pad_h, pad_w
+        if n_stuff[i]:
+            d.sem = sem.data_ptr() + i * Hs * Ws * elem
+            d.sem_stride, d.sem_is_i64 = Ws, int(sem.dtype == torch.int64)
+            d.stuff_labels = stuff.data_ptr() + i * num_stuff * 8
+            d.num_stuff = n_stuff[i]
+    st[:desc_bytes] = np.frombuffer(bytes(descs), dtype=np.uint8)
+    st[desc_bytes:desc_bytes + rows.nbytes] = rows.reshape(-1).view(np.uint8)
+    buf.copy_(staging, non_blocking=True)                          # a plain cudaMemcpyAsync from pinned memory
+    keep += [buf, staging]
+    images = buf[:desc_bytes]
+    rows_dev = buf[desc_bytes:desc_bytes + rows.nbytes].view(torch.int32).view(-1, 2)
+    return labels, PanopticTargets(images, rows_dev, num_gts, keep)
+
+
 def _reduce_mean(t):
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         t = t.clone()
@@ -187,15 +345,35 @@ class MatchingLosses:
     # ---- targets (mask2former_head.py:320-390)
     @torch.no_grad()
     def get_target_single(self, cls_score, cls_emb_logit, mask_pred, gt_labels, gt_masks):
+        """gt_masks: the dense (G, H, W) masks, whose matched rows are returned, or a one-image PanopticTargets, whose
+        matched target indices are returned."""
         dev = mask_pred.device
-        Q, G = mask_pred.shape[0], gt_labels.shape[0]
+        G = gt_labels.shape[0]
         coords = self.rand(1, self.num_points, 2, device=dev).to(dev)
+        if isinstance(gt_masks, PanopticTargets):
+            if len(gt_masks) != 1:
+                raise _lib.CggError('get_target_single takes the targets of one image, got %d' % len(gt_masks))
+            labels, pos_gt, mask_weights, n = self._assign(cls_score, cls_emb_logit, mask_pred, gt_labels,
+                                                           gt_masks.sample_shared(coords), coords)
+            return labels, pos_gt, mask_weights, n
+        if G == 0:
+            labels, _, mask_weights, _ = self._assign(cls_score, cls_emb_logit, mask_pred, gt_labels, None, coords)
+            return labels, gt_masks[:0], mask_weights, 0
+        labels, pos_gt, mask_weights, n = self._assign(cls_score, cls_emb_logit, mask_pred, gt_labels,
+                                                       point_sample(gt_masks.float(), coords), coords)
+        return labels, gt_masks[pos_gt], mask_weights, n
+
+    @torch.no_grad()
+    def _assign(self, cls_score, cls_emb_logit, mask_pred, gt_labels, gt_points, coords):
+        """One image's Hungarian assignment from its targets sampled at coords (None or no row: no target) ->
+        (labels (Q,), matched target indices in query order, mask_weights (Q,), number matched)."""
+        dev = mask_pred.device
+        Q = mask_pred.shape[0]
         labels = torch.full((Q,), self.head.num_classes, dtype=torch.long, device=dev)
         mask_weights = torch.zeros((Q,), dtype=torch.float32, device=dev)
-        if G == 0:
-            return labels, gt_masks[:0], mask_weights, 0
+        if gt_points is None or gt_points.shape[0] == 0:
+            return labels, torch.zeros((0,), dtype=torch.long, device=dev), mask_weights, 0
         mask_points = point_sample(mask_pred.detach(), coords)
-        gt_points = point_sample(gt_masks.float(), coords)
         cost = matching_cost(mask_points, gt_points, gt_labels, cls_score.detach(),
                              None if cls_emb_logit is None else cls_emb_logit.detach(), self.w_cls, self.w_cls_emb, self.w_mask,
                              self.w_dice, self.cost_dice_eps)
@@ -206,7 +384,28 @@ class MatchingLosses:
         pos_gt = torch.from_numpy(cols[order]).to(dev)
         labels[pos] = gt_labels[pos_gt]
         mask_weights[pos] = 1.0
-        return labels, gt_masks[pos_gt], mask_weights, int(pos.numel())
+        return labels, pos_gt, mask_weights, int(pos.numel())
+
+    @torch.no_grad()
+    def _targets_compact(self, cls_scores, cls_emb_logits, mask_preds, gt_labels_list, targets):
+        """get_target_single for every image of PanopticTargets, with all the cost matrices' ground truth sampled in one
+        launch -> (labels (B*Q,), mask_weights (B, Q), number matched, matched (image, target) rows in query order)."""
+        B = cls_scores.shape[0]
+        dev = cls_scores.device
+        if len(targets) != B:
+            raise _lib.CggError('%d images of targets for a batch of %d' % (len(targets), B))
+        # get_target_single's point draws, in the same order: no other draw falls between them
+        coords = [self.rand(1, self.num_points, 2, device=dev).to(dev) for _ in range(B)]
+        gt_points = targets.sample_shared(torch.cat(coords, 0))
+        labels, weights, rows, num_pos, at = [], [], [], 0, 0
+        for i in range(B):
+            G = targets.num_gts[i]
+            lab, pos_gt, mw, n = self._assign(cls_scores[i], None if cls_emb_logits is None else cls_emb_logits[i],
+                                              mask_preds[i], gt_labels_list[i].to(dev), gt_points[at:at + G], coords[i])
+            at += G
+            labels.append(lab), weights.append(mw), rows.append(torch.stack((torch.full_like(pos_gt, i), pos_gt), 1))
+            num_pos += n
+        return torch.stack(labels, 0).flatten(), torch.stack(weights, 0), num_pos, torch.cat(rows, 0).int()
 
     def uncertain_point_coords(self, mask_preds):
         """mmdet get_uncertain_point_coords_with_randomness on (N, h, w) logits -> (N, num_points, 2)."""
@@ -225,17 +424,23 @@ class MatchingLosses:
 
     # ---- one head call (mask2former_head.py:464-629 without the caption terms)
     def loss_single(self, cls_scores, cls_emb_logits, mask_preds, gt_labels_list, gt_masks_list):
+        """gt_masks_list: per image dense (G, H, W) masks, or the batch's PanopticTargets (preprocess_gt)."""
         B, Q = cls_scores.shape[:2]
         dev = cls_scores.device
-        labels, targets, weights, num_pos = [], [], [], 0
-        for i in range(B):
-            lab, mt, mw, n = self.get_target_single(cls_scores[i], None if cls_emb_logits is None else cls_emb_logits[i],
-                                                    mask_preds[i], gt_labels_list[i].to(dev), gt_masks_list[i].to(dev))
-            labels.append(lab), targets.append(mt), weights.append(mw)
-            num_pos += n
-        labels = torch.stack(labels, 0).flatten()
-        mask_targets = torch.cat(targets, 0)
-        mask_weights = torch.stack(weights, 0)
+        compact = isinstance(gt_masks_list, PanopticTargets)
+        if compact:
+            labels, mask_weights, num_pos, target_rows = self._targets_compact(cls_scores, cls_emb_logits, mask_preds,
+                                                                               gt_labels_list, gt_masks_list)
+        else:
+            labels, targets, weights, num_pos = [], [], [], 0
+            for i in range(B):
+                lab, mt, mw, n = self.get_target_single(cls_scores[i], None if cls_emb_logits is None else cls_emb_logits[i],
+                                                        mask_preds[i], gt_labels_list[i].to(dev), gt_masks_list[i].to(dev))
+                labels.append(lab), targets.append(mt), weights.append(mw)
+                num_pos += n
+            labels = torch.stack(labels, 0).flatten()
+            mask_targets = torch.cat(targets, 0)
+            mask_weights = torch.stack(weights, 0)
         cw = self.class_weight.to(dev)
         out = {}
         row_loss, row_w = _WeightedCE.apply(cls_scores.flatten(0, 1), labels, cw)
@@ -247,13 +452,16 @@ class MatchingLosses:
             out['loss_cls_emb'] = self.loss_cls_emb_weight * row_loss_e.sum() / avg
         num_total = float(max(float(_reduce_mean(torch.tensor([float(num_pos)], device=dev))), 1.0))
         pos_preds = mask_preds[mask_weights > 0]
-        if mask_targets.shape[0] == 0:                                   # zero match (:582-586)
+        if (target_rows if compact else mask_targets).shape[0] == 0:     # zero match (:582-586)
             out['loss_dice'] = pos_preds.sum()
             out['loss_mask'] = pos_preds.sum()
             return out, labels.view(B, Q), mask_weights
         with torch.no_grad():
             coords = self.uncertain_point_coords(pos_preds.detach())
-            point_targets = point_sample(mask_targets.float(), coords)
+            if compact:
+                point_targets = gt_masks_list.sample_rows(target_rows, coords)
+            else:
+                point_targets = point_sample(mask_targets.float(), coords)
         point_preds = point_sample(pos_preds, coords)
         dice_rows, bce_rows = _PointLosses.apply(point_preds, point_targets, self.dice_eps)
         out['loss_dice'] = self.loss_dice_weight * dice_rows.sum() / (num_total + EPS32)

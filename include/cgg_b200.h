@@ -320,6 +320,32 @@ int cgg_point_sample(cgg_handle *h, const float *in, const float *coords, float 
                      int num_points, int coords_shared, void *stream);
 int cgg_point_sample_backward(cgg_handle *h, const float *dout, const float *coords, float *din, int planes, int hh, int ww,
                               int num_points, int coords_shared, void *stream);
+/* Panoptic training targets without dense padded masks (mmdet 2.28.2 MaskFormerHead.preprocess_gt ->
+ * preprocess_panoptic_gt, head.py:903): things first in their given order, then one stuff target per label of
+ * [num_things, num_classes) present in the image's semantic map, ascending; other values (thing labels, >= num_classes,
+ * the 255 padding) give no target.
+ * cgg_panoptic_stuff_labels: sem (batch, 1, hs, ws) contiguous, uint8 (sem_is_i64 = 0) or int64 (1) -> stuff_labels
+ *   (batch, num_classes - num_things) int64, ascending, -1 past the image's count; counts (batch,) int32.  bitmap: scratch
+ *   of batch * ceil((num_classes - num_things) / 32) words (zeroed here).  num_classes - num_things <= 8192. */
+int cgg_panoptic_stuff_labels(cgg_handle *h, const void *sem, int sem_is_i64, int batch, int hs, int ws, int num_things,
+                              int num_classes, uint32_t *bitmap, int64_t *stuff_labels, int *counts, void *stream);
+/* One image's compact targets (DEVICE pointers).  things: num_things planes (h, w) of 0 / non-0 bytes at image size, not
+ * padded; the targets live on the padded plane (pad_h, pad_w) with zeros outside (h, w).  sem: the image's semantic map,
+ * (pad_h, pad_w) with a row stride of sem_stride elements, uint8 or int64 (sem_is_i64); stuff_labels: num_stuff labels,
+ * target num_things + k is `sem == stuff_labels[k]`.  sem / stuff_labels may be NULL when num_stuff == 0. */
+typedef struct cgg_gt_image {
+  const uint8_t *things;
+  const void *sem;
+  const int64_t *stuff_labels;
+  int64_t sem_stride;
+  int num_things, h, w, pad_h, pad_w, num_stuff, sem_is_i64, reserved;
+} cgg_gt_image;
+/* cgg_gt_point_sample: out[r, p] = point_sample(dense target, coords) bit for bit (cgg_point_sample's taps and order on
+ * the padded 0/1 plane), for rows r of `rows` (num_rows, 2) int32 = (image, target) into the DEVICE array `images`.
+ * coords (num_images, P, 2) when coords_per_image (every target of an image at the image's points: the cost matrix),
+ * else (num_rows, P, 2) (the matched rows' loss targets). */
+int cgg_gt_point_sample(cgg_handle *h, const cgg_gt_image *images, const int *rows, const float *coords, float *out,
+                        int num_rows, int num_points, int coords_per_image, void *stream);
 /* cost (num_q, num_gt) = w_cls * ClassificationCost(cls_scores) + w_cls_emb * ClassificationCost(cls_emb_logits)
  *                      + w_mask * CrossEntropyLossCost(use_sigmoid) + w_dice * DiceCost(pred_act, eps)   (assigner :98-125)
  * on the sampled mask logits (num_q, P) and sampled ground-truth masks (num_gt, P).  A class term with weight 0 may pass
