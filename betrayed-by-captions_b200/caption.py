@@ -147,7 +147,7 @@ class CaptionTransformerB200(nn.Module):
             # masked self-attention (transformers.py:102-134): fused qkv, per head [q | k | v] of 3*d columns
             tmp = ln(x, nz['mha'][0])
             qkv = lin(tmp, blk.mha_layer.qkv_layer).view(B, L, H, 3, d)
-            o = _AttentionViews.apply(k, qkv[:, :, :, 0], qkv[:, :, :, 1], qkv[:, :, :, 2], self_bits, scale)
+            o = _AttentionViews.apply(k, qkv[:, :, :, 0], qkv[:, :, :, 1], qkv[:, :, :, 2], self_bits, None, scale)
             x = ln(proj(o.view(B * L, C), blk.mha_layer.out_layer, tmp, blk.dropout_layer['mha']), nz['mha'][1])
             # cross-attention over the (adapted) query embeddings (:58-100)
             tmp = ln(x, nz['crx'][0])
@@ -155,7 +155,7 @@ class CaptionTransformerB200(nn.Module):
             q4 = lin(tmp, ca.to_qry).view(B, L, H, d)
             k4 = lin(mem, ca.to_key).view(B, Q, H, d)
             v4 = lin(mem, ca.to_val).view(B, Q, H, d)
-            o = _AttentionViews.apply(k, q4, k4, v4, None, scale)
+            o = _AttentionViews.apply(k, q4, k4, v4, None, None, scale)
             x = ln(proj(o.view(B * L, C), ca.to_out, tmp, blk.dropout_layer['crx']), nz['crx'][1])
             # FFN (:27-56; note the reference feeds `agg`, not the pre-normed tmp, :229)
             tmp = ln(x, nz['ffn'][0])
@@ -266,7 +266,7 @@ def _search_device(head, memory, BOS, EOS, max_len, beam_width, alpha):
                                                    k.s()), 'cgg_caption_self_attn_step')
             x = ln(lin(o, blk.mha_layer.out_layer, res=tmp), nz['mha'][1])
             tmp = ln(x, nz['crx'][0])
-            o = _AttentionViews.apply(k, lin(tmp, ca.to_qry).view(B, W, H, d), kv_mem[i][0], kv_mem[i][1], None, scale)
+            o = _AttentionViews.apply(k, lin(tmp, ca.to_qry).view(B, W, H, d), kv_mem[i][0], kv_mem[i][1], None, None, scale)
             x = ln(lin(o.view(n, D), ca.to_out, res=tmp), nz['crx'][1])
             tmp = ln(x, nz['ffn'][0])
             f0, f1 = blk.ffn_layer.linears[0], blk.ffn_layer.linears[1]

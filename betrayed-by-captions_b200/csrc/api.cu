@@ -414,7 +414,7 @@ extern "C" int cgg_masked_attention(cgg_handle* h, int batch, int num_keys, cons
     TC(h->tc, tc_attention(h->tc, batch, num_keys, q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, s));
     return CGG_OK;
   }
-  CU(launch_attention_f32(q, k, v, false, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, batch,
+  CU(launch_attention_f32(q, (const float*)k, (const float*)v, kv_stride, kv_batch_stride, bitmap, all_masked, out, batch,
                           h->cfg.num_queries, num_keys, h->cfg.num_heads, s));
   return CGG_OK;
 }
@@ -472,7 +472,7 @@ static int decoder_layer_impl(cgg_handle* h, const cgg_weights* w, int batch, in
   ST(linear_rows(h, s, x1, w->query_embed, Q, lw.self_in_w, lw.self_in_b, qb, rows, C, C, qscale));
   ST(linear_rows(h, s, x1, w->query_embed, Q, lw.self_in_w + (size_t)C * C, lw.self_in_b + C, kb, rows, C, C));
   ST(linear_rows(h, s, x1, nullptr, 1, lw.self_in_w + (size_t)2 * C * C, lw.self_in_b + 2 * C, vb, rows, C, C));
-  CU(launch_attention_f32(qb, kb, vb, false, C, (long)Q * C, nullptr, nullptr, o, nullptr, batch, Q, Q, c.num_heads, s));
+  CU(launch_attention_f32(qb, kb, vb, C, (long)Q * C, nullptr, nullptr, o, batch, Q, Q, c.num_heads, s));
   ST(linear_rows(h, s, o, nullptr, 1, lw.self_out_w, lw.self_out_b, t, rows, C, C, 1.f, x1));
   CU(launch_layernorm(t, nullptr, lw.norm_w[1], lw.norm_b[1], x2, rows, C, 1e-5f, true, s));
   // ---- FFN
@@ -813,34 +813,35 @@ extern "C" int cgg_sine_pos(cgg_handle* h, float* out, int hh, int ww, int C, vo
   return CGG_OK;
 }
 
-extern "C" int cgg_attention_f32(cgg_handle* h, int batch, int num_q, int num_keys, const float* q, const float* k,
-                                 const float* v, long kv_stride, long kv_batch_stride, const uint32_t* bitmap,
-                                 const uint8_t* all_masked, float* out, void* stream) {
+extern "C" int cgg_attention_f32(cgg_handle* h, int batch, int num_q, int num_keys, int heads, const float* q,
+                                 const float* k, const float* v, long kv_stride, long kv_batch_stride,
+                                 const uint32_t* bitmap, const uint8_t* all_masked, float* out, void* stream) {
   if (!h || !q || !k || !v || !out) return CGG_ERR_NULL;
   if (batch < 1 || num_q < 1 || num_keys < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
-  CU(launch_attention_f32(q, k, v, false, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, batch, num_q,
-                          num_keys, h->cfg.num_heads, (cudaStream_t)stream));
+  if (heads < 1 || kv_stride < 32L * heads) return fail(h, CGG_ERR_BAD_SHAPE, "heads < 1 or kv_stride < heads * 32");
+  CU(launch_attention_f32(q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, batch, num_q, num_keys, heads,
+                          (cudaStream_t)stream));
   return CGG_OK;
 }
 
-extern "C" int cgg_attention_backward(cgg_handle* h, int batch, int num_q, int num_keys, const float* q, const float* k,
-                                      const float* v, long kv_stride, long kv_batch_stride, const uint32_t* bitmap,
-                                      const uint8_t* all_masked, const float* out, const float* dout, float* dq,
-                                      float* dk, float* dv, long dkv_stride, long dkv_batch_stride, float* scratch,
-                                      void* stream) {
+extern "C" int cgg_attention_backward(cgg_handle* h, int batch, int num_q, int num_keys, int heads, const float* q,
+                                      const float* k, const float* v, long kv_stride, long kv_batch_stride,
+                                      const uint32_t* bitmap, const uint8_t* all_masked, const float* out,
+                                      const float* dout, float* dq, float* dk, float* dv, long dkv_stride,
+                                      long dkv_batch_stride, float* scratch, void* stream) {
   if (!h || !q || !k || !v || !out || !dout || !dq || !dk || !dv || !scratch) return CGG_ERR_NULL;
   if (batch < 1 || batch > 65535 || num_q < 1 || num_keys < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
-  const size_t n = (size_t)batch * h->cfg.num_heads * num_q;
+  if (heads < 1 || kv_stride < 32L * heads) return fail(h, CGG_ERR_BAD_SHAPE, "heads < 1 or kv_stride < heads * 32");
+  const size_t n = (size_t)batch * heads * num_q;
   CU(launch_attention_bwd(q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, dout, scratch, scratch + n, dq, dk,
-                          dv, dkv_stride, dkv_batch_stride, batch, num_q, num_keys, h->cfg.num_heads, (cudaStream_t)stream));
+                          dv, dkv_stride, dkv_batch_stride, batch, num_q, num_keys, heads, (cudaStream_t)stream));
   return CGG_OK;
 }
 
 extern "C" int cgg_attn_softmax_rows(cgg_handle* h, float* scores, const uint32_t* bitmap, const uint8_t* all_masked,
                                      int batch, int heads, int num_q, int num_keys, void* stream) {
   if (!h || !scores) return CGG_ERR_NULL;
-  if (heads <= 0) heads = h->cfg.num_heads;
-  if (batch < 1 || num_q < 1 || num_keys < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  if (batch < 1 || heads < 1 || num_q < 1 || num_keys < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
   CU(launch_attn_softmax_rows(scores, bitmap, all_masked, batch, heads, num_q, num_keys, (cudaStream_t)stream));
   return CGG_OK;
 }
@@ -848,8 +849,7 @@ extern "C" int cgg_attn_softmax_rows(cgg_handle* h, float* scores, const uint32_
 extern "C" int cgg_attn_dscore(cgg_handle* h, const float* probs, float* dprobs, const float* out, const float* dout,
                                int batch, int heads, int head_dim, int num_q, int num_keys, void* stream) {
   if (!h || !probs || !dprobs || !out || !dout) return CGG_ERR_NULL;
-  if (heads <= 0) { heads = h->cfg.num_heads; head_dim = h->cfg.embed_dim / h->cfg.num_heads; }
-  if (batch < 1 || num_q < 1 || num_keys < 1 || head_dim < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  if (batch < 1 || heads < 1 || head_dim < 1 || num_q < 1 || num_keys < 1) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
   CU(launch_attn_dscore(probs, dprobs, out, dout, batch, heads, head_dim, num_q, num_keys, (cudaStream_t)stream));
   return CGG_OK;
 }

@@ -63,11 +63,11 @@ cudaError_t launch_mask_bits(const float* mask_pred, int rows, int H4, int W4, i
 __global__ void all_masked_kernel(const uint32_t* __restrict__ bitmap, int rows, int W32, int K,
                                   uint8_t* __restrict__ all_masked);
 
-// K5/K6 attention core, fp32 SIMT flash-style (K/V fp32 or bf16).  q (B,Q,H*32) pre-scaled; k,v rows of H*32 at
+// K5/K6 attention core, fp32 SIMT flash-style.  q, out (B,Q,heads*32), q pre-scaled; k,v rows of heads*32 at
 // (b*kv_bstride + key*kv_stride); bitmap (B,Q,ceil(K/32)) or nullptr.
-cudaError_t launch_attention_f32(const float* q, const void* k, const void* v, bool kv_bf16, long kv_stride,
-                                 long kv_bstride, const uint32_t* bitmap, const uint8_t* all_masked,
-                                 float* out, __nv_bfloat16* out_bf16, int B, int Q, int K, int heads, cudaStream_t s);
+cudaError_t launch_attention_f32(const float* q, const float* k, const float* v, long kv_stride, long kv_bstride,
+                                 const uint32_t* bitmap, const uint8_t* all_masked, float* out, int B, int Q, int K,
+                                 int heads, cudaStream_t s);
 
 // K7 grounding: per (caption i, image j) pair distances, then the contrastive reduction.
 cudaError_t launch_grounding_pairs(const float* pred, const float* cap, const int64_t* cap_mask,

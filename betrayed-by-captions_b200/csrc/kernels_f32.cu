@@ -216,15 +216,10 @@ cudaError_t launch_mask_bits(const float* mask_pred, int rows, int H4, int W4, i
 // --------------------------------------------------------------- attention core (fp32)
 constexpr int AQT = 16, AKT = 128, AHD = 32;
 
-__device__ __forceinline__ float kv_to_float(float x) { return x; }
-__device__ __forceinline__ float kv_to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
-
-template <typename KV>
 __global__ void __launch_bounds__(128) attention_f32_kernel(
-    const float* __restrict__ q, const KV* __restrict__ k, const KV* __restrict__ v,
+    const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
     long kv_stride, long kv_bstride, const uint32_t* __restrict__ bitmap,
-    const uint8_t* __restrict__ all_masked, float* __restrict__ out, __nv_bfloat16* __restrict__ out_bf16, int Q,
-    int K, int heads) {
+    const uint8_t* __restrict__ all_masked, float* __restrict__ out, int Q, int K, int heads) {
   __shared__ float qs[AQT][AHD];
   __shared__ float Ks[AKT][AHD + 1];
   __shared__ __align__(16) float Vs[AKT][AHD];
@@ -267,8 +262,8 @@ __global__ void __launch_bounds__(128) attention_f32_kernel(
       float kv = 0.f, vv = 0.f;
       if (gk < K) {
         const long off = (long)b * kv_bstride + (long)gk * kv_stride + h * AHD + d;
-        kv = kv_to_float(k[off]);
-        vv = kv_to_float(v[off]);
+        kv = k[off];
+        vv = v[off];
       }
       Ks[kk][d] = kv;
       Vs[kk][d] = vv;
@@ -320,26 +315,16 @@ __global__ void __launch_bounds__(128) attention_f32_kernel(
   if (q0 + pq < Q) {
     const float inv = (l > 0.f) ? 1.0f / l : 0.f;
     const long off = ((long)b * Q + q0 + pq) * C + h * AHD + pd;
-    if (out) { out[off] = o[0] * inv; out[off + 1] = o[1] * inv; out[off + 2] = o[2] * inv; out[off + 3] = o[3] * inv; }
-    if (out_bf16) {
-      out_bf16[off] = __float2bfloat16_rn(o[0] * inv); out_bf16[off + 1] = __float2bfloat16_rn(o[1] * inv);
-      out_bf16[off + 2] = __float2bfloat16_rn(o[2] * inv); out_bf16[off + 3] = __float2bfloat16_rn(o[3] * inv);
-    }
+    out[off] = o[0] * inv; out[off + 1] = o[1] * inv; out[off + 2] = o[2] * inv; out[off + 3] = o[3] * inv;
   }
 }
 
-cudaError_t launch_attention_f32(const float* q, const void* k, const void* v, bool kv_bf16, long kv_stride,
-                                 long kv_bstride, const uint32_t* bitmap, const uint8_t* all_masked,
-                                 float* out, __nv_bfloat16* out_bf16, int B, int Q, int K, int heads, cudaStream_t s) {
+cudaError_t launch_attention_f32(const float* q, const float* k, const float* v, long kv_stride, long kv_bstride,
+                                 const uint32_t* bitmap, const uint8_t* all_masked, float* out, int B, int Q, int K,
+                                 int heads, cudaStream_t s) {
   if (B <= 0 || Q <= 0) return cudaSuccess;
   dim3 grid((Q + AQT - 1) / AQT, heads, B);
-  if (kv_bf16)
-    attention_f32_kernel<__nv_bfloat16><<<grid, 128, 0, s>>>(q, static_cast<const __nv_bfloat16*>(k),
-                                                             static_cast<const __nv_bfloat16*>(v), kv_stride, kv_bstride,
-                                                             bitmap, all_masked, out, out_bf16, Q, K, heads);
-  else
-    attention_f32_kernel<float><<<grid, 128, 0, s>>>(q, static_cast<const float*>(k), static_cast<const float*>(v),
-                                                     kv_stride, kv_bstride, bitmap, all_masked, out, out_bf16, Q, K, heads);
+  attention_f32_kernel<<<grid, 128, 0, s>>>(q, k, v, kv_stride, kv_bstride, bitmap, all_masked, out, Q, K, heads);
   count_launch();
   return cudaGetLastError();
 }

@@ -136,8 +136,8 @@ def load():
     lib.cgg_mem_prep.argtypes = [vp, vp, vp, vp, vp, vp, i, i, i, vp]
     lib.cgg_mem_prep_backward.argtypes = [vp, vp, vp, vp, i, i, i, vp]
     lib.cgg_sine_pos.argtypes = [vp, vp, i, i, i, vp]
-    lib.cgg_attention_f32.argtypes = [vp, i, i, i, vp, vp, vp, lg, lg, vp, vp, vp, vp]
-    lib.cgg_attention_backward.argtypes = [vp, i, i, i, vp, vp, vp, lg, lg, vp, vp, vp, vp, vp, vp, vp, lg, lg, vp, vp]
+    lib.cgg_attention_f32.argtypes = [vp, i, i, i, i, vp, vp, vp, lg, lg, vp, vp, vp, vp]
+    lib.cgg_attention_backward.argtypes = [vp, i, i, i, i, vp, vp, vp, lg, lg, vp, vp, vp, vp, vp, vp, vp, lg, lg, vp, vp]
     lib.cgg_attn_softmax_rows.argtypes = [vp, vp, vp, vp, i, i, i, i, vp]
     lib.cgg_attn_dscore.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, i, vp]
     f = C.c_float

@@ -290,88 +290,45 @@ class _MemPrep(torch.autograd.Function):
 
 
 class _Attention(torch.autograd.Function):
-    """softmax(q k^T + mask) v per head.  q (B, Q, C) scaled; k, v (B, K, C); bitmap / all_masked or None."""
+    """softmax(q k^T + mask) v over `heads` heads of 32 channels, the flash-style fp32 kernels.  q (B, Q, C) scaled;
+    k, v (B, K, C); bitmap / all_masked or None."""
 
     @staticmethod
-    def forward(ctx, k_, q, kk, v, bitmap, all_masked):
+    def forward(ctx, k_, q, kk, v, bitmap, all_masked, heads):
         B, Q, Cc = q.shape
         K = kk.shape[1]
         out = k_.new(B, Q, Cc)
-        k_.chk(k_.lib.cgg_attention_f32(k_.h, B, Q, K, _p(q), _p(kk), _p(v), Cc, K * Cc, _p(bitmap), _p(all_masked),
+        k_.chk(k_.lib.cgg_attention_f32(k_.h, B, Q, K, heads, _p(q), _p(kk), _p(v), Cc, K * Cc, _p(bitmap), _p(all_masked),
                                         _p(out), k_.s()), 'cgg_attention_f32')
-        ctx.k = k_
+        ctx.k, ctx.heads = k_, heads
         ctx.save_for_backward(q, kk, v, out, bitmap, all_masked)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        k_ = ctx.k
+        k_, heads = ctx.k, ctx.heads
         q, kk, v, out, bitmap, all_masked = ctx.saved_tensors
         B, Q, Cc = q.shape
         K = kk.shape[1]
         dout = dout.contiguous()
         dq, dk, dv = k_.new(B, Q, Cc), k_.new(B, K, Cc), k_.new(B, K, Cc)
-        heads = k_.rt.head.num_heads
         scratch = k_.new(2 * B * heads * Q)
-        k_.chk(k_.lib.cgg_attention_backward(k_.h, B, Q, K, _p(q), _p(kk), _p(v), Cc, K * Cc, _p(bitmap), _p(all_masked),
-                                             _p(out), _p(dout), _p(dq), _p(dk), _p(dv), Cc, K * Cc, _p(scratch),
-                                             k_.s()), 'cgg_attention_backward')
-        return None, dq, dk, dv, None, None
-
-
-class _AttentionGemm(torch.autograd.Function):
-    """The same attention written as tensor-core products (tf32 training mode): S = q k^T, P = softmax(S | bitmap),
-    O = P v and the four gradient products are calls of the tcgen05 GEMM over (image, head) batches; P is kept for the
-    backward (B * heads * Q * K floats)."""
-
-    @staticmethod
-    def forward(ctx, k_, q, kk, v, bitmap, all_masked):
-        B, Q, Cc = q.shape
-        K = kk.shape[1]
-        H = k_.rt.head.num_heads
-        d = Cc // H
-        P = k_.new(B, H, Q, K)
-        bh = dict(batch=B * H, batch_inner=H)
-        # S[b,h,q,key] = q[b,q,h,:] . k[b,key,h,:]
-        k_.gemm(q, (Q * Cc, Cc, 1), kk, (K * Cc, Cc, 1), P, (H * Q * K, K, 1), Q, K, d, s2=(d, d, Q * K), **bh)
-        k_.chk(k_.lib.cgg_attn_softmax_rows(k_.h, _p(P), _p(bitmap), _p(all_masked), B, H, Q, K, k_.s()), 'cgg_attn_softmax_rows')
-        out = k_.new(B, Q, Cc)
-        # O[b,q,h,:] = sum_key P[b,h,q,key] v[b,key,h,:]
-        k_.gemm(P, (H * Q * K, K, 1), v, (K * Cc, 1, Cc), out, (Q * Cc, Cc, 1), Q, d, K, s2=(Q * K, d, d), **bh)
-        ctx.k = k_
-        ctx.save_for_backward(q, kk, v, P, out)
-        return out
-
-    @staticmethod
-    def backward(ctx, dout):
-        k_ = ctx.k
-        q, kk, v, P, out = ctx.saved_tensors
-        B, Q, Cc = q.shape
-        K = kk.shape[1]
-        H = k_.rt.head.num_heads
-        d = Cc // H
-        dout = dout.contiguous()
-        bh = dict(batch=B * H, batch_inner=H)
-        dS = k_.new(B, H, Q, K)
-        # dP[b,h,q,key] = dO[b,q,h,:] . v[b,key,h,:]
-        k_.gemm(dout, (Q * Cc, Cc, 1), v, (K * Cc, Cc, 1), dS, (H * Q * K, K, 1), Q, K, d, s2=(d, d, Q * K), **bh)
-        k_.chk(k_.lib.cgg_attn_dscore(k_.h, _p(P), _p(dS), _p(out), _p(dout), B, H, d, Q, K, k_.s()), 'cgg_attn_dscore')
-        dq, dk, dv = k_.new(B, Q, Cc), k_.new(B, K, Cc), k_.new(B, K, Cc)
-        # dq[b,q,h,:] = sum_key dS k ;  dk[b,key,h,:] = sum_q dS q ;  dv[b,key,h,:] = sum_q P dO
-        k_.gemm(dS, (H * Q * K, K, 1), kk, (K * Cc, 1, Cc), dq, (Q * Cc, Cc, 1), Q, d, K, s2=(Q * K, d, d), **bh)
-        k_.gemm(dS, (H * Q * K, 1, K), q, (Q * Cc, 1, Cc), dk, (K * Cc, Cc, 1), K, d, Q, s2=(Q * K, d, d), a_mmajor=True, **bh)
-        k_.gemm(P, (H * Q * K, 1, K), dout, (Q * Cc, 1, Cc), dv, (K * Cc, Cc, 1), K, d, Q, s2=(Q * K, d, d), a_mmajor=True, **bh)
-        return None, dq, dk, dv, None, None
+        k_.chk(k_.lib.cgg_attention_backward(k_.h, B, Q, K, heads, _p(q), _p(kk), _p(v), Cc, K * Cc, _p(bitmap),
+                                             _p(all_masked), _p(out), _p(dout), _p(dq), _p(dk), _p(dv), Cc, K * Cc,
+                                             _p(scratch), k_.s()), 'cgg_attention_backward')
+        return None, dq, dk, dv, None, None, None
 
 
 class _AttentionViews(torch.autograd.Function):
-    """softmax(scale * q k^T | bitmap) v for (B, L, H, d) VIEWS q4, k4, v4 (last stride 1, any row / head / batch strides:
-    e.g. the three slices of a fused qkv projection) -> (B, Lq, H*d) contiguous.  Same products as _AttentionGemm, any
-    head count / head dim; a bit set in bitmap (B, Lq, ceil(Lk/32)) excludes the key, a row with no key left gives zeros.
-    Used by the caption transformer (row f4: 8 heads x 96)."""
+    """softmax(scale * q k^T | bitmap) v as tensor-core products, the GEMM-form attention of the decoder's tf32 training
+    mode and of the caption transformer (row f4: 8 heads x 96).  q4, k4, v4 are (B, L, H, d) VIEWS (last stride 1, any
+    row / head / batch strides: e.g. the three slices of a fused qkv projection) -> (B, Lq, H*d) contiguous.
+    S = q k^T, P = softmax(S | bitmap), O = P v and the four gradient products are calls of the tcgen05 GEMM over
+    (image, head) batches; P is kept for the backward (B * H * Lq * Lk floats).  A bit set in bitmap (B, Lq, ceil(Lk/32))
+    excludes the key; an all_masked row attends every key; a row with no key left gives zeros."""
 
     @staticmethod
-    def forward(ctx, k_, q4, k4, v4, bitmap, scale):
+    def forward(ctx, k_, q4, k4, v4, bitmap, all_masked, scale):
         B, Lq, H, d = q4.shape
         Lk = k4.shape[1]
         for t in (q4, k4, v4):
@@ -379,10 +336,12 @@ class _AttentionViews(torch.autograd.Function):
         P = k_.new(B, H, Lq, Lk)
         bh = dict(batch=B * H, batch_inner=H)
         sq, sk, sv = q4.stride(), k4.stride(), v4.stride()
+        # S[b,h,q,key] = scale * q[b,q,h,:] . k[b,key,h,:]
         k_.gemm(q4, (sq[0], sq[1], 1), k4, (sk[0], sk[1], 1), P, (H * Lq * Lk, Lk, 1), Lq, Lk, d, s2=(sq[2], sk[2], Lq * Lk),
                 alpha=scale, **bh)
-        k_.chk(k_.lib.cgg_attn_softmax_rows(k_.h, _p(P), _p(bitmap), None, B, H, Lq, Lk, k_.s()), 'cgg_attn_softmax_rows')
+        k_.chk(k_.lib.cgg_attn_softmax_rows(k_.h, _p(P), _p(bitmap), _p(all_masked), B, H, Lq, Lk, k_.s()), 'cgg_attn_softmax_rows')
         out = k_.new(B, Lq, H * d)
+        # O[b,q,h,:] = sum_key P[b,h,q,key] v[b,key,h,:]
         k_.gemm(P, (H * Lq * Lk, Lk, 1), v4, (sv[0], 1, sv[1]), out, (Lq * H * d, H * d, 1), Lq, d, Lk, s2=(Lq * Lk, sv[2], d), **bh)
         ctx.k, ctx.scale = k_, scale
         ctx.save_for_backward(q4, k4, v4, P, out)
@@ -399,16 +358,18 @@ class _AttentionViews(torch.autograd.Function):
         bh = dict(batch=B * H, batch_inner=H)
         sq, sk, sv = q4.stride(), k4.stride(), v4.stride()
         dS = k_.new(B, H, Lq, Lk)
+        # dP[b,h,q,key] = dO[b,q,h,:] . v[b,key,h,:]
         k_.gemm(dout, (Lq * Cc, Cc, 1), v4, (sv[0], sv[1], 1), dS, (H * Lq * Lk, Lk, 1), Lq, Lk, d, s2=(d, sv[2], Lq * Lk), **bh)
         k_.chk(k_.lib.cgg_attn_dscore(k_.h, _p(P), _p(dS), _p(out), _p(dout), B, H, d, Lq, Lk, k_.s()), 'cgg_attn_dscore')
         dq, dk, dv = k_.new(B, Lq, H, d), k_.new(B, Lk, H, d), k_.new(B, Lk, H, d)
+        # dq[b,q,h,:] = scale * sum_key dS k ;  dk[b,key,h,:] = scale * sum_q dS q ;  dv[b,key,h,:] = sum_q P dO
         k_.gemm(dS, (H * Lq * Lk, Lk, 1), k4, (sk[0], 1, sk[1]), dq, (Lq * Cc, Cc, 1), Lq, d, Lk, s2=(Lq * Lk, sk[2], d),
                 alpha=scale, **bh)
         k_.gemm(dS, (H * Lq * Lk, 1, Lk), q4, (sq[0], 1, sq[1]), dk, (Lk * Cc, Cc, 1), Lk, d, Lq, s2=(Lq * Lk, sq[2], d),
                 alpha=scale, a_mmajor=True, **bh)
         k_.gemm(P, (H * Lq * Lk, 1, Lk), dout, (Lq * Cc, 1, Cc), dv, (Lk * Cc, Cc, 1), Lk, d, Lq, s2=(Lq * Lk, d, d),
                 a_mmajor=True, **bh)
-        return None, dq, dk, dv, None, None
+        return None, dq, dk, dv, None, None, None
 
 
 class _GradSink:
@@ -476,7 +437,9 @@ def decoder_forward_train(head, mask_features, multi_scale_memorys, forced_attn_
     B, Cc, H4, W4 = mf.shape
     Q, L = head.num_queries, head.num_transformer_decoder_layers
     sizes = [tuple(m.shape[-2:]) for m in mems]
-    scale = 1.0 / math.sqrt(Cc // head.num_heads)
+    H = head.num_heads
+    d = Cc // H
+    scale = 1.0 / math.sqrt(d)
     dec = head.transformer_decoder
     qe = head.query_embed.weight
     with torch.no_grad():
@@ -509,7 +472,13 @@ def decoder_forward_train(head, mask_features, multi_scale_memorys, forced_attn_
     def ln(x, m):
         return _LayerNorm.apply(k, x, m.weight, m.bias, 1e-5)
 
-    attention = _AttentionGemm if k.tf32 else _Attention          # fp32: the flash-style FMA kernels (exact mode)
+    def attention(q, kk, v, bm, am):
+        """q (B * Q, C) scaled, k / v (B * K, C) -> (B, Q, C): the tcgen05 products in the tf32 mode, the flash-style FMA
+        kernels (exact mode) in fp32."""
+        if k.tf32:
+            return _AttentionViews.apply(k, q.view(B, Q, H, d), kk.view(B, -1, H, d), v.view(B, -1, H, d), bm, am, 1.0)
+        return _Attention.apply(k, q.view(B, Q, Cc), kk.view(B, -1, Cc), v.view(B, -1, Cc), bm, am, H)
+
     cls_list, emb_list, mask_list = [], [], []
     mf_sink = _GradSink()
 
@@ -542,7 +511,7 @@ def decoder_forward_train(head, mask_features, multi_scale_memorys, forced_attn_
         q = lin_in(xq, ca, 0, scale)
         kk = lin_in(key_in.view(B * K, Cc), ca, 1)
         vv = lin_in(val_in.view(B * K, Cc), ca, 2)
-        o = attention.apply(k, q.view(B, Q, Cc), kk.view(B, K, Cc), vv.view(B, K, Cc), bm, am)
+        o = attention(q, kk, vv, bm, am)
         t = lin(o.view(B * Q, Cc), ca.out_proj, res=x2d)
         x1 = ln(t, layer.norms[0])
         # ---- self-attention: q = k-input = x1 + query_embed, v-input = x1
@@ -550,7 +519,7 @@ def decoder_forward_train(head, mask_features, multi_scale_memorys, forced_attn_
         q2 = lin_in(x1q, sa, 0, scale)
         k2 = lin_in(x1q, sa, 1)
         v2 = lin_in(x1, sa, 2)
-        o2 = attention.apply(k, q2.view(B, Q, Cc), k2.view(B, Q, Cc), v2.view(B, Q, Cc), None, None)
+        o2 = attention(q2, k2, v2, None, None)
         t2 = lin(o2.view(B * Q, Cc), sa.out_proj, res=x1)
         x2 = ln(t2, layer.norms[1])
         # ---- FFN

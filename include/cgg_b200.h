@@ -286,12 +286,13 @@ int cgg_mem_prep_backward(cgg_handle *h, const float *dkey_in, const float *dval
 /* mmdet SinePositionalEncoding(normalize=True) of an (hh, ww) map -> (hh*ww, C) fp32 (head.py:798-804) */
 int cgg_sine_pos(cgg_handle *h, float *out, int hh, int ww, int C, void *stream);
 /* softmax(q k^T + mask) v for num_q queries (cross-attention: Q queries; self-attention: num_q = num_keys), fp32, and
- * its backward (dq, dk, dv; softmax recomputed from the saved q, k; bitmap as in the forward).
+ * its backward (dq, dk, dv; softmax recomputed from the saved q, k; bitmap as in the forward).  `heads` heads of 32
+ * channels: q, out, dout, dq rows of heads * 32; kv_stride >= heads * 32.
  * scratch: 2 * batch * heads * num_q floats. */
-int cgg_attention_f32(cgg_handle *h, int batch, int num_q, int num_keys, const float *q, const float *k, const float *v,
-                      long kv_stride, long kv_batch_stride, const uint32_t *bitmap, const uint8_t *all_masked,
-                      float *out, void *stream);
-int cgg_attention_backward(cgg_handle *h, int batch, int num_q, int num_keys, const float *q, const float *k,
+int cgg_attention_f32(cgg_handle *h, int batch, int num_q, int num_keys, int heads, const float *q, const float *k,
+                      const float *v, long kv_stride, long kv_batch_stride, const uint32_t *bitmap,
+                      const uint8_t *all_masked, float *out, void *stream);
+int cgg_attention_backward(cgg_handle *h, int batch, int num_q, int num_keys, int heads, const float *q, const float *k,
                            const float *v, long kv_stride, long kv_batch_stride, const uint32_t *bitmap,
                            const uint8_t *all_masked, const float *out, const float *dout, float *dq, float *dk,
                            float *dv, long dkv_stride, long dkv_batch_stride, float *scratch, void *stream);
@@ -301,7 +302,7 @@ int cgg_attention_backward(cgg_handle *h, int batch, int num_q, int num_keys, co
  *   cgg_attn_softmax_rows: scores -> softmax over the keys the bitmap leaves (all keys for all_masked rows; a row with
  *                          no key left becomes zeros);
  *   cgg_attn_dscore:       dprobs -> probs * (dprobs - D),  D[b,h,q] = dout[b,q,h,:] . out[b,q,h,:].
- * heads / head_dim: 0 = the handle's (8 x 32); the caption transformer (row f4) passes its own (8 x 96). */
+ * heads, head_dim >= 1: the decoder's attention runs 8 x 32, the caption transformer's (row f4) 8 x 96. */
 int cgg_attn_softmax_rows(cgg_handle *h, float *scores, const uint32_t *bitmap, const uint8_t *all_masked, int batch,
                           int heads, int num_q, int num_keys, void *stream);
 int cgg_attn_dscore(cgg_handle *h, const float *probs, float *dprobs, const float *out, const float *dout, int batch,

@@ -120,10 +120,10 @@ def test_two_level_batch_matches_fp64(kern):
 
 
 @pytest.mark.parametrize('Q,K,masked', [(40, 320, True), (24, 20, True), (100, 100, False), (200, 4096, True)])
-def test_attention_as_tensor_core_products_matches_fp32_kernels(kern, Q, K, masked):
-    """_AttentionGemm (tf32 products + row softmax with the bitmap) against the flash-style fp32 kernels: forward and
-    the three gradients, including all-masked fallback rows."""
-    from cgg_b200.train import _Attention, _AttentionGemm
+def test_attention_views_as_tensor_core_products_match_fp32_kernels(kern, Q, K, masked):
+    """_AttentionViews (tf32 products + row softmax with the bitmap) on (B, L, 8, 32) views, the decoder's tf32 attention,
+    against the flash-style fp32 kernels: forward and the three gradients, including all-masked fallback rows."""
+    from cgg_b200.train import _Attention, _AttentionViews
     B, Cc = 2, 256
     g = torch.Generator().manual_seed(Q + K)
     mk = lambda *s: (torch.randn(s, generator=g) * 0.5).to(DEV).requires_grad_(True)
@@ -137,9 +137,9 @@ def test_attention_as_tensor_core_products_matches_fp32_kernels(kern, Q, K, mask
         am = m.all(-1).to(torch.uint8).to(DEV)
     k32 = _K(kern.rt, tf32=False)
     dout = torch.randn((B, Q, Cc), generator=g).to(DEV)
-    o_ref = _Attention.apply(k32, q, kk, v, bitmap, am)
+    o_ref = _Attention.apply(k32, q, kk, v, bitmap, am, 8)
     g_ref = torch.autograd.grad(o_ref, (q, kk, v), dout)
-    o = _AttentionGemm.apply(kern, q, kk, v, bitmap, am)
+    o = _AttentionViews.apply(kern, q.view(B, Q, 8, 32), kk.view(B, K, 8, 32), v.view(B, K, 8, 32), bitmap, am, 1.0)
     g_tc = torch.autograd.grad(o, (q, kk, v), dout)
     torch.cuda.synchronize()
     assert float((o - o_ref).abs().max()) < 5e-3 * float(o_ref.abs().max())

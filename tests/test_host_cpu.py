@@ -32,6 +32,32 @@ def test_library_exports_every_declared_symbol(lib):
     assert set(clib.EXPORTS) == declared
 
 
+def test_argtypes_match_header_prototypes(lib):
+    """Every argtypes list of lib.py against its prototype in include/cgg_b200.h: arity, pointer versus scalar, and for
+    scalars the width and float versus integer.  ctypes passes whatever argtypes says, so a list left behind by an ABI
+    change shifts every later argument without any error."""
+    hdr = open(os.path.join(ROOT, 'include', 'cgg_b200.h')).read()
+    hdr = re.sub(r'//[^\n]*', '', re.sub(r'/\*.*?\*/', '', hdr, flags=re.S))
+    protos = re.findall(r'\b(cgg_\w+)\s*\(([^()]*)\)\s*;', hdr)
+    assert {name for name, _ in protos} == set(clib.EXPORTS)
+    scalars = {'int': C.c_int, 'long': C.c_long, 'size_t': C.c_size_t, 'float': C.c_float, 'double': C.c_double}
+
+    def kind(t):    # ('ptr',) or (float?, bytes)
+        if isinstance(t, str):
+            if '*' in t or '[' in t:
+                return ('ptr',)
+            t = scalars[' '.join(t.split()[:-1])]
+        if t in (C.c_void_p, C.c_char_p) or issubclass(t, C._Pointer):
+            return ('ptr',)
+        return (t in (C.c_float, C.c_double), C.sizeof(t))
+
+    for name, params in protos:
+        want = [kind(p) for p in params.split(',')] if params.strip() != 'void' else []
+        got = getattr(lib, name).argtypes
+        assert got is not None or not want, name + ': no argtypes'
+        assert [kind(t) for t in got or []] == want, name
+
+
 def test_version_names_sm100a(lib):
     assert b'sm_100a' in lib.cgg_version()
 
