@@ -1466,7 +1466,11 @@ int tc_mask_einsum(TcState* t, int batch, int first_call, int num_calls, const v
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, "mask out, swizzled", &t->err))
       return CGG_ERR_CUDA;
     const size_t e_chunk = (size_t)p.q_rows * 128;
-    const size_t smem = 1024 + 4 * A_CHUNK_BYTES + 8 * e_chunk + 4 * e_chunk + 24 * 8 + 64;
+    // The MMA reads 128 rows of every E chunk (rows past q_rows land in TMEM lanes that are never stored).  From the
+    // last ring chunk that read ends 7 e_chunk + 16 KB past the ring's start; below ~26 rows per chunk (Q <= 24) it
+    // would run past the staging tiles and barriers out of the allocation, which is extended to cover it.
+    const size_t e_read_end = 7 * e_chunk + 128 * 128, e_alloc = 12 * e_chunk + 24 * 8 + 64;
+    const size_t smem = 1024 + 4 * A_CHUNK_BYTES + (e_read_end > e_alloc ? e_read_end : e_alloc);
     return launch_pairs(t, tc_einsum_t_kernel, smem, s, mA, mB, mC, p, HW, batch);
   }
   // pixel-on-lane CTA-pair kernel: q_pad / N_TILE tiles per head call, each CTA loads N_TILE/2 rows of every B chunk

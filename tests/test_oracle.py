@@ -105,6 +105,21 @@ def test_bilinear_matches_torch():
         assert bool(((a.sigmoid() < 0.5) == (b.sigmoid() < 0.5)).all())
 
 
+def test_level_resample_formula_is_torch_bilinear():
+    """The reference of the bf16 path's level resample (test_gpu_bf16_stages.level_resample_ref, the arithmetic of
+    downsample3_kernel) is torch's bilinear resize: on bf16-valued inputs, what the pixel decoder hands the head,
+    fp16(formula) == fp16(F.interpolate(bilinear, align_corners=False)) bit for bit at the ratios 8, 4 and 2.  The
+    comparison is made in fp16, the precision the resampled features are stored in: in fp32, torch's vectorised CPU
+    loop rounds a few in 10^6 values one ulp differently at ratios 4 and 8."""
+    import torch.nn.functional as F
+    from test_gpu_bf16_stages import RATIOS, level_resample_ref
+    mf = torch.randn((2, 256, 264, 200), generator=torch.Generator().manual_seed(0)).bfloat16()
+    for r in RATIOS:
+        want = F.interpolate(mf.float(), (264 // r, 200 // r), mode='bilinear', align_corners=False).half()
+        got = level_resample_ref(mf, r).half()
+        assert torch.equal(got.view(torch.int16), want.view(torch.int16)), r
+
+
 def test_pack_bits_layout():
     m = torch.zeros(1, 2, 40, dtype=torch.bool)
     m[0, 0, 0] = m[0, 0, 31] = m[0, 0, 33] = True
