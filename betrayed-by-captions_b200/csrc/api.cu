@@ -406,12 +406,21 @@ extern "C" int cgg_mask_einsum(cgg_handle* h, int batch, int first_call, int num
 
 extern "C" int cgg_masked_attention(cgg_handle* h, int batch, int num_keys, const float* q, const void* k,
                                     const void* v, long kv_stride, long kv_batch_stride, const uint32_t* bitmap,
-                                    const uint8_t* all_masked, float* out, void* stream) {
-  if (!h || !q || !k || !v || !out) return CGG_ERR_NULL;
+                                    const uint8_t* all_masked, int layer, float* out, void* out_half, void* stream) {
+  if (!h || !q || !k || !v || (!out && !out_half)) return CGG_ERR_NULL;
   if (batch <= 0 || num_keys <= 0) return fail(h, CGG_ERR_BAD_SHAPE, "bad shape");
+  if (layer < -1 || layer >= h->cfg.num_layers) return fail(h, CGG_ERR_BAD_SHAPE, "bad layer index");
+  if (h->cfg.precision != CGG_BF16 && (layer >= 0 || out_half))
+    return fail(h, CGG_ERR_UNSUPPORTED, "key-bias table and half output are CGG_BF16 options (fp32 keys carry their bias)");
+  if (layer >= 0) {
+    const int l = layer % CGG_NUM_LEVELS;
+    if (!h->prepared) return fail(h, CGG_ERR_BAD_SHAPE, "a layer's key-bias table needs cgg_prepare()");
+    if (num_keys != h->lh[l] * h->lw[l]) return fail(h, CGG_ERR_BAD_SHAPE, "num_keys is not the layer level's key count");
+  }
   cudaStream_t s = (cudaStream_t)stream;
   if (h->cfg.precision == CGG_BF16) {
-    TC(h->tc, tc_attention(h->tc, batch, num_keys, q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked, out, nullptr, s));
+    TC(h->tc, tc_layer_attention(h->tc, layer, batch, num_keys, q, k, v, kv_stride, kv_batch_stride, bitmap, all_masked,
+                                 out, out_half, s));
     return CGG_OK;
   }
   CU(launch_attention_f32(q, (const float*)k, (const float*)v, kv_stride, kv_batch_stride, bitmap, all_masked, out, batch,
@@ -465,7 +474,7 @@ static int decoder_layer_impl(cgg_handle* h, const cgg_weights* w, int batch, in
   const long kv_stride = (long)n * 2 * C, kv_bstride = (long)K * kv_stride;
   const float* kv = at<float>(workspace, ws.kv[l]);
   ST(cgg_masked_attention(h, batch, K, qb, kv + (size_t)sl * C, kv + (size_t)(n + sl) * C, kv_stride, kv_bstride,
-                          bitmap, all_masked, o, stream));
+                          bitmap, all_masked, -1, o, nullptr, stream));
   ST(linear_rows(h, s, o, nullptr, 1, lw.cross_out_w, lw.cross_out_b, t, rows, C, C, 1.f, x_in));
   CU(launch_layernorm(t, nullptr, lw.norm_w[0], lw.norm_b[0], x1, rows, C, 1e-5f, true, s));
   // ---- self-attention (K6): q = k-input = x1 + query_embed, v-input = x1

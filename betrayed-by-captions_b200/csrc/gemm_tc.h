@@ -90,5 +90,10 @@ int tc_attention(TcState* t, int batch, int num_keys, const float* q, const void
 // r_table: optional bf16 (num_keys, r_cols) key-bias table stored as [hi | lo] column halves;
 // S += Q . (R_hi + R_lo)[:, r_col0 + head*32 ...]^T
 const void* tc_key_bias_table(const TcState* t, int level, long* cols);
+// K5 with the arguments of decoder layer `layer`'s cross-attention (its level's key-bias table at its slot's columns),
+// or without a table for layer < 0; out fp32 and / or out_half IEEE half rows (either may be null).
+int tc_layer_attention(TcState* t, int layer, int batch, int num_keys, const float* q, const void* k, const void* v,
+                       long kv_stride, long kv_bstride, const uint32_t* bitmap, const uint8_t* all_masked, float* out,
+                       void* out_half, cudaStream_t s);
 
 }  // namespace cgg

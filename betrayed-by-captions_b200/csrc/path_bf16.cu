@@ -262,6 +262,23 @@ int tc_query_heads(TcState* t, const cgg_weights* w, int batch, const float* x, 
   return CGG_OK;
 }
 
+// K5 as the decoder layer calls it, shared with the cgg_masked_attention stage entry.  layer >= 0: the cross-attention
+// of that layer, with the key-bias table of its level (layer % 3) at the columns of its slot (layer / 3); layer < 0: no
+// table.  out: fp32 rows, out_half: IEEE half rows (either may be null).
+int tc_layer_attention(TcState* t, int layer, int batch, int num_keys, const float* q, const void* k, const void* v,
+                       long kv_stride, long kv_bstride, const uint32_t* bitmap, const uint8_t* all_masked, float* out,
+                       void* out_half, cudaStream_t s) {
+  long rcols = 0;
+  const void* rtab = nullptr;
+  int r_col0 = 0;
+  if (layer >= 0) {
+    rtab = tc_key_bias_table(t, layer % CGG_NUM_LEVELS, &rcols);
+    r_col0 = layer / CGG_NUM_LEVELS * t->cfg.embed_dim;
+  }
+  return tc_attention(t, batch, num_keys, q, k, v, kv_stride, kv_bstride, bitmap, all_masked, out,
+                      static_cast<__nv_bfloat16*>(out_half), s, rtab, rcols, r_col0, /*out_mode: IEEE half*/ 2);
+}
+
 // K5 + K6: one DetrTransformerDecoderLayer (head.py:829-840), bf16 operands on tensor cores.
 int tc_decoder_layer(TcState* t, const cgg_weights* w, int batch, int layer, const float* x_in, const void* k,
                      const void* v, long kv_stride, long kv_bstride, int num_keys, const uint32_t* bitmap,
@@ -296,13 +313,7 @@ int tc_decoder_layer(TcState* t, const cgg_weights* w, int batch, int layer, con
     TcSeg sq[1] = {seg(0, C, qf, C, false, false, qscale)};
     TST(tc_linear(t, xqb, M, C, pw.wq_c, C, lw.cross_in_b, sq, 1, s, false, 1, 0, /*f16=*/true));
   }
-  {
-    const int level = layer % CGG_NUM_LEVELS, slot = layer / CGG_NUM_LEVELS;
-    long rcols = 0;
-    const void* rtab = tc_key_bias_table(t, level, &rcols);
-    TST(tc_attention(t, batch, num_keys, qf, k, v, kv_stride, kv_bstride, bitmap, all_masked, nullptr, ob, s, rtab, rcols,
-                     slot * C, /*out_mode: IEEE half*/ 2));
-  }
+  TST(tc_layer_attention(t, layer, batch, num_keys, qf, k, v, kv_stride, kv_bstride, bitmap, all_masked, nullptr, ob, s));
   // x1 = LN(x + o Wo^T + bo);  also bf16(x1 + query_embed) for the self-attention projections
   TcSeg so[1] = {seg(0, C, t1, C, false, false, 1.f, nullptr, 1, 0, false, x_in, C)};
   TST(tc_linear(t, ob, M, C, pw.wo_c, C, lw.cross_out_b, so, 1, s, false, 1, 0, true));
@@ -313,8 +324,7 @@ int tc_decoder_layer(TcState* t, const cgg_weights* w, int batch, int layer, con
                  seg(2 * C, C, kvb + C, 2 * C, true, false, 1.f, pw.rowbias_v, Q, C)};
   TST(tc_linear(t, xqb, M, C, pw.wqkv_s, 3 * C, lw.self_in_b, sk, 3, s, false, 1, 0, true));
   // the 100 x 100 self-attention runs on the same tcgen05 attention kernel (one key tile, no mask)
-  TST(tc_attention(t, batch, Q, qs, kvb, kvb + C, 2 * C, (long)Q * 2 * C, nullptr, nullptr, nullptr, ob, s, nullptr, 0, 0,
-                   /*out_mode: IEEE half*/ 2));
+  TST(tc_layer_attention(t, -1, batch, Q, qs, kvb, kvb + C, 2 * C, (long)Q * 2 * C, nullptr, nullptr, nullptr, ob, s));
   TcSeg so2[1] = {seg(0, C, t1, C, false, false, 1.f, nullptr, 1, 0, false, x1, C)};
   TST(tc_linear(t, ob, M, C, pw.wo_s, C, lw.self_out_b, so2, 1, s, false, 1, 0, true));
   TCU(launch_ln_rows(t1, lw.norm_w[1], lw.norm_b[1], M, x2, xb, nullptr, nullptr, 0, nullptr, s));

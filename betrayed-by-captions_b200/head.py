@@ -629,17 +629,22 @@ class _Runtime:
         _lib.check(st, self.handle, 'cgg_attn_mask_from_logits')
         return bm, am
 
-    def masked_attention(self, q, k, v, bitmap=None, all_masked=None):
-        """q (B,Q,C) pre-scaled fp32; k, v (B,K,C) contiguous (fp32 in fp32 mode, bf16 in bf16 mode)."""
+    def masked_attention(self, q, k, v, bitmap=None, all_masked=None, layer=-1, out_half=False):
+        """q (B,Q,C) pre-scaled fp32; k, v (B,K,C) views with unit channel stride and the same strides (fp32 in fp32
+        mode, bf16 in bf16 mode), e.g. column slices of one K/V buffer.  layer >= 0 (bf16 mode): add decoder layer
+        `layer`'s key-bias table to the keys, as that layer's cross-attention does.  Returns the fp32 output, or
+        (fp32, IEEE half) outputs of the same launch with out_half=True."""
         B, Q, Cc = q.shape
         K = k.shape[1]
+        assert k.stride() == v.stride() and k.stride(-1) == 1 and k.shape == v.shape, (k.stride(), v.stride())
         out = torch.empty_like(q)
-        st = self.lib.cgg_masked_attention(self.handle, B, K, _ptr(q), _ptr(k), _ptr(v), Cc, K * Cc,
+        half = torch.empty(q.shape, dtype=torch.float16, device=q.device) if out_half else None
+        st = self.lib.cgg_masked_attention(self.handle, B, K, _ptr(q), _ptr(k), _ptr(v), k.stride(1), k.stride(0),
                                            _ptr(bitmap) if bitmap is not None else None,
-                                           _ptr(all_masked) if all_masked is not None else None, _ptr(out),
-                                           self._stream())
+                                           _ptr(all_masked) if all_masked is not None else None, layer, _ptr(out),
+                                           _ptr(half) if out_half else None, self._stream())
         _lib.check(st, self.handle, 'cgg_masked_attention')
-        return out
+        return (out, half) if out_half else out
 
     # ---- grounding side
     def similarity(self, a, b, scale):

@@ -112,7 +112,7 @@ def load():
     lib.cgg_mask_einsum.argtypes = [vp, i, i, i, vp, vp, vp, sz, vp]
     lib.cgg_attn_mask_from_logits.argtypes = [vp, i, vp, i, i, i, i, vp, vp, vp]
     lib.cgg_decoder_layer.argtypes = [vp, C.POINTER(Weights), i, i, vp, vp, vp, vp, vp, sz, vp]
-    lib.cgg_masked_attention.argtypes = [vp, i, i, vp, vp, vp, C.c_long, C.c_long, vp, vp, vp, vp]
+    lib.cgg_masked_attention.argtypes = [vp, i, i, vp, vp, vp, C.c_long, C.c_long, vp, vp, i, vp, vp, vp]
     lib.cgg_noun_embeddings.argtypes = [vp, vp, vp, vp, vp, i, i, C.c_float, i, vp, vp]
     lib.cgg_similarity.argtypes = [vp, vp, vp, i, i, i, C.c_float, vp, vp]
     lib.cgg_grounding_scratch_bytes.argtypes = [i, i, i]

@@ -181,13 +181,20 @@ int cgg_decoder_layer(cgg_handle *h, const cgg_weights *w, int batch, int layer,
                       const float *x_in, const uint32_t *bitmap, const uint8_t *all_masked,
                       float *x_out, void *workspace, size_t workspace_bytes, void *stream);
 
-/* K5 alone: masked multi-head cross-attention core softmax(q k^T + mask) v.
+/* K5 alone: masked multi-head cross-attention core, per head h (32 channels)
+ *   out[b,q,h] = softmax_k(s[b,q,k] + mask[b,q,k]) v[b,k,h],  s = q[b,q,h] . (k[b,k,h] + R[k,h])
  * q (B,Q,C) fp32 already scaled by 1/sqrt(d); k, v (B,K,C) fp32 (CGG_FP32) or bf16 with row
- * stride kv_stride elements; bitmap/all_masked may be NULL (= no mask). out (B,Q,C) fp32. */
+ * stride kv_stride and image stride kv_batch_stride elements (K and V may be column views of one
+ * buffer); bitmap/all_masked may be NULL (= no mask); a row with all_masked set attends to every key.
+ * layer: -1 = no key-bias term (R = 0).  0 <= layer < num_layers (CGG_BF16, prepared handle,
+ * num_keys = the key count of level layer % 3): R is the handle's key-bias table of decoder layer
+ * `layer`, (pos + level_embed) Wk^T + bk, exactly the call that layer's cross-attention makes.
+ * out (B,Q,C) fp32 and / or out_half (B,Q,C) IEEE half (CGG_BF16 only); one of them may be NULL,
+ * both given are written by the same launch.  At most 65536 keys in CGG_BF16 mode. */
 int cgg_masked_attention(cgg_handle *h, int batch, int num_keys, const float *q, const void *k,
                          const void *v, long kv_stride, long kv_batch_stride,
-                         const uint32_t *bitmap, const uint8_t *all_masked,
-                         float *out, void *stream);
+                         const uint32_t *bitmap, const uint8_t *all_masked, int layer,
+                         float *out, void *out_half, void *stream);
 
 /* ---- grounding side -------------------------------------------------------------- */
 

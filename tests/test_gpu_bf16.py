@@ -275,41 +275,3 @@ def test_bf16_full_size_1024_properties_other_routes(Q):
     the pixel-on-lane pair kernel with two N tiles and the attention-mask GEMM with two query slices.  (An accumulator
     overlap of the attention-mask GEMM at 129..256 queries once made two runs at Q = 200 differ within the 1e-2 bar.)"""
     _full_size_properties(Q)
-
-
-@pytest.mark.parametrize('K,density,blob', [(64, 0.5, False), (128, 0.0, False), (777, 0.9, False), (4096, 0.5, False),
-                                            (4096, 0.9, True), (16384, 0.5, True)])
-def test_bf16_masked_attention_stage(K, density, blob):
-    """K5 on tensor cores vs fp32 softmax(q k^T + mask) v on the same bf16-rounded operands; incl.
-    fallback rows, ragged key counts and blob-shaped masks (whole key tiles skipped)."""
-    B, Q, C = 2, 100, 256
-    sd = synth.make_params(seed=1, num_queries=Q)
-    head = build_head_from_state_dict(sd, Q, 49, 'bf16', DEV)
-    rt = head._runtime(torch.device(DEV, 0))
-    rt.prepare(64, 64, [(8, 8), (16, 16), (32, 32)], B)
-    g = torch.Generator().manual_seed(K + int(blob))
-    q = (torch.randn((B, Q, C), generator=g) * 0.4)
-    k = torch.randn((B, K, C), generator=g).bfloat16()
-    v = torch.randn((B, K, C), generator=g).bfloat16()
-    if blob:
-        # each query sees one contiguous window of keys: most 128-key tiles are masked for everyone
-        masked = torch.ones((B, Q, K), dtype=torch.bool)
-        start = torch.randint(0, max(1, K // 8), (B, Q), generator=g)
-        width = max(1, int(K * (1 - density) / 4))
-        for b in range(B):
-            for qi in range(Q):
-                masked[b, qi, start[b, qi]:start[b, qi] + width] = False
-    else:
-        masked = torch.rand((B, Q, K), generator=g) < density
-    masked[0, 0] = True                      # fully masked row -> fallback (attend everywhere)
-    masked[1, 5, : K // 2] = True
-    am = masked.all(-1)
-    eff = O.apply_fallback(masked)
-    qb = q.bfloat16().float()
-    s = torch.einsum('bqhd,bkhd->bhqk', qb.view(B, Q, 8, 32), k.float().view(B, K, 8, 32))
-    s = s.masked_fill(eff[:, None], float('-inf'))
-    want = torch.einsum('bhqk,bkhd->bqhd', torch.softmax(s, -1), v.float().view(B, K, 8, 32)).reshape(B, Q, C)
-    got = rt.masked_attention(q.to(DEV), k.to(DEV), v.to(DEV), O.pack_mask_bits(masked).to(DEV),
-                              am.to(torch.uint8).to(DEV))
-    err = float((got.cpu() - want).abs().max())
-    assert err < 1e-2 * float(want.abs().max()) + 2e-3, (err, float(want.abs().max()))

@@ -8,6 +8,9 @@ would still pass.
   K2  mask einsum        mask[call, b, q, p] = sum_c bf16(me)[b, call, q, c] mf[b, c, p]            (bf16 output)
   K3  attention-mask     bit = sum_c fp16(me)[b, q, c] fds_l[b, c, key] <= MASKED_LOGIT_MAX            (fp32 accumulate)
   K4  K/V projection     kv_l[b, key, :] = mem_l[b, :, key] [Wk; Wv]^T (+ level_embed Wv^T + bv on V)   (bf16 output)
+  K5  cross-attention    out[b, q, h] = softmax_k(bf16(q) . (k + R_layer) | mask) v, R the key-bias table of the layer,
+                         K / V the layer slot's column views of kv_l                     (fp32 and IEEE-half output)
+  K6  self-attention     the same kernel on K, V interleaved in one (B, Q, 2C) buffer, K = Q, no mask, no table
 
 Workspace layouts the tests read (each test asserts the one it relies on, so that a layout change fails loudly):
   me_all  (TcWs::carve, store_me_kernel): rows [image][call * q_pad + q], 2C wide; columns [0, C) bf16(me) (K2),
@@ -428,3 +431,436 @@ def test_k1_query_heads_within_propagated_bound(Q, ncls1):
         print('K1 Q=%d %s: worst %.3g of the bound, relative RMS error %.3g' % (Q, name, worst, rms))
         assert worst <= 1.0, (name, worst)
         assert rms <= K1_RMS_BAR[name], (name, rms)
+
+
+# ------------------------------------------------------------------------------------------------- K5 / K6 attention
+# K5 (cross-attention, cgg_masked_attention with `layer`: the handle's key-bias table, IEEE-half rows, K and V as the
+# column views of kv_l that tc_decoder_layer passes) and the K6 self-attention form (K and V interleaved in one
+# (B, Q, 2C) buffer, no bitmap) against tests/golden/attention_ref.py: exact on constructed scores (every score 0: a
+# masked mean; +-1 key codes: one-hot), elsewhere within the rounding bound of attention_ref.reference.
+import attention_ref as AR                       # noqa: E402
+from cgg_b200 import lib as _clib                 # noqa: E402
+from oracle import cgg_oracle as O               # noqa: E402
+
+# Relative RMS error (RMS(got - ref) / RMS(ref)) of the fp32 output, the largest over the cases of each kind in a
+# correct run on a B200 (1000 W power limit): production cross-attention ('prod') and random keys ('rand') at each q
+# scale, the score ramps and the two-level scores.  The bars are about 4x those values.
+K5_RMS_MEASURED = {('prod', 0.25): 6.0e-4, ('prod', 1.0): 7.6e-4, ('prod', 16.0): 3.0e-4,
+                   ('rand', 0.25): 1.6e-3, ('rand', 1.0): 9.4e-4, ('rand', 16.0): 2.4e-4,
+                   'ramp': 1.15e-3, 'two': 2.1e-3}
+K5_RMS_BAR = {key: 4 * val for key, val in K5_RMS_MEASURED.items()}
+
+
+def _attn_rt(Q, B, H=256, W=256, sd=None):
+    head = _head(Q, seed=1, sd=sd)
+    return _Stage(head, H, W, B)
+
+
+def _bits(masked, offset):
+    """bitmap (B, Q, W32) int32 on the device; offset: a view one word into its buffer (a misaligned base)."""
+    words = O.pack_mask_bits(masked)
+    if not offset:
+        return words.to(DEV)
+    buf = torch.zeros(words.numel() + 1, dtype=torch.int32)
+    buf[1:] = words.flatten()
+    return buf.to(DEV)[1:].view(words.shape)
+
+
+def _nan_kv(k, v):
+    """k, v (B, K, C) as column views of a NaN-filled (B, K, 4C) bf16 buffer: columns the call must not read are NaN."""
+    B, K, _ = k.shape
+    buf = torch.full((B, K, 4 * C), NAN16, dtype=torch.int16).view(torch.bfloat16)
+    buf[:, :, C:2 * C] = k.bfloat16()
+    buf[:, :, 3 * C:] = v.bfloat16()
+    buf = buf.to(DEV)
+    return buf[:, :, C:2 * C], buf[:, :, 3 * C:]
+
+
+def _attend(rt, q, k, v, masked=None, am=None, layer=-1, offset=False):
+    """Runs the attention twice (bit-identical, and out_half == fp16(out)) and, at B = 3, image 1 alone (bit-identical
+    to its rows of the batch).  k, v: device views.  Returns (out, out_half) on the CPU."""
+    qd = q.to(DEV)
+    bm = _bits(masked, offset) if masked is not None else None
+    amd = am.to(torch.uint8).to(DEV) if am is not None else None
+    runs = [rt.masked_attention(qd, k, v, bm, amd, layer=layer, out_half=True) for _ in range(2)]
+    out, half = runs[0][0].cpu(), runs[0][1].cpu()
+    assert torch.equal(out.view(torch.int32), runs[1][0].cpu().view(torch.int32)), 'two runs differ (fp32)'
+    assert torch.equal(half.view(torch.int16), runs[1][1].cpu().view(torch.int16)), 'two runs differ (half)'
+    assert torch.equal(half.view(torch.int16), out.half().view(torch.int16)), 'out_half != fp16(out)'
+    if q.shape[0] == 3:
+        one = lambda t: t[1:2] if t is not None else None
+        o1, h1 = rt.masked_attention(qd[1:2], k[1:2], v[1:2], one(bm), one(amd), layer=layer, out_half=True)
+        assert torch.equal(o1.cpu().view(torch.int32), out[1:2].view(torch.int32)), 'image alone != image in a batch'
+        assert torch.equal(h1.cpu().view(torch.int16), half[1:2].view(torch.int16)), 'image alone != image in a batch'
+    return out, half
+
+
+def _check_bound(what, out, half, ref, bound, rms_bar=None):
+    for name, got in (('fp32', out), ('half', half)):
+        err = (got.double() - ref).abs()
+        bad = err > bound
+        if bad.any():
+            b, qi, c = [int(x) for x in bad.nonzero()[0]]
+            raise AssertionError('%s %s: %d outputs outside the bound, first at image %d row %d head %d channel %d: got '
+                                 '%.9g want %.9g bound %.3g' % (what, name, int(bad.sum()), b, qi, c // 32, c % 32,
+                                                                float(got[b, qi, c]), float(ref[b, qi, c]),
+                                                                float(bound[b, qi, c])))
+    rms = float((out.double() - ref).pow(2).mean().sqrt() / ref.pow(2).mean().sqrt().clamp(min=1e-300))
+    worst = float(((out.double() - ref).abs() / bound.clamp(min=1e-300)).max())
+    print('K5 %s: worst %.3g of the bound, relative RMS error %.3g' % (what, worst, rms))
+    if rms_bar is not None:
+        assert rms <= rms_bar, '%s: relative RMS error %.3g above the bar %.3g' % (what, rms, rms_bar)
+
+
+def _live_mask(g, B, Q, K, counts):
+    """Rows of query tile qt of image b allow keys (density 1/2) only inside n = counts[(b * nqt + qt) % len] chosen
+    key tiles, so that exactly n tiles are live for that CTA (0: every row wholly masked)."""
+    nt, nqt = (K + AR.KT - 1) // AR.KT, (Q + 127) // 128
+    masked = torch.ones((B, Q, K), dtype=torch.bool)
+    for b in range(B):
+        for qt in range(nqt):
+            n = counts[(b * nqt + qt) % len(counts)]
+            tiles = torch.randperm(nt, generator=g)[:n]
+            rows = slice(qt * 128, min(Q, qt * 128 + 128))
+            for t in tiles.tolist():
+                cols = slice(t * AR.KT, min(K, t * AR.KT + AR.KT))
+                blk = masked[b, rows, cols]
+                blk[:] = torch.rand(blk.shape, generator=g) < 0.5
+                blk[:, 0] = False                     # the tile is live for every row
+    return masked
+
+
+LIVE_COUNTS = (0, 1, 2, 3, 4, 6, 7)
+# (Q, B, K, mask): 1..4 query tiles with rows >= Q in the last; the key tail inside a word and in a new word; 1..3 key
+# tiles (fewer than the three score buffers); the 6-stage ring boundary (769 keys = 7 tiles); 512 tiles at 65536 keys.
+# 'live': exactly LIVE_COUNTS live tiles per CTA among 32 or more; 'blob': windows; the masks with a '+' run the
+# bitmap's word path on a base one word off the alignment (W32 % 4 == 0 takes the vector path otherwise).
+K5_EXACT_CASES = [(8, 3, 1, 'rand'), (8, 3, 31, 'rand'), (100, 3, 33, 'rand+'), (100, 3, 64, 'rand'),
+                  (100, 3, 99, 'rand'), (128, 3, 128, 'rand+'), (129, 3, 129, 'rand'), (129, 1, 383, 'blob'),
+                  (300, 3, 385, 'rand'), (300, 1, 768, 'rand'), (512, 1, 769, 'rand'), (100, 3, 825, 'rand+'),
+                  (512, 3, 4096, 'live'), (129, 3, 4096, 'live+'), (100, 1, 16384, 'blob'), (8, 1, 65536, 'rand'),
+                  (100, 1, 65536, 'blob+')]
+
+
+@pytest.mark.parametrize('Q,B,K,kind', K5_EXACT_CASES)
+def test_k5_exact_masked_mean(Q, B, K, kind):
+    """Case a: q = 0, so every score is 0 and every allowed key has P = exp2(0) = 1; l is the count of allowed keys, O
+    an exact integer sum of V in [-8, 8] (< 2^24), and no rescale happens.  out must EQUAL f32(sum) * f32(1 / l) (IEEE
+    division, no fast math), out_half fp16 of that, and a row without an allowed key (a full bitmap row without the
+    all-masked flag; with 'live' whole CTAs of them: no live tile) zeros.  One wrong mask bit, tail bit, live-tile
+    flag, fallback row or quarter merge changes a count or a sum.  Relies on ex2.approx giving exactly 1 at 0 and 0 at
+    -inf.  Also at 396 keys with layer 4's key-bias table: q = 0 makes the table's term 0 as well."""
+    st = _attn_rt(Q, B)
+    g = torch.Generator().manual_seed(Q * 7 + K)
+    base = kind.rstrip('+')
+    if base == 'live':
+        masked, am = _live_mask(g, B, Q, K, LIVE_COUNTS), None
+    else:
+        masked = AR.random_mask(g, B, Q, K, 0.9 if base == 'blob' else 0.5, blob=base == 'blob')
+        am = masked.all(-1)
+        am[B - 1, Q - 1] = False                           # a wholly masked row without the flag: no allowed key
+        masked[B - 1, Q - 1] = True
+    allowed = AR.effective_allowed(masked, am).double()
+    k = AR.bf16(torch.randn((B, K, C), generator=g))
+    v = torch.randint(-8, 9, (B, K, C), generator=g).float()
+    kd, vd = _nan_kv(k, v)
+    out, half = _attend(st.rt, torch.zeros((B, Q, C)), kd, vd, masked, am, offset=kind.endswith('+'))
+    cnt = allowed.sum(-1, keepdim=True).numpy().astype(np.float32)
+    sums = (allowed @ v.double()).numpy().astype(np.float32)
+    with np.errstate(divide='ignore'):
+        inv = np.where(cnt > 0, np.float32(1) / cnt, np.float32(0)).astype(np.float32)
+    want = torch.from_numpy(sums * inv)
+    assert not out.isnan().any(), 'NaN in the output'
+    bad = out != want
+    assert not bad.any(), '%d outputs differ, first at %s' % (int(bad.sum()), bad.nonzero()[0].tolist())
+    assert torch.equal(half.view(torch.int16), want.half().view(torch.int16))
+
+
+def test_k5_exact_masked_mean_with_table():
+    B, Q, H, W, layer = 3, 100, 352, 288, 4
+    st = _attn_rt(Q, B, H, W)
+    K = st.K[layer % 3]
+    g = torch.Generator().manual_seed(4)
+    masked = AR.random_mask(g, B, Q, K, 0.5)
+    am = masked.all(-1)
+    v = torch.randint(-8, 9, (B, K, C), generator=g).float()
+    kd, vd = _nan_kv(AR.bf16(torch.randn((B, K, C), generator=g)), v)
+    out, half = _attend(st.rt, torch.zeros((B, Q, C)), kd, vd, masked, am, layer=layer)
+    allowed = AR.effective_allowed(masked, am).double()
+    cnt = allowed.sum(-1, keepdim=True).numpy().astype(np.float32)
+    want = torch.from_numpy((allowed @ v.double()).numpy().astype(np.float32) * (np.float32(1) / cnt))
+    assert torch.equal(out, want), int((out != want).sum())
+
+
+ALPHA = 64.0
+
+
+def _codes(K, heads_perm):
+    """(K, C) key rows of +-1 codes: per head, bits of the key index in channels 0..15 and bits of a permuted index
+    (k * a + c mod 2^16, a odd) in channels 16..31."""
+    idx = torch.arange(K)
+    bits = lambda x: ((x[:, None] >> torch.arange(16)) & 1).float() * 2 - 1
+    rows = []
+    for a, c in heads_perm:
+        rows += [bits(idx), bits((idx * a + c) % 65536)]
+    return torch.cat(rows, 1)
+
+
+def _one_hot_case(g, B, Q, K):
+    """Key codes, V of bf16 normals with 2^-6 <= |v| < 16 (exact in half), a random mask, q = ALPHA x the code of an
+    allowed key t per (row, head), so t wins by >= 2 ALPHA = 128 (184 log2 units: every other P flushes to 0).  Every
+    4th row instead takes q = ALPHA x [code1(m), 0] of a MASKED key m: its one allowed distance-1 neighbour t wins by
+    2 ALPHA, the other neighbours are masked, so a lost mask bit returns v_m or a 50/50 blend.  Row (0, 0) is a
+    fallback row (q = the code of any key).  Returns q, k, v, masked, all_masked, t (B, Q, heads)."""
+    perm = [(2 * int(torch.randint(1, 30000, (1,), generator=g)) + 1, int(torch.randint(0, 65536, (1,), generator=g)))
+            for _ in range(8)]
+    k = _codes(K, perm)[None].expand(B, K, C).contiguous()
+    e = torch.randint(-6, 4, (B, K, C), generator=g).double()
+    mant = 1 + torch.randint(0, 128, (B, K, C), generator=g).double() / 128
+    sign = torch.randint(0, 2, (B, K, C), generator=g).double() * 2 - 1
+    v = (sign * mant * 2 ** e).float()
+    masked = torch.rand((B, Q, K), generator=g) < 0.5
+    am = torch.zeros((B, Q), dtype=torch.bool)
+    q = torch.zeros((B, Q, C))
+    t = torch.zeros((B, Q, 8), dtype=torch.long)
+    for b in range(B):
+        for qi in range(Q):
+            row = masked[b, qi]
+            if b == 0 and qi == 0:
+                row[:] = True
+                am[b, qi] = True
+            if qi % 4 == 3 and K > 1:
+                m = int(torch.randint(0, K, (1,), generator=g))
+                nb = [m ^ (1 << j) for j in range(16) if m ^ (1 << j) < K]
+                tt = nb[int(torch.randint(0, len(nb), (1,), generator=g))]
+                row[m] = True
+                row[nb] = True
+                row[tt] = False
+                for h in range(8):
+                    q[b, qi, h * 32:h * 32 + 16] = ALPHA * k[0, m, h * 32:h * 32 + 16]
+                t[b, qi] = tt
+                continue
+            if not (~row).any():
+                row[int(torch.randint(0, K, (1,), generator=g))] = False
+            ok = (~row).nonzero()[:, 0] if not am[b, qi] else torch.arange(K)
+            for h in range(8):
+                tt = int(ok[int(torch.randint(0, len(ok), (1,), generator=g))])
+                q[b, qi, h * 32:(h + 1) * 32] = ALPHA * k[0, tt, h * 32:(h + 1) * 32]
+                t[b, qi, h] = tt
+    return q, k, v, masked, am, t
+
+
+def _check_one_hot(what, out, half, v, t):
+    B, Q, _ = out.shape
+    idx = t.repeat_interleave(32, -1)                                 # (B, Q, C): key of each output channel
+    want = torch.gather(v, 1, idx)
+    bad = half.view(torch.int16) != want.half().view(torch.int16)
+    assert not bad.any(), '%s: %d half outputs are not the winning key\'s V, first at %s' % (
+        what, int(bad.sum()), bad.nonzero()[0].tolist())
+    err = float(((out.double() - want.double()).abs() / want.double().abs()).max())
+    assert err <= 2.0 ** -13, (what, err)
+
+
+@pytest.mark.parametrize('Q,B,K', [(8, 3, 2), (100, 3, 99), (129, 3, 777), (300, 1, 4096), (8, 1, 65536)])
+def test_k5_one_hot_exact(Q, B, K):
+    """Case b without a table: out_half must equal fp16(v_t) of the winning key t bit for bit, out within 2^-13 |v_t|
+    (the fp32 rounding residual of s_t log2e at s_t = 2048 leaves p_t = 2^(+-2^-13) in l)."""
+    st = _attn_rt(Q, B)
+    g = torch.Generator().manual_seed(K + Q)
+    q, k, v, masked, am, t = _one_hot_case(g, B, Q, K)
+    kd, vd = _nan_kv(k, v)
+    out, half = _attend(st.rt, q, kd, vd, masked, am)
+    _check_one_hot('Q=%d B=%d K=%d' % (Q, B, K), out, half, v, t)
+
+
+@pytest.mark.parametrize('H,W', [(352, 288), (1056, 800)])
+def test_k5_one_hot_exact_with_table(H, W):
+    """Case b with the production key-bias table of every layer (every level and slot): the cross-attention K weights
+    and key bias of the state dict are scaled by 2^-10, and the fp64 table must keep |q . R| <= ALPHA / 4, so that
+    the winner still wins by >= 96 (138 log2 units)."""
+    Q, B = 100, 3
+    sd = synth.make_params(seed=1, num_queries=Q, perturb=True)
+    for i in range(L):
+        p = 'transformer_decoder.layers.%d.attentions.0.attn.' % i
+        sd[p + 'in_proj_weight'][C:2 * C] *= 2.0 ** -10
+        sd[p + 'in_proj_bias'][C:2 * C] *= 2.0 ** -10
+    st = _attn_rt(Q, B, H, W, sd=sd)
+    g = torch.Generator().manual_seed(H)
+    for layer in range(L):
+        level = layer % 3
+        K = st.K[level]
+        r, _ = AR.key_bias_table(sd, layer, *st.sizes[level])
+        assert float(ALPHA * r.abs().view(K, 8, 32).sum(-1).max()) <= ALPHA / 4
+        q, k, v, masked, am, t = _one_hot_case(g, B, Q, K)
+        kd, vd = _nan_kv(k, v)
+        out, half = _attend(st.rt, q, kd, vd, masked, am, layer=layer)
+        _check_one_hot('%dx%d layer %d' % (H, W, layer), out, half, v, t)
+
+
+def _kv_views(st, level, sl):
+    """The production K, V views of layer slot sl in kv_l; every other column (the other slots' K and V) is NaN."""
+    buf = st.kv(level)
+    keep = torch.zeros(NL * 2 * C, dtype=torch.bool)
+    keep[sl * C:(sl + 1) * C] = True
+    keep[(NL + sl) * C:(NL + sl + 1) * C] = True
+    buf[:, :, ~keep.to(DEV)] = float('nan')
+    return buf[:, :, sl * C:(sl + 1) * C], buf[:, :, (NL + sl) * C:(NL + sl + 1) * C]
+
+
+Q_SCALES = (0.25, 1.0, 16.0)
+
+
+@pytest.mark.parametrize('H,W,layers', [(352, 288, tuple(range(L))), (1056, 800, (0, 4, 8))])
+def test_k5_production_cross_attention_within_bound(H, W, layers):
+    """Case c: K and V from cgg_kv_project of random bf16 memories with the synth weights, read as the column views
+    that tc_decoder_layer passes (every other column NaN), the handle's key-bias table of the layer, random / blob /
+    fallback masks, q at three scales.  Bound: attention_ref.reference against R = (pos + level_embed) Wk^T + bk in
+    fp64, plus the RMS bar.  At the sharpest scale the test first shows that the bound can fail: references with the
+    table's bf16 hi part only, the neighbouring slot's table and no table each exceed it somewhere."""
+    Q, B = 100, 3
+    sd = synth.make_params(seed=21, num_queries=Q, perturb=True)
+    st = _attn_rt(Q, B, H, W, sd=sd)
+    g = torch.Generator().manual_seed(W)
+    mems = [_bf16_randn(g, (B, C) + s) for s in st.sizes]
+    for layer in layers:
+        level, sl = layer % 3, layer // 3
+        K = st.K[level]
+        st.rt.kv_project([m.to(DEV) for m in mems])
+        kv = st.kv(level).cpu()
+        k, v = kv[:, :, sl * C:(sl + 1) * C].float(), kv[:, :, (NL + sl) * C:(NL + sl + 1) * C].float()
+        kd, vd = _kv_views(st, level, sl)
+        r, r_abs = AR.key_bias_table(sd, layer, *st.sizes[level])
+        masked = AR.random_mask(g, B, Q, K, (0.5, 0.9, 0.3)[layer % 3], blob=layer % 2 == 1)
+        am = masked.all(-1)
+        allowed = AR.effective_allowed(masked, am)
+        for sigma in Q_SCALES:
+            what = '%dx%d layer %d sigma %g' % (H, W, layer, sigma)
+            q = torch.randn((B, Q, C), generator=g) * sigma
+            ref, bound, _ = AR.reference(q, k, v, allowed, r=r, r_abs=r_abs, half=True)
+            if sigma == Q_SCALES[-1]:
+                nbr = layer + 3 if layer + 3 < L else layer - 3
+                for name, rm in (('hi only', AR.split_hi_lo(r)[0]), ('neighbouring slot', AR.key_bias_table(sd, nbr, *st.sizes[level])[0]),
+                                 ('no table', None)):
+                    refm = AR.reference(q, k, v, allowed, r=rm)[0]
+                    assert bool(((refm - ref).abs() > bound).any()), '%s: the %s reference is within the bound' % (what, name)
+            out, half = _attend(st.rt, q, kd, vd, masked, am, layer=layer)
+            _check_bound(what, out, half, ref, bound, K5_RMS_BAR[('prod', sigma)])
+
+
+# the (K, density, blob) cases of the former fp32-output stage test, then score ramps through one channel of K
+@pytest.mark.parametrize('case', [('rand', 64, 0.5, False), ('rand', 128, 0.0, False), ('rand', 777, 0.9, False),
+                                  ('rand', 4096, 0.5, False), ('rand', 4096, 0.9, True), ('rand', 16384, 0.5, True),
+                                  ('ramp', 4096, 10.0, False), ('ramp', 4096, -10.0, False), ('ramp', 1000, 7.5, False),
+                                  ('two', 1000, 0.3, False), ('two', 4096, 0.5, True)], ids=str)
+def test_k5_random_keys_within_bound(case):
+    """Cases c (no table: random bf16 K, V at q scales 0.25 / 1 / 16) and d (attention_ref.ramp_case: the lazy rescale
+    with 0 < sc < 2^-8 on every tile, never after the first, and P up to 2^7.5 before a move) and the two-level case
+    (attention_ref.two_level_case: exact scores, so the output also must match the float32 emulation within 2^-16 of
+    sum p |v| / l; a truncated P is off by 2^-8)."""
+    kind, K, density, blob = case
+    Q, B = 129, 3
+    st = _attn_rt(Q, B)
+    g = torch.Generator().manual_seed(K + int(density * 10))
+    keep = AR.TWO_LEVEL_ANCHORS if kind == 'two' else ()
+    masked = AR.random_mask(g, B, Q, K, density, blob=blob, keep=keep)
+    am = masked.all(-1)
+    allowed = AR.effective_allowed(masked, am)
+    if kind == 'rand':
+        k, v = _bf16_randn(g, (B, K, C)).float(), _bf16_randn(g, (B, K, C)).float()
+        qs = [(torch.randn((B, Q, C), generator=g) * s, s) for s in Q_SCALES]
+    elif kind == 'ramp':
+        q, k, v = AR.ramp_case(g, B, Q, K, density)
+        qs = [(q, 'ramp')]
+    else:
+        q, k, v = AR.two_level_case(g, B, Q, K)
+        qs = [(q, 'two')]
+    kd, vd = _nan_kv(k, v)
+    for q, bar in qs:
+        what = '%s K=%d %s' % (kind, K, bar)
+        ref, bound, _ = AR.reference(q, k, v, allowed, half=True)
+        out, half = _attend(st.rt, q, kd, vd, masked, am)
+        _check_bound(what, out, half, ref, bound, K5_RMS_BAR[('rand', bar) if kind == 'rand' else bar])
+        if kind == 'two':
+            emu = AR.emulate(q, k, v, allowed)[0]
+            a = AR.reference(q, k, v.abs(), allowed)[0]
+            err = float(((out.double() - emu.double()).abs() / a.clamp(min=1e-300)).max())
+            assert err <= 2.0 ** -16, (what, err)
+
+
+@pytest.mark.parametrize('Q', [100, 300])
+def test_k6_self_attention_form(Q):
+    """Case e: the decoder layer's self-attention call -- K and V interleaved in one buffer (row stride 2C plus 64
+    NaN padding columns, image stride Q rows), K = Q keys, no bitmap, half output -- with cases a (q = 0: column means,
+    exact), b (one-hot) and c (random, within the bound)."""
+    B = 3
+    st = _attn_rt(Q, B)
+    g = torch.Generator().manual_seed(Q)
+    W2 = 2 * C + 64
+
+    def interleaved(k, v):
+        buf = torch.full((B, Q, W2), NAN16, dtype=torch.int16).view(torch.bfloat16)
+        buf[:, :, :C], buf[:, :, C:2 * C] = k.bfloat16(), v.bfloat16()
+        buf = buf.to(DEV)
+        return buf[:, :, :C], buf[:, :, C:2 * C]
+
+    # a: every score 0
+    v = torch.randint(-8, 9, (B, Q, C), generator=g).float()
+    kd, vd = interleaved(AR.bf16(torch.randn((B, Q, C), generator=g)), v)
+    out, half = _attend(st.rt, torch.zeros((B, Q, C)), kd, vd)
+    want = torch.from_numpy(v.double().sum(1, keepdim=True).numpy().astype(np.float32) * (np.float32(1) / np.float32(Q)))
+    assert torch.equal(out, want.expand(B, Q, C)), int((out != want).sum())
+    # b: one-hot over Q keys, no mask
+    q, k, v, _, _, t = _one_hot_case(g, B, Q, Q)
+    for b in range(B):                     # without a bitmap every key is allowed: winners of the unmasked case
+        for qi in range(Q):
+            for h in range(8):
+                q[b, qi, h * 32:(h + 1) * 32] = ALPHA * k[0, t[b, qi, h], h * 32:(h + 1) * 32]
+    kd, vd = interleaved(k, v)
+    out, half = _attend(st.rt, q, kd, vd)
+    _check_one_hot('self-attention Q=%d' % Q, out, half, v, t)
+    # c: random operands
+    k, v = _bf16_randn(g, (B, Q, C)).float(), _bf16_randn(g, (B, Q, C)).float()
+    kd, vd = interleaved(k, v)
+    allowed = torch.ones((B, Q, Q), dtype=torch.bool)
+    for sigma in Q_SCALES:
+        q = torch.randn((B, Q, C), generator=g) * sigma
+        ref, bound, _ = AR.reference(q, k, v, allowed, half=True)
+        out, half = _attend(st.rt, q, kd, vd)
+        _check_bound('self-attention Q=%d sigma %g' % (Q, sigma), out, half, ref, bound)
+
+
+def test_k5_rejected_on_host():
+    """Arguments the entry must refuse, each before any launch (the library's launch count does not move)."""
+    Q, B, K = 100, 1, 64
+    head = _head(Q, seed=1)
+    rt = head._runtime(torch.device(DEV, 0))
+    lib = rt.lib
+    q = torch.zeros((B, Q, C), device=DEV)
+    kv = torch.zeros((B, 65537, C), dtype=torch.bfloat16, device=DEV)
+    k = kv[:, :K]
+
+    def refused(code, fn):
+        n0 = lib.cgg_launch_count()
+        with pytest.raises(_clib.CggError, match=code):
+            fn()
+        assert lib.cgg_launch_count() == n0, code + ': a kernel was launched'
+
+    refused('CGG_ERR_BAD_SHAPE', lambda: rt.masked_attention(q, k, k, layer=0))          # not prepared: no table
+    st = _Stage(head, 256, 256, B)
+    refused('CGG_ERR_BAD_SHAPE', lambda: rt.masked_attention(q, k, k, layer=L))
+    refused('CGG_ERR_BAD_SHAPE', lambda: rt.masked_attention(q, k, k, layer=-2))
+    refused('CGG_ERR_BAD_SHAPE', lambda: rt.masked_attention(q, k, k, layer=1))          # level 1 has 256 keys
+    refused('CGG_ERR_BAD_SHAPE', lambda: rt.masked_attention(q, kv, kv))                 # 65537 keys: 513 tiles
+    rt.masked_attention(q, kv[:, :65536], kv[:, :65536])                                 # 65536 keys: accepted
+    rt.masked_attention(q, kv[:, :st.K[0]], kv[:, :st.K[0]], layer=0)
+
+    def no_output():
+        _clib.check(lib.cgg_masked_attention(rt.handle, B, K, q.data_ptr(), k.data_ptr(), k.data_ptr(), C, K * C,
+                                             None, None, -1, None, None, rt._stream()), rt.handle, 'no output')
+    refused('CGG_ERR_NULL', no_output)
+    sd = synth.make_params(seed=1, num_queries=Q, perturb=True)
+    rt32 = build_head_from_state_dict(sd, Q, 49, 'fp32', DEV)._runtime(torch.device(DEV, 0))
+    rt32.prepare(32, 32, [(4, 4), (8, 8), (16, 16)], B)
+    k32 = torch.zeros((B, 16, C), device=DEV)
+    refused('CGG_ERR_UNSUPPORTED', lambda: rt32.masked_attention(q, k32, k32, layer=0))
+    refused('CGG_ERR_UNSUPPORTED', lambda: rt32.masked_attention(q, k32, k32, out_half=True))

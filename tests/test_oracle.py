@@ -162,3 +162,52 @@ def test_oracle_pred_emb_norm_matches_live_reference():
         assert float((ref[1][j] - out['emb'][j]).abs().max()) < TOL
         assert float((out['emb'][j].norm(dim=-1) - 1).abs().max()) < 1e-5
 
+
+
+def _bound_ratio(got, ref, bound):
+    """max |got - ref| / bound; a nonzero error where the bound is 0 (a row without an allowed key) counts as inf."""
+    err = (got.double() - ref).abs()
+    r = torch.where(bound > 0, err / bound.clamp(min=1e-300), torch.where(err > 0, float('inf'), 0.0))
+    return float(r.max())
+
+
+def test_attention_bound_passes_the_kernel_emulation_and_fails_its_mutants():
+    """The elementwise bound of the bf16 attention kernel (tests/golden/attention_ref.py, used by the K5 GPU tests) on
+    a float32 emulation of the kernel's arithmetic: bf16(q), P = bf16(e) with an fp32 l, the per-quarter lazy
+    reference, the half store.  The emulation must stay within it, and each mutant -- the table's hi part only, the
+    neighbouring slot's table, P truncated to bf16, no rescale (sc = 1), the tail mask ignored, the fallback ignored --
+    must exceed it somewhere, so the GPU tests' bound is known to be able to fail.  Production-like inputs: layer 4's
+    table (level 1, slot 1) on a 22x18 level (396 keys, a partial last tile)."""
+    import attention_ref as A
+    g = torch.Generator().manual_seed(0)
+    B, Q, C = 2, 64, 256
+    sd = synth.make_params(seed=3, num_queries=Q, perturb=True)
+    h, w, layer = 22, 18, 4
+    K = h * w
+    r, r_abs = A.key_bias_table(sd, layer, h, w)
+    hi, lo = A.split_hi_lo(r)
+    nhi, nlo = A.split_hi_lo(A.key_bias_table(sd, layer + 3, h, w)[0])
+    wkv = sd['transformer_decoder.layers.%d.attentions.0.attn.in_proj_weight' % layer][C:]
+    mem = torch.randn((B, K, C), generator=g)
+    k, v = A.bf16(mem @ wkv[:C].t()), A.bf16(mem @ wkv[C:].t())
+    masked = A.random_mask(g, B, Q, K, 0.5)
+    am = masked.all(-1)
+    allowed = A.effective_allowed(masked, am)
+    q = torch.randn((B, Q, C), generator=g) * 16          # sharp: the table's lo part matters
+    ref, bound, _ = A.reference(q, k, v, allowed, r=r, r_abs=r_abs, half=True)
+    out, half = A.emulate(q, k, v, allowed, hi, lo)
+    assert _bound_ratio(out, ref, bound) <= 0.5 and _bound_ratio(half, ref, bound) <= 0.5
+    mutants = {'hi only': A.emulate(q, k, v, allowed, hi)[0],
+               'neighbouring slot': A.emulate(q, k, v, allowed, nhi, nlo)[0],
+               'sc = 1': A.emulate(q, k, v, allowed, hi, lo, mutant='sc_one')[0],
+               'tail ignored': A.emulate(q, k, v, allowed, hi, lo, mutant='tail')[0],
+               'fallback ignored': A.emulate(q, k, v, A.effective_allowed(masked, None), hi, lo)[0]}
+    # P's rounding, on exact two-level scores and positive V (a truncated P is 2^-7.5 low, the bound allows 2^-8)
+    K2 = 1000
+    q2, k2, v2 = A.two_level_case(g, B, Q, K2)
+    al2 = A.effective_allowed(A.random_mask(g, B, Q, K2, 0.3, keep=A.TWO_LEVEL_ANCHORS), None)
+    ref2, bound2, _ = A.reference(q2, k2, v2, al2, half=True)
+    assert _bound_ratio(A.emulate(q2, k2, v2, al2)[1], ref2, bound2) <= 0.75
+    worst = {name: _bound_ratio(got, ref, bound) for name, got in mutants.items()}
+    worst['P truncated'] = _bound_ratio(A.emulate(q2, k2, v2, al2, mutant='p_trunc')[0], ref2, bound2)
+    assert all(x > 1.1 for x in worst.values()), worst
